@@ -22,6 +22,9 @@ synthetic jets (128 particles, 3 continuous + 8 tokens), batch 4096 per GPU, 100
                  sample of the same workload, rank 0, N=1 only
   roofline_dense the same kernel on a batch whose jets all have 128 live particles (the C2 multiplicities skip dead rows)
   --impl reference   times that CPU port alone (the reference is pure Python and does not travel)
+  --dump-outputs DIR c2: after the timed steps, the jets the last timed step generated (all ranks' jets when N > 1) as float32
+                 DIR/{continuous,discrete,mask,jet_index}.npy; the inputs depend on the arguments alone, so two builds can be
+                 compared output for output
   --workload     c2 (default, the headline) | c3 (one transepic evaluation, B=8192) | c4 (absorbing-flow generation, B=4096) |
                  c5 (1 M jets sharded over the GPUs: source + generation + observables + histograms + gather); with N > 1 the
                  c2 line carries a bounded c5 leg as well (`c5_million_jets`); wide = the C2 loop on an EPiC of the reference's
@@ -36,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is cached in it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -48,6 +52,7 @@ C5_MICRO_BATCH = 16384
 FLOP_PER_JET_STEP = 0.819e6          # SURVEY.md §8d (2*MAC, default widths)
 UPDATE_BYTES_PER_PARTICLE = 75       # SURVEY.md §8d / BASELINE.md §4
 CPU_SAMPLE_JETS = 16384              # bounded CPU sample: ~15 s on 16 host threads at ~1.1 K jets/s
+DUMP_MAX_JETS = 16384                # --dump-outputs: 16384 jets x 128 particles x 5 float32 values = 42 MB (bound: 64 MB)
 
 
 def peaks():
@@ -114,6 +119,21 @@ def source_batch(n_jets, seed):
     return jetclass_like_databatch(n_jets, N_PART, generator=torch.Generator().manual_seed(seed))
 
 
+def dump_outputs(directory, **arrays):
+    """--dump-outputs: one float32 DIR/<name>.npy per array (jet-major), and the jets' indices in jet_index.npy.  Beyond
+    DUMP_MAX_JETS jets a fixed, seeded sample of the jets is written."""
+    import numpy as np
+    import torch
+    n = next(iter(arrays.values())).shape[0]
+    idx = torch.arange(n)
+    if n > DUMP_MAX_JETS:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_MAX_JETS].sort().values
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "jet_index.npy"), idx.numpy().astype(np.float32))
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), t.cpu()[idx].float().numpy())
+
+
 def host_threads():
     """Threads the CPU arm uses: every core this process may run on.  Set explicitly — torchrun exports OMP_NUM_THREADS=1,
     which would otherwise serialise the OpenMP port (round 1: the reference arm timed out at N = 2, 4, 8)."""
@@ -178,7 +198,12 @@ def main():
                     help="N > 1: per-batch exchange of the generated jets (auto: copy-engine push over NVLink peer memory, else NCCL)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the C3 / C4 / C5 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="c2: write the jets generated by the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl, args.workload) != ("native", "c2"):
+        ap.error("--dump-outputs writes the jets of the c2 generation (--impl native --workload c2)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -278,6 +303,15 @@ def main():
         t_end.record(stream)
         torch.cuda.synchronize()
         t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs:
+        last = W + K - 1
+        if world > 1:   # what a rank holds after a step: the generated jets of every rank, from the exchange
+            g = gather_bufs[last & 1]
+            x_out, k_out, m_out = (torch.cat([view(r) for r in range(world)]) for view in (g.x, g.k, g.mask))
+        else:
+            x_out, k_out, m_out = xs[last], ks[last], mask
+        if rank == 0:
+            dump_outputs(args.dump_outputs, continuous=x_out, discrete=k_out, mask=m_out)
     if world > 1:
         dist.barrier()
     ms = t_begin.elapsed_time(t_end)
@@ -419,18 +453,19 @@ def side_workload_line(args, torch, dist, _native, device, pk, rank, world, W, K
     if args.workload == "c5":
         from multimodal_particles_b200.pipeline import sharded_generation_run
         cfg, model = build_model(device)
-        with ClockSampler(device.index or 0) as clocks:
-            rec = sharded_generation_run(model, cfg, 1 << 20, rank, world, device, micro_batch=C5_MICRO_BATCH, n_particles=N_PART,
-                                         precision=args.precision, gather=args.gather)
+        with ClockSampler(device.index or 0) as clocks:   # a step: one timed 1 M-jet run (each after its own 2 warm-up micro-batches)
+            recs = [sharded_generation_run(model, cfg, 1 << 20, rank, world, device, micro_batch=C5_MICRO_BATCH, n_particles=N_PART,
+                                           precision=args.precision, gather=args.gather) for _ in range(K)]
         if rank != 0:
             return None
-        return {"metric": METRIC, "value": rec["value"], "unit": "jets/s", "n_gpus": world, "steps": 1, "warmup": 2,
-                "ms_per_step": rec["seconds"] * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+        rec, seconds = recs[-1], sum(r["seconds"] for r in recs)
+        return {"metric": METRIC, "value": K * (1 << 20) / seconds, "unit": "jets/s", "n_gpus": world, "steps": K, "warmup": 2,
+                "ms_per_step": seconds * 1e3 / K, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": {"f16": "f16", "bf16": "bf16", "fp32": "f32"}[rec["precision"]], "data": "synthetic",
                 "config": {"workload": rec["workload"], "global_batch": 1 << 20}, "c5_million_jets": rec, "clocks": clocks.summary(),
-                "gpu_launches": 5 * ((1 << 20) // B_PER_GPU // world)}
+                "gpu_launches": K * 5 * ((1 << 20) // B_PER_GPU // world)}
     with ClockSampler(device.index or 0) as clocks:
-        rec = secondary_configs(torch, _native, device, pk, only=args.workload, reps=max(K, 2), warm=max(W, 2))
+        rec = secondary_configs(torch, _native, device, pk, only=args.workload, reps=K, warm=max(W, 2))
     key = {"c3": "C3_transepic_evaluation", "c4": "C4_absorbing_generation", "wide": "wide_epic"}[args.workload]
     r = rec[key]
     rate = r["jet_evals_per_s"] if args.workload == "c3" else r["jets_per_s"]
@@ -442,7 +477,7 @@ def side_workload_line(args, torch, dist, _native, device, pk, rank, world, W, K
         return None
     metric = "TransdimensionalEPiC evaluations/sec (jets, 128 particles)" if args.workload == "c3" else METRIC
     return {"metric": metric, "value": rate, "unit": "jet-evaluations/s" if args.workload == "c3" else "jets/s", "n_gpus": world,
-            "steps": max(K, 2), "warmup": max(W, 2), "ms_per_step": float(t.item()), "higher_is_better": True, "scaling": "weak",
+            "steps": K, "warmup": max(W, 2), "ms_per_step": float(t.item()), "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "bf16", "data": "synthetic", "config": {"workload": r["workload"]},
             "roofline": r.get("roofline") or r.get("roofline_head"), "clocks": clocks.summary(), "detail": r}
 
@@ -468,11 +503,11 @@ def secondary_configs(torch, _native, device, pk, only=None, reps=None, warm=Non
     if only in (None, "c4"):
         out.update(_c4(torch, _native, device, pk, timed, reps or 2, warm or 1))
     if only in (None, "wide"):
-        out.update(_wide(torch, _native, device, pk, timed, reps or 3, warm or 2))
+        out.update(_wide(torch, _native, device, pk, timed, reps or 3, warm or 2, gen_reps=reps or 1))
     return out
 
 
-def _wide(torch, _native, device, pk, timed, reps, warm):
+def _wide(torch, _native, device, pk, timed, reps, warm, gen_reps):
     """The C2 workload on an encoder of the reference's CLASS-DEFAULT widths (EPiCNetwork: num_blocks = 6, dim_hidden_local =
     128, dim_hidden_global = 10; architectures/epic.py:99-101) — the shape where the trunk is GEMM work: 0.415 MFLOP per
     particle and evaluation (12 x 2 x 128 x 128 + local_0 + output layer), all 128 slots of a jet in the reference."""
@@ -507,7 +542,7 @@ def _wide(torch, _native, device, pk, timed, reps, warm):
     ev = timed(lambda: five(m), reps, warm) / 5
     ev_full = timed(lambda: five(ones), reps, warm) / 5
     ev_fp32 = timed(lambda: native.forward(x[:512], k[:512], m[:512], temb, precision="fp32"), 1, 1) * (B / 512)
-    gen = timed(lambda: native.generate(x.clone(), k.clone(), m, table, seed=1, jet_offset=0, precision="bf16"), max(1, reps // 2), 1)
+    gen = timed(lambda: native.generate(x.clone(), k.clone(), m, table, seed=1, jet_offset=0, precision="bf16"), gen_reps, 1)
     live = float(m.float().mean().item())
     return {"wide_epic": {"workload": "EPiC at the class-default widths (H=128, L=6, G=10), B=4096, N=128: one evaluation and a 99-step generation",
                           "ms": gen, "jets_per_s": B / (gen * 1e-3), "evaluation_ms": ev, "jet_evals_per_s": B / (ev * 1e-3),

@@ -1,6 +1,6 @@
 """End-to-end latency of simulate_dynamics (pinned host state in, host state out) for different numbers of pipeline slices."""
-import sys, time, torch
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys, time, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench
 from multimodal_particles_b200 import HybridState
 dev = torch.device("cuda:0")

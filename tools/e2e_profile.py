@@ -1,6 +1,6 @@
 """Where the host-side microseconds of one simulate_dynamics call (pinned host state in, host state out) go."""
-import sys, time, gc, torch
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys, time, gc, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench
 from multimodal_particles_b200 import HybridState, _native
 dev = torch.device("cuda:0")

@@ -1,7 +1,7 @@
 """Where the end-to-end time of mmb_generate_host goes: wall clock of the bare C call + synchronise (buffers preallocated),
 device time between the caller-stream events around it, and the same through simulate_dynamics."""
-import ctypes, sys, time, torch
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, ctypes, sys, time, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench
 from multimodal_particles_b200 import HybridState, _native
 from multimodal_particles_b200.steptable import CStepTable
