@@ -480,6 +480,29 @@ int mmb_jet_observables(const float* x, const uint8_t* k, const uint8_t* mask, c
                         float* x_phys, int8_t* flavor_charge, float* jets, void* stream);
 
 /*
+ * Jet substructure of a generated batch (the clustering-based observables of JetClassHighLevelFeatures.substructure,
+ * mp/data/particle_clouds/jets.py:204-240), so that validation on tau21, tau32 and D2 needs the 32-byte rows, not the clouds:
+ *   constituents (pt, eta, phi) = (x * std + mean) in fp32 (mean / std: HOST float[3], or NULL for physical input), massless;
+ *   a particle is used iff mask != 0 && pt > 0.
+ *   Exclusive kt clustering with WTA_pt recombination over the used particles, in fp64 without contraction:
+ *     d_ij = min(pt_i^2, pt_j^2) dR_ij^2 (1 / R^2) (dphi wrapped into [-pi, pi]), d_iB = pt_i^2; each step takes the minimum of
+ *     all d_ij and d_iB, ties to the smaller (lower, upper) index pair, a beam candidate being (i, i).  A pair merges into the
+ *     lower index with pt_i + pt_j and the direction of the harder one (lower index on a pt tie); a beam step removes the
+ *     object.  The exclusive n-jet axes are the objects left when n remain (n = 3, 2, 1).
+ *   tau_N = sum_i pt_i min_a dR(i,a)^beta / sum_i pt_i R^beta;  tau21 = tau2 / tau1, tau32 = tau3 / tau2;
+ *   with z_i = pt_i / sum_j pt_j (arXiv:1409.6298): e2 = sum_{i<j} z_i z_j dR_ij^beta,
+ *   e3 = sum_{i<j<k} z_i z_j z_k (dR_ij dR_ik dR_jk)^beta, D2 = e3 / e2^3.
+ * A jet with fewer than 3 used particles gets NaN in every column and axes -1; 0/0 ratios are NaN.
+ * x [B,N,3] f32, mask [B,N] u8, N <= 256 (larger N: MMB_EINVAL); R > 0, beta > 0.
+ * Outputs: out [B][MMB_SUB_OBS] f32 in the order of the enum below; axes [B][6] int16 (nullable): the particle slot (0..N-1)
+ * whose direction is each WTA axis — tau1 axis | tau2 axes | tau3 axes, each set in ascending order of its object's slot.
+ */
+enum { MMB_SUB_TAU1 = 0, MMB_SUB_TAU2, MMB_SUB_TAU3, MMB_SUB_TAU21, MMB_SUB_TAU32, MMB_SUB_E2, MMB_SUB_E3, MMB_SUB_D2, MMB_SUB_OBS };
+#define MMB_SUB_MAX_N 256
+int mmb_jet_substructure(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N, float R, float beta,
+                         float* out, int16_t* axes, void* stream);
+
+/*
  * Source-state construction on the device (SURVEY.md §8f N3), so that a generation run needs no host data loader:
  *   sample_noise("GaussNoise") (mp/data/particle_clouds/utils.py:222-251): x ~ N(0,1) * scale, flavor ~ Categorical(cat_probs[5]),
  *   charge = +-1 (0 for photons / neutral hadrons), turned into the 8 tokens of physics_to_onehot + argmax

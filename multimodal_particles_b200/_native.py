@@ -106,6 +106,7 @@ SIGNATURES = {
                                     _vp, _sz, _i, _vp]),
     "mmb_validation_histograms": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _f, _i, _vp, _vp]),
     "mmb_jet_observables": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
+    "mmb_jet_substructure": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _f, _vp, _vp, _vp]),
     "mmb_sample_source": (_i, [_vp, _vp, _vp, _i, _i, _f, _vp, _vp, _u64, _u64, _vp]),
     "mmb_sample_bridges": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _f, _i, _vp, _vp, _u64, _u64, _i, _i, _vp, _vp, _vp]),
     "mmb_absorbing_sample": (_i, [_vp, _vp, _vp, _u64, _u64, _i, _i, _vp, _vp]),

@@ -734,6 +734,17 @@ int mmb_jet_observables(const float* x, const uint8_t* k, const uint8_t* mask, c
     return launch_jet_observables(x, k, mask, mean, std, B, N, x_phys, flavor_charge, jets, static_cast<cudaStream_t>(stream));
 }
 
+int mmb_jet_substructure(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N, float R, float beta,
+                         float* out, int16_t* axes, void* stream) {
+    if (!x || !mask || !out) return fail(MMB_EINVAL, "mmb_jet_substructure: null argument");
+    if ((mean == nullptr) != (std == nullptr)) return fail(MMB_EINVAL, "mmb_jet_substructure: mean and std go together");
+    if (B < 0 || N < 0) return fail(MMB_EINVAL, "mmb_jet_substructure: negative size");
+    if (N > MMB_SUB_MAX_N) return fail(MMB_EINVAL, "mmb_jet_substructure: N = %d exceeds %d particle slots", N, MMB_SUB_MAX_N);
+    if (!(R > 0.0f) || !(beta > 0.0f)) return fail(MMB_EINVAL, "mmb_jet_substructure: R and beta must be positive");
+    if (B == 0) return MMB_OK;
+    return launch_jet_substructure(x, mask, mean, std, B, N, R, beta, out, axes, static_cast<cudaStream_t>(stream));
+}
+
 int mmb_sample_source(float* x, uint8_t* k, uint8_t* mask, int B, int N, float scale, const float* cat_probs, const float* mult_cdf,
                       uint64_t seed, uint64_t jet_offset, void* stream) {
     if (!x || !k || !mask || !cat_probs) return fail(MMB_EINVAL, "mmb_sample_source: null argument");

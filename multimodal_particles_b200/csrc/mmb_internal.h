@@ -104,6 +104,10 @@ int launch_validation_histograms(const float* x, const uint8_t* k, const uint8_t
 int launch_jet_observables(const float* x, const uint8_t* k, const uint8_t* mask, const float* mean, const float* sd, int B, int N,
                            float* x_phys, int8_t* fc, float* jets, cudaStream_t stream);
 
+// substructure.cu — N-subjettiness and energy correlation functions, one block per jet, N <= MMB_SUB_MAX_N
+int launch_jet_substructure(const float* x, const uint8_t* mask, const float* mean, const float* sd, int B, int N, float R, float beta,
+                            float* out, int16_t* axes, cudaStream_t stream);
+
 int launch_sample_source(float* x, uint8_t* k, uint8_t* mask, int B, int N, float scale, const float* cat_probs, const float* mult_cdf,
                          uint64_t seed, uint64_t jet_offset, cudaStream_t stream);
 

@@ -2,8 +2,9 @@
 ``ParticleClouds`` (mp/data/particle_clouds/particles.py:22-156: construction from a ``HybridState``, ``postprocess``,
 ``compute_4mom``) and ``JetClassHighLevelFeatures`` (mp/data/particle_clouds/jets.py:85-141, 329-332: jet kinematics,
 multiplicity, jet charges, 1-D Wasserstein distance), SURVEY.md §8f N1.  One fused kernel (``mmb_jet_observables``) does the
-de-standardisation, ``tokens_to_physics``, the 4-momenta and the per-jet sums; only the clustering-based substructure
-(fastjet N-subjettiness / D2, jets.py:204-240) is not provided.
+de-standardisation, ``tokens_to_physics``, the 4-momenta and the per-jet sums.  The clustering-based substructure (fastjet
+N-subjettiness on exclusive kt / WTA axes and D2, jets.py:204-240) is a second kernel (``mmb_jet_substructure``,
+``jet_substructure``); ``JetClassHighLevelFeatures.compute_substructure`` sets its columns.
 """
 import ctypes
 
@@ -32,6 +33,29 @@ def jet_observables(x, k_u8, mask_u8, stats=None, want_particles=True):
         _native.check(_native.load().mmb_jet_observables(_native._ptr(x), _native._ptr(k_u8), _native._ptr(mask_u8), mean, std, B, N,
                                                          _native._ptr(x_phys), _native._ptr(fc), _native._ptr(jets), _native._stream()))
     return x_phys, fc, jets
+
+
+SUBSTRUCTURE_COLUMNS = ("tau1", "tau2", "tau3", "tau21", "tau32", "e2", "e3", "d2")
+
+
+def jet_substructure(x, mask_u8, stats=None, R=0.8, beta=1.0, want_axes=False):
+    """x [B,N,3] f32 (pt, eta, phi; standardised when ``stats`` is given), mask [B,N] u8 on the GPU, N <= 256
+    -> [B,8] f32 in the order of ``SUBSTRUCTURE_COLUMNS`` (, axes [B,6] int16: the particle slot of the tau1 axis, the two tau2
+    axes and the three tau3 axes).  Jets with fewer than 3 used particles (mask and pt > 0) are NaN, axes -1.  R: radius of
+    the exclusive kt clustering; beta: angular exponent of tau_N and of the energy correlation functions."""
+    _native._require_cuda(x, mask_u8)
+    B, N, _ = x.shape
+    dev = x.device
+    out = torch.empty(B, len(SUBSTRUCTURE_COLUMNS), dtype=torch.float32, device=dev)
+    axes = torch.empty(B, 6, dtype=torch.int16, device=dev) if want_axes else None
+    mean = std = None
+    if stats is not None:
+        mean = (ctypes.c_float * 3)(*[float(v) for v in stats["mean"][:3]])
+        std = (ctypes.c_float * 3)(*[float(v) for v in stats["std"][:3]])
+    with torch.cuda.device(dev):
+        _native.check(_native.load().mmb_jet_substructure(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(R), float(beta),
+                                                          _native._ptr(out), _native._ptr(axes), _native._stream()))
+    return (out, axes) if want_axes else out
 
 
 class ParticleClouds:
@@ -108,6 +132,19 @@ class JetClassHighLevelFeatures:
 
     def substructure(self):
         raise NotImplementedError("fastjet substructure (jets.py:204-240) stays on the CPU side of the reference")
+
+    def compute_substructure(self, R=0.8, beta=1.0):
+        """N-subjettiness and D2 on the device (``jet_substructure``) from the physical constituents: sets ``tau1``, ``tau2``,
+        ``tau3``, ``tau21``, ``tau32`` and ``d2`` over the jets with at least 3 used particles (the others are dropped, as
+        the reference drops them), so that ``Wassertein1D("tau21", other)`` compares them."""
+        c = self.constituents
+        dev = c.continuous.device if c.continuous.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        out, axes = jet_substructure(c.continuous.to(dev, torch.float32).contiguous(), as_u8(c.mask.to(dev)), None, R, beta,
+                                     want_axes=True)
+        keep = axes[:, 0] >= 0
+        out = out[keep].to(c.continuous.device)
+        for name in ("tau1", "tau2", "tau3", "tau21", "tau32", "d2"):
+            setattr(self, name, out[:, SUBSTRUCTURE_COLUMNS.index(name)])
 
     def Wassertein1D(self, feature, reference):
         import scipy.stats

@@ -8,7 +8,8 @@ particles.py:85-89,124-156, jets.py:90-107) and the validation histograms (``mmb
 per-GPU int64 counts.  Exchanges (SURVEY.md §8e): the packed micro-batch (1 792 B / jet) goes to every rank once per micro-batch,
 on a side stream under the next micro-batch's generation — pushed over NVLink peer memory by the copy engines
 (``sharding.PeerGather``; one NCCL all-gather where peer memory is unavailable) — and one all-reduce of the histograms and of the
-jet-observable sums at the end.  The reference has no multi-GPU code (SURVEY.md §2.1); ``tools/million_jets.py`` and the
+jet-observable sums at the end.  With ``substructure=True`` the side stream also runs ``mmb_jet_substructure`` on every micro-batch
+and histograms tau21, tau32 and D2 into int64 counts of their own (SUBSTRUCTURE_BINS).  The reference has no multi-GPU code (SURVEY.md §2.1); ``tools/million_jets.py`` and the
 multi-GPU arms of ``bench.py`` call this.
 """
 import hashlib
@@ -18,16 +19,49 @@ import torch
 import torch.distributed as dist
 
 from . import sharding
-from .observables import jet_observables
+from .observables import SUBSTRUCTURE_COLUMNS, jet_observables, jet_substructure
 from .source import sample_source_state
 
 STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisation to a jet-like scale (pT > 0)
+# substructure histograms: (column, lo, hi) with 100 bins each, out-of-range values in the edge bins, then one count of the jets
+# where the observable is undefined (NaN); counts layout [3][101]
+SUBSTRUCTURE_HISTS = (("tau21", 0.0, 1.0), ("tau32", 0.0, 1.0), ("d2", 0.0, 10.0))
+SUBSTRUCTURE_BINS = 100
+
+
+class SubstructureHistograms:
+    """int64 counts [3 * 101] and sums of the defined values [3] (f64) of tau21, tau32 and D2; integer scatter-adds only, so
+    the counts do not depend on the batching or on the order of the jets."""
+
+    def __init__(self, device):
+        nb = SUBSTRUCTURE_BINS
+        self.cols = [SUBSTRUCTURE_COLUMNS.index(c) for c, _, _ in SUBSTRUCTURE_HISTS]
+        self.lo = torch.tensor([h[1] for h in SUBSTRUCTURE_HISTS], dtype=torch.float32, device=device)
+        self.scale = torch.tensor([nb / (h[2] - h[1]) for h in SUBSTRUCTURE_HISTS], dtype=torch.float32, device=device)
+        self.offset = torch.arange(3, device=device) * (nb + 1)
+        self.counts = torch.zeros(3 * (nb + 1), dtype=torch.int64, device=device)
+        self.sums = torch.zeros(3, dtype=torch.float64, device=device)
+
+    def add(self, sub):
+        """Adds one batch of ``jet_substructure`` rows [B, 8]."""
+        nb = SUBSTRUCTURE_BINS
+        v = sub[:, self.cols]
+        undefined = torch.isnan(v)
+        b = ((v - self.lo) * self.scale).floor().clamp_(0, nb - 1)
+        b = torch.where(undefined, float(nb), b).long() + self.offset
+        self.counts.scatter_add_(0, b.reshape(-1), torch.ones(b.numel(), dtype=torch.int64, device=sub.device))
+        self.sums.add_(torch.where(undefined, 0.0, v).double().sum(0))
+
+    def zero_(self):
+        self.counts.zero_()
+        self.sums.zero_()
 
 
 def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_batch=4096, n_particles=128, precision="auto",
-                           warmup_batches=2, gather="auto"):
+                           warmup_batches=2, gather="auto", substructure=False):
     """-> dict (rank 0: the C5 record; other ranks: None).  Device time by CUDA events around the whole slice incl. the final
-    all-reduce, max over ranks."""
+    all-reduce, max over ranks.  ``substructure``: also histogram tau21, tau32 and D2 of every jet (``substructure_sha1``,
+    ``substructure_counts`` and the means of the defined values join the record)."""
     native = model.encoder.native_model(device)
     table = model.step_table()
     lo, hi = sharding.shard_range(total_jets, rank, world)
@@ -36,6 +70,7 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     hist = sharding.ValidationHistograms(device, vocab_size=cfg.data.vocab_size_features)
     counts = torch.zeros(hist.size, dtype=torch.int64, device=device)
     jet_sums = torch.zeros(11, dtype=torch.float64, device=device)
+    sub_hist = SubstructureHistograms(device) if substructure else None
     packs = [sharding.PackedJets(MB, N, 3, device) for _ in range(3)]      # state of a micro-batch: [x | tokens | mask], one allocation
     recv = [sharding.make_gather(MB, N, 3, world, device, mode=gather) for _ in range(2)] if world > 1 else None
     side = torch.cuda.Stream(device=device)
@@ -62,6 +97,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
                 _, _, jets = jet_observables(x, k, m, STATS, want_particles=False)
                 counts.add_(hist.accumulate(x, k, m))
                 jet_sums.add_(torch.nan_to_num(jets.double()).sum(0))
+                if substructure:
+                    sub_hist.add(jet_substructure(x, m, STATS))
                 if world > 1 and B == MB:
                     recv[i & 1].gather(pk)          # the packed micro-batch to every rank (copy-engine push, or one all-gather)
                 for t in (x, k, m):
@@ -73,6 +110,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     run(lo, min(hi, lo + warmup_batches * MB))       # warm-up, then reset the accumulators
     counts.zero_()
     jet_sums.zero_()
+    if substructure:
+        sub_hist.zero_()
     torch.cuda.synchronize(device)
     if world > 1:
         dist.barrier()
@@ -82,6 +121,9 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     if world > 1:
         dist.all_reduce(counts)
         dist.all_reduce(jet_sums)
+        if substructure:
+            dist.all_reduce(sub_hist.counts)
+            dist.all_reduce(sub_hist.sums)
     e.record(main_s)
     torch.cuda.synchronize(device)
     t = torch.tensor([s.elapsed_time(e)], dtype=torch.float64, device=device)
@@ -93,7 +135,7 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     off = 3 * hist.bins + cfg.data.vocab_size_features
     host_counts = counts.cpu().numpy()
     mult = host_counts[off:]
-    return {"workload": f"C5: {total_jets} jets, N={N}, {table.n_steps} solver steps; source + generation + observables + histograms on "
+    rec = {"workload": f"C5: {total_jets} jets, N={N}, {table.n_steps} solver steps; source + generation + observables + histograms on "
                         f"the device, per-micro-batch all-gather of the jets + final all-reduce of the histograms",
             "n_gpus": world, "micro_batch": MB, "exchange": recv[0].kind if recv else "none", "seconds": ms * 1e-3, "value": total_jets / (ms * 1e-3), "unit": "jets/s",
             "precision": native.generate_precision(N, precision),
@@ -102,3 +144,13 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
             "token_counts": host_counts[3 * hist.bins:off].tolist(),
             # integer counts of jets keyed by their GLOBAL index: identical for every number of GPUs
             "histogram_sha1": hashlib.sha1(host_counts.astype(np.int64).tobytes()).hexdigest()}
+    if substructure:
+        sc = sub_hist.counts.cpu().numpy().astype(np.int64)
+        per = sc.reshape(3, SUBSTRUCTURE_BINS + 1)
+        sums = sub_hist.sums.cpu().numpy()
+        rec["substructure_counts"] = {name: per[i].tolist() for i, (name, _, _) in enumerate(SUBSTRUCTURE_HISTS)}
+        for i, (name, _, _) in enumerate(SUBSTRUCTURE_HISTS):
+            defined = int(per[i, :SUBSTRUCTURE_BINS].sum())
+            rec[f"mean_{name}"] = float(sums[i] / defined) if defined else float("nan")
+        rec["substructure_sha1"] = hashlib.sha1(sc.tobytes()).hexdigest()
+    return rec
