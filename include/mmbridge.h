@@ -503,6 +503,25 @@ int mmb_jet_substructure(const float* x, const uint8_t* mask, const float* mean,
                          float* out, int16_t* axes, void* stream);
 
 /*
+ * 1-D Wasserstein distance per column between two samples (JetClassHighLevelFeatures.Wassertein1D, jets.py:329-332, which is
+ * scipy.stats.wasserstein_distance), so that scoring generated jets against a reference needs no host copy of either sample:
+ *   the non-finite values (NaN, +-inf) of each column are dropped and counted out; n' and m' finite x and y values remain;
+ *   z_0 <= z_1 <= ... is the merged sorted sequence of both, i_k and j_k the numbers of x and y values <= z_k;
+ *   W1 = sum_k |i_k m' - j_k n'| (z_{k+1} - z_k) / (n' m'),  |i_k m' - j_k n'| exact in int64, differences and sum in fp64;
+ *   n' = 0 or m' = 0: NaN.
+ * Radix sort of each column (CUB), merge-path integration in fixed tiles, fixed-order sums: the result is bit-identical from
+ * call to call and for any order of the rows.
+ * x: row r, column c at x[r*ldx + c] (ldx >= K), n rows; y likewise with ldy, m rows; device f32 (NULL allowed for 0 rows).
+ * out [K] f64 (device): W1 per column over the finite values; n_used [2K] int64 (device, nullable): finite x values per column,
+ * then finite y values per column.  0 < K <= MMB_W1_MAX_K, 0 <= n, m <= 2^31 - 1, else MMB_EINVAL.  workspace: 256-byte aligned,
+ * mmb_wasserstein1d_workspace_bytes(n, m, K) bytes (0 for invalid sizes), else MMB_ENOMEM.
+ */
+#define MMB_W1_MAX_K 64
+size_t mmb_wasserstein1d_workspace_bytes(int n, int m, int K);
+int mmb_wasserstein1d(const float* x, int64_t ldx, int n, const float* y, int64_t ldy, int m, int K,
+                      double* out, int64_t* n_used, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * Source-state construction on the device (SURVEY.md §8f N3), so that a generation run needs no host data loader:
  *   sample_noise("GaussNoise") (mp/data/particle_clouds/utils.py:222-251): x ~ N(0,1) * scale, flavor ~ Categorical(cat_probs[5]),
  *   charge = +-1 (0 for photons / neutral hadrons), turned into the 8 tokens of physics_to_onehot + argmax

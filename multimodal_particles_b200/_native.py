@@ -81,7 +81,7 @@ class JumpSchedule(ctypes.Structure):
 _lib = None
 
 # name -> (restype, argtypes); lists every symbol include/mmbridge.h declares
-_vp, _i, _f, _sz, _u64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_float, ctypes.c_size_t, ctypes.c_uint64
+_vp, _i, _f, _sz, _u64, _i64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_float, ctypes.c_size_t, ctypes.c_uint64, ctypes.c_int64
 SIGNATURES = {
     "mmb_abi_version": (_i, []),
     "mmb_last_error": (ctypes.c_char_p, []),
@@ -107,6 +107,8 @@ SIGNATURES = {
     "mmb_validation_histograms": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _f, _i, _vp, _vp]),
     "mmb_jet_observables": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "mmb_jet_substructure": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _f, _vp, _vp, _vp]),
+    "mmb_wasserstein1d_workspace_bytes": (_sz, [_i, _i, _i]),
+    "mmb_wasserstein1d": (_i, [_vp, _i64, _i, _vp, _i64, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "mmb_sample_source": (_i, [_vp, _vp, _vp, _i, _i, _f, _vp, _vp, _u64, _u64, _vp]),
     "mmb_sample_bridges": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _f, _i, _vp, _vp, _u64, _u64, _i, _i, _vp, _vp, _vp]),
     "mmb_absorbing_sample": (_i, [_vp, _vp, _vp, _u64, _u64, _i, _i, _vp, _vp]),

@@ -785,6 +785,25 @@ int mmb_bridge_losses(const float* v, const float* logits, const float* x0, cons
                                 static_cast<cudaStream_t>(stream));
 }
 
+size_t mmb_wasserstein1d_workspace_bytes(int n, int m, int K) {
+    if (n < 0 || m < 0 || K < 1 || K > MMB_W1_MAX_K) return 0;
+    return wasserstein1d_workspace_bytes(n, m, K);
+}
+
+int mmb_wasserstein1d(const float* x, int64_t ldx, int n, const float* y, int64_t ldy, int m, int K,
+                      double* out, int64_t* n_used, void* workspace, size_t workspace_bytes, void* stream) {
+    if (K < 1 || K > MMB_W1_MAX_K) return fail(MMB_EINVAL, "mmb_wasserstein1d: K = %d outside 1..%d", K, MMB_W1_MAX_K);
+    if (n < 0 || m < 0) return fail(MMB_EINVAL, "mmb_wasserstein1d: negative size");
+    if (ldx < K || ldy < K) return fail(MMB_EINVAL, "mmb_wasserstein1d: row strides must be >= K = %d", K);
+    if ((!x && n > 0) || (!y && m > 0) || !out || !workspace) return fail(MMB_EINVAL, "mmb_wasserstein1d: null argument");
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(MMB_EINVAL, "mmb_wasserstein1d: workspace not 256-byte aligned");
+    const size_t need = wasserstein1d_workspace_bytes(n, m, K);
+    if (need == 0) return MMB_ECUDA;   // the size query failed and set the error text
+    if (workspace_bytes < need) return fail(MMB_ENOMEM, "mmb_wasserstein1d: workspace %zu B, needs %zu B", workspace_bytes, need);
+    return launch_wasserstein1d(x, ldx, n, y, ldy, m, K, out, reinterpret_cast<long long*>(n_used), workspace,
+                                static_cast<cudaStream_t>(stream));
+}
+
 // debug only (not part of include/mmbridge.h): phase timestamps of the tcgen05 generation kernel, see tools/tc_trace.py
 int mmb_debug_read_trace(long long* out, int n) { return tc_read_trace(out, n); }
 int mmb_debug_read_stack_trace(long long* out, int n) { return stack_read_trace(out, n); }

@@ -108,6 +108,11 @@ int launch_jet_observables(const float* x, const uint8_t* k, const uint8_t* mask
 int launch_jet_substructure(const float* x, const uint8_t* mask, const float* mean, const float* sd, int B, int N, float R, float beta,
                             float* out, int16_t* axes, cudaStream_t stream);
 
+// wasserstein.cu — per-column 1-D W1: key pre-pass, CUB radix sort per column, merge-path integration in fixed tiles
+size_t wasserstein1d_workspace_bytes(int n, int m, int K);   // 0 when the CUB size query fails
+int launch_wasserstein1d(const float* x, long long ldx, int n, const float* y, long long ldy, int m, int K, double* out, long long* n_used,
+                         void* workspace, cudaStream_t stream);
+
 int launch_sample_source(float* x, uint8_t* k, uint8_t* mask, int B, int N, float scale, const float* cat_probs, const float* mult_cdf,
                          uint64_t seed, uint64_t jet_offset, cudaStream_t stream);
 

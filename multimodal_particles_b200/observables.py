@@ -4,7 +4,9 @@
 multiplicity, jet charges, 1-D Wasserstein distance), SURVEY.md §8f N1.  One fused kernel (``mmb_jet_observables``) does the
 de-standardisation, ``tokens_to_physics``, the 4-momenta and the per-jet sums.  The clustering-based substructure (fastjet
 N-subjettiness on exclusive kt / WTA axes and D2, jets.py:204-240) is a second kernel (``mmb_jet_substructure``,
-``jet_substructure``); ``JetClassHighLevelFeatures.compute_substructure`` sets its columns.
+``jet_substructure``); ``JetClassHighLevelFeatures.compute_substructure`` sets its columns.  The 1-D Wasserstein distance the
+reference scores with (scipy.stats.wasserstein_distance, jets.py:329-332) is a third (``mmb_wasserstein1d``, ``wasserstein1d``,
+``JetClassHighLevelFeatures.wasserstein1d``).
 """
 import ctypes
 
@@ -56,6 +58,40 @@ def jet_substructure(x, mask_u8, stats=None, R=0.8, beta=1.0, want_axes=False):
         _native.check(_native.load().mmb_jet_substructure(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(R), float(beta),
                                                           _native._ptr(out), _native._ptr(axes), _native._stream()))
     return (out, axes) if want_axes else out
+
+
+def _rows(t):
+    """[n] or [n, K] f32 CUDA tensor -> ([n, K] view with unit column stride, row stride)."""
+    if t.dtype != torch.float32 or not t.is_cuda:
+        raise _native.MmbError("wasserstein1d takes float32 CUDA tensors; there is no CPU path")
+    t = t.reshape(-1, 1) if t.dim() == 1 else t
+    if t.stride(1) != 1 or (t.shape[0] > 1 and t.stride(0) < t.shape[1]):
+        t = t.contiguous()
+    return t, t.stride(0) if t.shape[0] > 1 else t.shape[1]
+
+
+def wasserstein1d(x, y, return_counts=False):
+    """x [n] or [n, K], y [m] or [m, K] f32 on the GPU -> W1 per column [K] f64 on the device (0-d for 1-D inputs): the
+    scipy.stats.wasserstein_distance of the finite values of each column, NaN when a sample has none (DESIGN.md §4.6c).
+    ``return_counts``: also the numbers of finite x and y values, [2, K] int64 ([2] for 1-D inputs)."""
+    one = x.dim() == 1
+    x2, ldx = _rows(x)
+    y2, ldy = _rows(y)
+    if x2.device != y2.device or x2.shape[1] != y2.shape[1]:
+        raise _native.MmbError(f"wasserstein1d: x {tuple(x.shape)} on {x.device} and y {tuple(y.shape)} on {y.device} do not match")
+    (n, K), m = x2.shape, y2.shape[0]
+    dev = x2.device
+    lib = _native.load()
+    with torch.cuda.device(dev):
+        need = lib.mmb_wasserstein1d_workspace_bytes(n, m, K)
+        ws = torch.empty(max(need, 256), dtype=torch.uint8, device=dev)
+        out = torch.empty(K, dtype=torch.float64, device=dev)
+        used = torch.empty(2, K, dtype=torch.int64, device=dev)
+        _native.check(lib.mmb_wasserstein1d(_native._ptr(x2) if n else None, ldx, n, _native._ptr(y2) if m else None, ldy, m, K,
+                                            _native._ptr(out), _native._ptr(used), _native._ptr(ws), ws.numel(), _native._stream()))
+    if one:
+        out, used = out[0], used[:, 0]
+    return (out, used) if return_counts else out
 
 
 class ParticleClouds:
@@ -145,6 +181,21 @@ class JetClassHighLevelFeatures:
         out = out[keep].to(c.continuous.device)
         for name in ("tau1", "tau2", "tau3", "tau21", "tau32", "d2"):
             setattr(self, name, out[:, SUBSTRUCTURE_COLUMNS.index(name)])
+
+    def wasserstein1d(self, reference, features=("pt", "m", "eta", "phi", "multiplicity", "Q_total", "Q_jet")):
+        """{feature: W1 between this sample and ``reference``} on the device (``wasserstein1d``), one host synchronisation;
+        the same values as ``Wassertein1D(feature, reference)``.  tau1, tau2, tau3, tau21, tau32 and d2 need
+        ``compute_substructure`` on both objects; they cover fewer jets, so features are grouped by length (one call each)."""
+        dev = self.pt.device if self.pt.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        col = lambda obj, f: getattr(obj, f).reshape(-1).to(dev, torch.float32)
+        groups = {}
+        for f in features:
+            groups.setdefault((getattr(self, f).numel(), getattr(reference, f).numel()), []).append(f)
+        names, values = [], []
+        for group in groups.values():
+            values.append(wasserstein1d(torch.stack([col(self, f) for f in group], 1), torch.stack([col(reference, f) for f in group], 1)))
+            names += group
+        return dict(zip(names, torch.cat(values).tolist()))
 
     def Wassertein1D(self, feature, reference):
         import scipy.stats

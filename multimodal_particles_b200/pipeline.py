@@ -9,8 +9,10 @@ per-GPU int64 counts.  Exchanges (SURVEY.md §8e): the packed micro-batch (1 792
 on a side stream under the next micro-batch's generation — pushed over NVLink peer memory by the copy engines
 (``sharding.PeerGather``; one NCCL all-gather where peer memory is unavailable) — and one all-reduce of the histograms and of the
 jet-observable sums at the end.  With ``substructure=True`` the side stream also runs ``mmb_jet_substructure`` on every micro-batch
-and histograms tau21, tau32 and D2 into int64 counts of their own (SUBSTRUCTURE_BINS).  The reference has no multi-GPU code (SURVEY.md §2.1); ``tools/million_jets.py`` and the
-multi-GPU arms of ``bench.py`` call this.
+and histograms tau21, tau32 and D2 into int64 counts of their own (SUBSTRUCTURE_BINS).  With ``w1_reference`` the side stream
+keeps the W1_COLUMNS of every jet; after the timed window they are all-gathered and scored against the reference with
+``mmb_wasserstein1d`` (``reference_observables`` builds an independent reference sample).  The reference has no multi-GPU code
+(SURVEY.md §2.1); ``tools/million_jets.py`` and the multi-GPU arms of ``bench.py`` call this.
 """
 import hashlib
 
@@ -19,7 +21,7 @@ import torch
 import torch.distributed as dist
 
 from . import sharding
-from .observables import SUBSTRUCTURE_COLUMNS, jet_observables, jet_substructure
+from .observables import JET_COLUMNS, SUBSTRUCTURE_COLUMNS, jet_observables, jet_substructure, wasserstein1d
 from .source import sample_source_state
 
 STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisation to a jet-like scale (pT > 0)
@@ -27,6 +29,30 @@ STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisatio
 # where the observable is undefined (NaN); counts layout [3][101]
 SUBSTRUCTURE_HISTS = (("tau21", 0.0, 1.0), ("tau32", 0.0, 1.0), ("d2", 0.0, 10.0))
 SUBSTRUCTURE_BINS = 100
+# jet-level columns scored by W1 against a reference sample; with substructure, W1_SUBSTRUCTURE_COLUMNS follow
+W1_COLUMNS = ("pt", "m", "eta", "phi", "multiplicity", "Q_total", "Q_jet")
+W1_SUBSTRUCTURE_COLUMNS = ("tau21", "tau32", "d2")
+
+
+def w1_columns(substructure=False):
+    return W1_COLUMNS + (W1_SUBSTRUCTURE_COLUMNS if substructure else ())
+
+
+def _w1_index(device):
+    """Device index tensors of W1_COLUMNS in jet_observables rows and of W1_SUBSTRUCTURE_COLUMNS in jet_substructure rows (made
+    once, so that picking the columns of a micro-batch copies nothing from the host)."""
+    return (torch.tensor([JET_COLUMNS.index(c) for c in W1_COLUMNS], device=device),
+            torch.tensor([SUBSTRUCTURE_COLUMNS.index(c) for c in W1_SUBSTRUCTURE_COLUMNS], device=device))
+
+
+def _w1_rows(jets, sub, index):
+    """[B, K] f32: the W1 columns of one micro-batch from its jet_observables (and jet_substructure) rows."""
+    rows = jets.index_select(1, index[0])
+    return rows if sub is None else torch.cat([rows, sub.index_select(1, index[1])], 1)
+
+
+def _target_multiplicity(N):
+    return np.clip(np.rint(np.random.default_rng(0).normal(45, 18, 20000)), 1, N).astype(int)     # JetClass-like multiplicities
 
 
 class SubstructureHistograms:
@@ -58,19 +84,28 @@ class SubstructureHistograms:
 
 
 def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_batch=4096, n_particles=128, precision="auto",
-                           warmup_batches=2, gather="auto", substructure=False):
+                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None):
     """-> dict (rank 0: the C5 record; other ranks: None).  Device time by CUDA events around the whole slice incl. the final
     all-reduce, max over ranks.  ``substructure``: also histogram tau21, tau32 and D2 of every jet (``substructure_sha1``,
-    ``substructure_counts`` and the means of the defined values join the record)."""
+    ``substructure_counts`` and the means of the defined values join the record).  ``w1_reference``: [m, K] f32 device tensor
+    of reference values of ``w1_columns(substructure)``; after the timed window the generated values of every jet are gathered
+    in jet order and ``w1`` ({column: W1}), ``w1_used`` ({column: [finite generated, finite reference]}),
+    ``w1_reference_jets`` and ``w1_seconds`` (CUDA events around the W1 call) join the record."""
     native = model.encoder.native_model(device)
     table = model.step_table()
     lo, hi = sharding.shard_range(total_jets, rank, world)
     MB, N = micro_batch, n_particles
-    mult_hist = np.clip(np.rint(np.random.default_rng(0).normal(45, 18, 20000)), 1, N).astype(int)     # JetClass-like multiplicities
+    mult_hist = _target_multiplicity(N)
     hist = sharding.ValidationHistograms(device, vocab_size=cfg.data.vocab_size_features)
     counts = torch.zeros(hist.size, dtype=torch.int64, device=device)
     jet_sums = torch.zeros(11, dtype=torch.float64, device=device)
     sub_hist = SubstructureHistograms(device) if substructure else None
+    w1_cols = w1_columns(substructure)
+    if w1_reference is not None:
+        if w1_reference.dim() != 2 or w1_reference.shape[1] != len(w1_cols):
+            raise ValueError(f"w1_reference must be [m, {len(w1_cols)}] ({', '.join(w1_cols)}), got {tuple(w1_reference.shape)}")
+        w1_buf = torch.empty(hi - lo, len(w1_cols), dtype=torch.float32, device=device)   # this rank's jets, in jet order
+        w1_index = _w1_index(device)
     packs = [sharding.PackedJets(MB, N, 3, device) for _ in range(3)]      # state of a micro-batch: [x | tokens | mask], one allocation
     recv = [sharding.make_gather(MB, N, 3, world, device, mode=gather) for _ in range(2)] if world > 1 else None
     side = torch.cuda.Stream(device=device)
@@ -97,8 +132,11 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
                 _, _, jets = jet_observables(x, k, m, STATS, want_particles=False)
                 counts.add_(hist.accumulate(x, k, m))
                 jet_sums.add_(torch.nan_to_num(jets.double()).sum(0))
+                sub = jet_substructure(x, m, STATS) if substructure else None
                 if substructure:
-                    sub_hist.add(jet_substructure(x, m, STATS))
+                    sub_hist.add(sub)
+                if w1_reference is not None:
+                    w1_buf[start - lo:start - lo + B].copy_(_w1_rows(jets, sub, w1_index))
                 if world > 1 and B == MB:
                     recv[i & 1].gather(pk)          # the packed micro-batch to every rank (copy-engine push, or one all-gather)
                 for t in (x, k, m):
@@ -129,6 +167,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     t = torch.tensor([s.elapsed_time(e)], dtype=torch.float64, device=device)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    if w1_reference is not None:
+        w1_all = _gather_rows(w1_buf, total_jets, world, device) if world > 1 else w1_buf
     if rank != 0:
         return None
     ms = float(t.item())
@@ -153,4 +193,51 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
             defined = int(per[i, :SUBSTRUCTURE_BINS].sum())
             rec[f"mean_{name}"] = float(sums[i] / defined) if defined else float("nan")
         rec["substructure_sha1"] = hashlib.sha1(sc.tobytes()).hexdigest()
+    if w1_reference is not None:
+        rec.update(_score_w1(w1_all, w1_reference.to(device, torch.float32), w1_cols))
     return rec
+
+
+def _gather_rows(buf, total, world, device):
+    """Every rank's [hi - lo, K] rows -> [total, K] in rank (= jet) order: padded to the largest shard, all-gathered, trimmed."""
+    sizes = [b - a for a, b in (sharding.shard_range(total, r, world) for r in range(world))]
+    S = max(sizes)
+    padded = torch.zeros(S, buf.shape[1], dtype=buf.dtype, device=device)
+    padded[:buf.shape[0]].copy_(buf)
+    out = torch.empty(world * S, buf.shape[1], dtype=buf.dtype, device=device)
+    dist.all_gather_into_tensor(out, padded)
+    return torch.cat([out[r * S:r * S + sizes[r]] for r in range(world)])
+
+
+def _score_w1(values, reference, cols):
+    stream = torch.cuda.current_stream(values.device)
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record(stream)
+    w1, used = wasserstein1d(values, reference, return_counts=True)
+    e.record(stream)
+    torch.cuda.synchronize(values.device)
+    w1, used = w1.tolist(), used.tolist()
+    return {"w1": dict(zip(cols, w1)), "w1_used": {c: [used[0][i], used[1][i]] for i, c in enumerate(cols)},
+            "w1_reference_jets": int(reference.shape[0]), "w1_seconds": s.elapsed_time(e) * 1e-3}
+
+
+def reference_observables(model, cfg, n_jets, device, n_particles=128, substructure=False, jet_offset=1 << 40, micro_batch=16384,
+                          precision="auto", stats=STATS):
+    """[n_jets, K] f32 on ``device``: the ``w1_columns(substructure)`` of ``n_jets`` jets made as ``sharded_generation_run`` makes
+    them (same model, source, solver, observables) but from the Philox jet offsets ``jet_offset + j``, disjoint from any run's
+    [0, total), so the sample is independent of it.  W1 between two such samples is the seed-to-seed noise floor.  ``stats``:
+    the de-standardisation of the observables."""
+    native = model.encoder.native_model(device)
+    table = model.step_table()
+    N = n_particles
+    mult_hist = _target_multiplicity(N)
+    out = torch.empty(n_jets, len(w1_columns(substructure)), dtype=torch.float32, device=device)
+    index = _w1_index(device)
+    for start in range(0, n_jets, micro_batch):
+        B = min(micro_batch, n_jets - start)
+        x, k, m = sample_source_state(B, N, target_multiplicity=mult_hist, min_num_particles=0, device=device, seed=7,
+                                      jet_offset=jet_offset + start, compact=True)
+        native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start, precision=precision)
+        _, _, jets = jet_observables(x, k, m, stats, want_particles=False)
+        out[start:start + B] = _w1_rows(jets, jet_substructure(x, m, stats) if substructure else None, index)
+    return out

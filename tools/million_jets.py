@@ -1,14 +1,17 @@
 """BASELINE config 5: a 1 M-jet generation run sharded over the GPUs of one box (multimodal_particles_b200/pipeline.py).
 
-    python tools/million_jets.py [--jets 1048576] [--substructure]                           # one GPU
+    python tools/million_jets.py [--jets 1048576] [--substructure] [--w1-reference-jets M | --w1-reference FILE.npz] [--out F]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/million_jets.py
 
-Prints one JSON line on rank 0 (device time by CUDA events, max over ranks; `histogram_sha1` is the same for every GPU count)."""
+Prints one JSON line on rank 0 (device time by CUDA events, max over ranks; `histogram_sha1` is the same for every GPU count).
+With a W1 reference — M jets built by `pipeline.reference_observables` from disjoint Philox streams, or one array per column
+of `pipeline.w1_columns` in an .npz file — the record also holds the W1 of every column against it (`w1`, `w1_seconds`)."""
 import argparse
 import json
 import os
 import sys
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -16,7 +19,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench  # noqa: E402
-from multimodal_particles_b200.pipeline import sharded_generation_run  # noqa: E402
+from multimodal_particles_b200.pipeline import reference_observables, sharded_generation_run, w1_columns  # noqa: E402
 
 
 def main():
@@ -25,6 +28,9 @@ def main():
     ap.add_argument("--micro-batch", type=int, default=16384)
     ap.add_argument("--precision", default="auto")
     ap.add_argument("--substructure", action="store_true", help="also histogram tau21, tau32 and D2 of every jet on the device")
+    ap.add_argument("--w1-reference-jets", type=int, default=0, help="score W1 against an independent reference sample of this size")
+    ap.add_argument("--w1-reference", default=None, help="score W1 against this .npz (one array per column name)")
+    ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     args = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     torch.cuda.set_device(local)
@@ -32,10 +38,21 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     cfg, model = bench.build_model(dev)
+    reference = None
+    if args.w1_reference:
+        with np.load(args.w1_reference) as f:
+            reference = torch.from_numpy(np.stack([f[c].astype(np.float32).reshape(-1) for c in w1_columns(args.substructure)], 1)).to(dev)
+    elif args.w1_reference_jets > 0:
+        reference = reference_observables(model, cfg, args.w1_reference_jets, dev, n_particles=bench.N_PART,
+                                          substructure=args.substructure, micro_batch=args.micro_batch, precision=args.precision)
     rec = sharded_generation_run(model, cfg, args.jets, rank, world, dev, micro_batch=args.micro_batch, n_particles=bench.N_PART,
-                                 precision=args.precision, substructure=args.substructure)
+                                 precision=args.precision, substructure=args.substructure, w1_reference=reference)
     if rank == 0:
-        print(json.dumps(rec))
+        line = json.dumps(rec)
+        print(line)
+        if args.out:
+            with open(args.out, "w") as f:
+                f.write(line + "\n")
     if world > 1:
         dist.destroy_process_group()
 
