@@ -522,6 +522,51 @@ int mmb_wasserstein1d(const float* x, int64_t ldx, int n, const float* y, int64_
                       double* out, int64_t* n_used, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * Energy flow polynomials of a generated batch (the features of the W1-EFP, FPD and KPD metrics, arXiv:2211.10295, as JetNet
+ * computes them with energyflow: hadronic measure, kappa = 1, normalised energies):
+ *   constituents as for mmb_jet_substructure ((x * std + mean) in fp32, massless, y = eta; used iff mask != 0 && pt > 0);
+ *   z_i = pt_i / sum_j pt_j over the used particles, theta_ij = dR_ij^beta (dphi wrapped into [-pi, pi]), theta_ii = 0;
+ *   EFP_G = sum over all index tuples (coincident indices included) of z_i1 ... z_iV prod_{(a,b) in G} theta_{ia ib}.
+ * With s_i = sum_j z_j theta_ij, q_i = sum_j z_j theta_ij^2 and M = Theta diag(z) Theta, the columns are
+ *   EFP_1            one edge                          sum_i z_i s_i
+ *   EFP_4_SQUARE     4-cycle                           sum_{i,k} z_i z_k M_ik^2
+ *   EFP_4_PAW        triangle plus pendant             sum_i z_i s_i sum_k z_k theta_ik M_ik
+ *   EFP_4_PATH_MID2  3-edge path, middle edge doubled  sum_{j,k} z_j z_k s_j theta_jk^2 s_k
+ *   EFP_4_PATH_END2  3-edge path, end edge doubled     sum_{j,k} z_j z_k q_j theta_jk s_k
+ *   EFP_4_STAR2      3-star, one edge doubled          sum_i z_i q_i s_i^2
+ * (the last five are every connected multigraph with 4 vertices and 4 edges).  theta and M are fp32, every sum fp64.
+ * A jet with no used particle gets NaN in every column (one used particle: 0).
+ * x [B,N,3] f32, mask [B,N] u8, N <= MMB_SUB_MAX_N (larger N: MMB_EINVAL); beta > 0.  out [B][MMB_EFP_OBS] f32.
+ * Bit-identical from call to call.
+ */
+enum { MMB_EFP_1 = 0, MMB_EFP_4_SQUARE, MMB_EFP_4_PAW, MMB_EFP_4_PATH_MID2, MMB_EFP_4_PATH_END2, MMB_EFP_4_STAR2, MMB_EFP_OBS };
+int mmb_energy_flow_polynomials(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N, float beta,
+                                float* out, void* stream);
+
+/*
+ * Sample statistics of the Frechet and kernel physics distances (FPD, KPD; arXiv:2211.10295) over rows the caller draws:
+ * x: row r, column c at x[r*ldx + c] (ldx >= d), n rows, device f32; every value is used as x * scale[c] in fp64 (scale: device
+ * f32 [d], NULL for 1).  Row indices are device int32 in [0, n) (not checked).  0 < d <= MMB_MET_MAX_D.
+ *
+ * mmb_sampled_moments: for each draw t, over the rows idx[t][0..rows): sum[t][a] = sum x_a, sumsq[t][a][b] = sum x_a x_b
+ * (both triangles written), fp64 on the device.  draws > 0, rows > 0.
+ *
+ * mmb_kpd_mmd: for each batch t, with r_i = real[idx_real[t][i]], g_j = gen[idx_gen[t][j]] (i, j < B) and
+ * k(u, v) = (u . v / d + 1)^degree, the unbiased MMD^2
+ *   out[t] = (sum_{i != j} k(r_i, r_j) + sum_{i != j} k(g_i, g_j)) / (B (B - 1)) - 2 sum_{i,j} k(r_i, g_j) / B^2,
+ * dot products, powers and sums in fp64.  batches in 1..65535, B >= 2, degree >= 1.  workspace: 256-byte aligned,
+ * mmb_kpd_mmd_workspace_bytes(batches, B, d) bytes (0 for invalid sizes), else MMB_ENOMEM.
+ * Both are stream-ordered, allocate nothing and are bit-identical from call to call.
+ */
+#define MMB_MET_MAX_D 64
+int mmb_sampled_moments(const float* x, int64_t ldx, int n, int d, const float* scale, const int32_t* idx, int draws, int rows,
+                        double* sum, double* sumsq, void* stream);
+size_t mmb_kpd_mmd_workspace_bytes(int batches, int B, int d);
+int mmb_kpd_mmd(const float* real, int64_t ldr, int n, const float* gen, int64_t ldg, int m, int d, const float* scale,
+                const int32_t* idx_real, const int32_t* idx_gen, int batches, int B, int degree, double* out, void* workspace,
+                size_t workspace_bytes, void* stream);
+
+/*
  * Source-state construction on the device (SURVEY.md §8f N3), so that a generation run needs no host data loader:
  *   sample_noise("GaussNoise") (mp/data/particle_clouds/utils.py:222-251): x ~ N(0,1) * scale, flavor ~ Categorical(cat_probs[5]),
  *   charge = +-1 (0 for photons / neutral hadrons), turned into the 8 tokens of physics_to_onehot + argmax

@@ -804,6 +804,47 @@ int mmb_wasserstein1d(const float* x, int64_t ldx, int n, const float* y, int64_
                                 static_cast<cudaStream_t>(stream));
 }
 
+int mmb_energy_flow_polynomials(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N, float beta,
+                                float* out, void* stream) {
+    if (!x || !mask || !out) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials: null argument");
+    if ((mean == nullptr) != (std == nullptr)) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials: mean and std go together");
+    if (B < 0 || N < 0) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials: negative size");
+    if (N > MMB_SUB_MAX_N) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials: N = %d exceeds %d particle slots", N, MMB_SUB_MAX_N);
+    if (!(beta > 0.0f)) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials: beta must be positive");
+    if (B == 0) return MMB_OK;
+    return launch_energy_flow_polynomials(x, mask, mean, std, B, N, beta, out, static_cast<cudaStream_t>(stream));
+}
+
+int mmb_sampled_moments(const float* x, int64_t ldx, int n, int d, const float* scale, const int32_t* idx, int draws, int rows,
+                        double* sum, double* sumsq, void* stream) {
+    if (d < 1 || d > MMB_MET_MAX_D) return fail(MMB_EINVAL, "mmb_sampled_moments: d = %d outside 1..%d", d, MMB_MET_MAX_D);
+    if (n < 1 || draws < 1 || rows < 1) return fail(MMB_EINVAL, "mmb_sampled_moments: n, draws and rows must be positive");
+    if (ldx < d) return fail(MMB_EINVAL, "mmb_sampled_moments: row stride must be >= d = %d", d);
+    if (!x || !idx || !sum || !sumsq) return fail(MMB_EINVAL, "mmb_sampled_moments: null argument");
+    return launch_sampled_moments(x, ldx, d, scale, idx, draws, rows, sum, sumsq, static_cast<cudaStream_t>(stream));
+}
+
+static bool kpd_sizes_ok(int batches, int B, int d) { return batches >= 1 && batches <= 65535 && B >= 2 && d >= 1 && d <= MMB_MET_MAX_D; }
+
+size_t mmb_kpd_mmd_workspace_bytes(int batches, int B, int d) {
+    return kpd_sizes_ok(batches, B, d) ? kpd_mmd_workspace_bytes(batches, B, d) : 0;
+}
+
+int mmb_kpd_mmd(const float* real, int64_t ldr, int n, const float* gen, int64_t ldg, int m, int d, const float* scale,
+                const int32_t* idx_real, const int32_t* idx_gen, int batches, int B, int degree, double* out, void* workspace,
+                size_t workspace_bytes, void* stream) {
+    if (!kpd_sizes_ok(batches, B, d))
+        return fail(MMB_EINVAL, "mmb_kpd_mmd: batches = %d, B = %d, d = %d (need 1..65535, >= 2, 1..%d)", batches, B, d, MMB_MET_MAX_D);
+    if (n < 1 || m < 1 || degree < 1) return fail(MMB_EINVAL, "mmb_kpd_mmd: n, m and degree must be positive");
+    if (ldr < d || ldg < d) return fail(MMB_EINVAL, "mmb_kpd_mmd: row strides must be >= d = %d", d);
+    if (!real || !gen || !idx_real || !idx_gen || !out || !workspace) return fail(MMB_EINVAL, "mmb_kpd_mmd: null argument");
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(MMB_EINVAL, "mmb_kpd_mmd: workspace not 256-byte aligned");
+    const size_t need = kpd_mmd_workspace_bytes(batches, B, d);
+    if (workspace_bytes < need) return fail(MMB_ENOMEM, "mmb_kpd_mmd: workspace %zu B, needs %zu B", workspace_bytes, need);
+    return launch_kpd_mmd(real, ldr, gen, ldg, d, scale, idx_real, idx_gen, batches, B, degree, out, workspace,
+                          static_cast<cudaStream_t>(stream));
+}
+
 // debug only (not part of include/mmbridge.h): phase timestamps of the tcgen05 generation kernel, see tools/tc_trace.py
 int mmb_debug_read_trace(long long* out, int n) { return tc_read_trace(out, n); }
 int mmb_debug_read_stack_trace(long long* out, int n) { return stack_read_trace(out, n); }

@@ -113,6 +113,17 @@ size_t wasserstein1d_workspace_bytes(int n, int m, int K);   // 0 when the CUB s
 int launch_wasserstein1d(const float* x, long long ldx, int n, const float* y, long long ldy, int m, int K, double* out, long long* n_used,
                          void* workspace, cudaStream_t stream);
 
+// efp.cu — energy flow polynomials, one block per jet, Theta as an upper triangle of 32 x 32 blocks in shared memory
+int launch_energy_flow_polynomials(const float* x, const uint8_t* mask, const float* mean, const float* sd, int B, int N, float beta,
+                                   float* out, cudaStream_t stream);
+
+// jet_metrics.cu — FPD moments over drawn rows, KPD unbiased MMD^2 over row strips with fixed-order partials
+int launch_sampled_moments(const float* x, long long ldx, int d, const float* scale, const int* idx, int draws, int rows, double* sum,
+                           double* sumsq, cudaStream_t stream);
+size_t kpd_mmd_workspace_bytes(int batches, int B, int d);
+int launch_kpd_mmd(const float* real, long long ldr, const float* gen, long long ldg, int d, const float* scale, const int* idx_real,
+                   const int* idx_gen, int batches, int B, int degree, double* out, void* workspace, cudaStream_t stream);
+
 int launch_sample_source(float* x, uint8_t* k, uint8_t* mask, int B, int N, float scale, const float* cat_probs, const float* mult_cdf,
                          uint64_t seed, uint64_t jet_offset, cudaStream_t stream);
 

@@ -6,7 +6,9 @@ de-standardisation, ``tokens_to_physics``, the 4-momenta and the per-jet sums.  
 N-subjettiness on exclusive kt / WTA axes and D2, jets.py:204-240) is a second kernel (``mmb_jet_substructure``,
 ``jet_substructure``); ``JetClassHighLevelFeatures.compute_substructure`` sets its columns.  The 1-D Wasserstein distance the
 reference scores with (scipy.stats.wasserstein_distance, jets.py:329-332) is a third (``mmb_wasserstein1d``, ``wasserstein1d``,
-``JetClassHighLevelFeatures.wasserstein1d``).
+``JetClassHighLevelFeatures.wasserstein1d``).  The energy flow polynomials of the JetNet metrics (arXiv:2211.10295) are a fourth
+(``mmb_energy_flow_polynomials``, ``energy_flow_polynomials``, ``JetClassHighLevelFeatures.compute_efps``); ``fpd`` and ``kpd``
+score them with the sample statistics of ``mmb_sampled_moments`` and ``mmb_kpd_mmd``.
 """
 import ctypes
 
@@ -92,6 +94,156 @@ def wasserstein1d(x, y, return_counts=False):
     if one:
         out, used = out[0], used[:, 0]
     return (out, used) if return_counts else out
+
+
+# energy flow polynomials (DESIGN.md §4.6d): the d = 1 EFP, then the five connected multigraphs with 4 vertices and 4 edges, the
+# set JetNet's efps / w1efp use by default (("n==", 4), ("d==", 4), ("p==", 1)); W1-EFP, FPD and KPD score EFP_COLUMNS[1:]
+EFP_COLUMNS = ("efp1", "efp4_square", "efp4_paw", "efp4_path_mid2", "efp4_path_end2", "efp4_star2")
+# conventions of the JetNet metrics (arXiv:2211.10295), each in one place
+EFP_BETA = 1.0                               # theta = dR^beta, hadronic measure, kappa = 1, normalised energies
+KPD_DEGREE = 4                               # k(x, y) = (x . y / d + 1)^degree: gamma = 1 / d, c = 1
+KPD_ERROR_RANGE = (16.275, 83.725)           # KPD error: half of this percentile range of the per-batch values
+
+
+def energy_flow_polynomials(x, mask_u8, stats=None, beta=EFP_BETA):
+    """x [B,N,3] f32 (pt, eta, phi; standardised when ``stats`` is given), mask [B,N] u8 on the GPU, N <= 256 -> [B,6] f32 in the
+    order of ``EFP_COLUMNS``.  Jets with no used particle (mask and pt > 0) are NaN; jets with one are 0."""
+    _native._require_cuda(x, mask_u8)
+    B, N, _ = x.shape
+    dev = x.device
+    out = torch.empty(B, len(EFP_COLUMNS), dtype=torch.float32, device=dev)
+    mean = std = None
+    if stats is not None:
+        mean = (ctypes.c_float * 3)(*[float(v) for v in stats["mean"][:3]])
+        std = (ctypes.c_float * 3)(*[float(v) for v in stats["std"][:3]])
+    with torch.cuda.device(dev):
+        _native.check(_native.load().mmb_energy_flow_polynomials(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(beta),
+                                                                 _native._ptr(out), _native._stream()))
+    return out
+
+
+def _metric_rows(t, name):
+    if t.dim() != 2 or t.dtype != torch.float32 or not t.is_cuda:
+        raise _native.MmbError(f"{name} takes [n, d] float32 CUDA tensors; there is no CPU path")
+    if t.shape[1] > 64:
+        raise _native.MmbError(f"{name}: d = {t.shape[1]} exceeds 64 features")
+    if t.stride(1) != 1 or (t.shape[0] > 1 and t.stride(0) < t.shape[1]):
+        t = t.contiguous()
+    return t, t.stride(0) if t.shape[0] > 1 else t.shape[1]
+
+
+def _index(idx):
+    return idx.to(torch.int32).contiguous()
+
+
+def sampled_moments(x, idx, scale=None):
+    """x [n, d] f32, idx [draws, rows] (row indices) on the GPU -> (sum [draws, d], sum of x x^T [draws, d, d]) in f64 on the
+    device, every value taken as x * scale (``scale`` [d] f32, None for 1; the product is exact in fp64)."""
+    x2, ldx = _metric_rows(x, "sampled_moments")
+    (n, d), (draws, rows) = x2.shape, idx.shape
+    idx = _index(idx)
+    sums = torch.empty(draws, d, dtype=torch.float64, device=x2.device)
+    sumsq = torch.empty(draws, d, d, dtype=torch.float64, device=x2.device)
+    with torch.cuda.device(x2.device):
+        _native.check(_native.load().mmb_sampled_moments(_native._ptr(x2), ldx, n, d, _native._ptr(scale), _native._ptr(idx), draws, rows,
+                                                         _native._ptr(sums), _native._ptr(sumsq), _native._stream()))
+    return sums, sumsq
+
+
+def _mean_cov(sums, sumsq, rows):
+    mu = sums / rows
+    return mu, (sumsq - rows * mu[:, :, None] * mu[:, None, :]) / (rows - 1)
+
+
+def frechet_distances(real, gen, idx_real, idx_gen, scale=None):
+    """Per draw t: the Frechet distance between Gaussians fitted (mean, unbiased covariance) to real[idx_real[t]] and
+    gen[idx_gen[t]], ||mu1 - mu2||^2 + Tr S1 + Tr S2 - 2 sum_i sqrt(max(l_i, 0)) with l the eigenvalues of S1^1/2 S2 S1^1/2
+    (batched fp64 eigh on the device) -> [draws] f64 on the device."""
+    m1, c1 = _mean_cov(*sampled_moments(real, idx_real, scale), idx_real.shape[1])
+    m2, c2 = _mean_cov(*sampled_moments(gen, idx_gen, scale), idx_gen.shape[1])
+    return _frechet(m1, c1, m2, c2)
+
+
+def _frechet(m1, c1, m2, c2):
+    w, v = torch.linalg.eigh(c1)
+    root = (v * w.clamp(min=0).sqrt()[:, None, :]) @ v.transpose(1, 2)
+    lam = torch.linalg.eigvalsh(root @ c2 @ root)
+    diff = m1 - m2
+    return (diff * diff).sum(1) + c1.diagonal(dim1=1, dim2=2).sum(1) + c2.diagonal(dim1=1, dim2=2).sum(1) - 2 * lam.clamp(min=0).sqrt().sum(1)
+
+
+def kpd_mmd(real, gen, idx_real, idx_gen, scale=None, degree=KPD_DEGREE):
+    """Per batch t: the unbiased MMD^2 between real[idx_real[t]] and gen[idx_gen[t]] (B rows each) with the polynomial kernel
+    k(x, y) = (x . y / d + 1)^degree, in fp64 -> [batches] f64 on the device."""
+    r2, ldr = _metric_rows(real, "kpd_mmd")
+    g2, ldg = _metric_rows(gen, "kpd_mmd")
+    if r2.shape[1] != g2.shape[1] or r2.device != g2.device or idx_real.shape != idx_gen.shape:
+        raise _native.MmbError(f"kpd_mmd: real {tuple(real.shape)}, gen {tuple(gen.shape)}, indices {tuple(idx_real.shape)} / "
+                               f"{tuple(idx_gen.shape)} do not match")
+    (n, d), m = r2.shape, g2.shape[0]
+    batches, B = idx_real.shape
+    lib = _native.load()
+    ir, ig = _index(idx_real), _index(idx_gen)
+    with torch.cuda.device(r2.device):
+        need = lib.mmb_kpd_mmd_workspace_bytes(batches, B, d)
+        ws = torch.empty(max(need, 256), dtype=torch.uint8, device=r2.device)
+        out = torch.empty(batches, dtype=torch.float64, device=r2.device)
+        _native.check(lib.mmb_kpd_mmd(_native._ptr(r2), ldr, n, _native._ptr(g2), ldg, m, d, _native._ptr(scale), _native._ptr(ir),
+                                      _native._ptr(ig), batches, B, int(degree), _native._ptr(out), _native._ptr(ws), ws.numel(),
+                                      _native._stream()))
+    return out
+
+
+def _finite_rows_and_scale(real, gen, normalise):
+    """Drops the rows with a non-finite value (one host synchronisation each) and returns the per-column scale 1 / max|real|
+    (None without ``normalise``; 1 where a column of real is all zero)."""
+    real, gen = [t[torch.isfinite(t).all(1)].to(torch.float32).contiguous() for t in (real, gen)]
+    if len(real) == 0 or len(gen) == 0:
+        raise ValueError("fpd / kpd: a sample has no row without a non-finite value")
+    scale = None
+    if normalise:
+        top = real.abs().amax(0)
+        scale = torch.where(top > 0, 1.0 / top, torch.ones_like(top)).contiguous()
+    return real, gen, scale
+
+
+def _generator(device, seed):
+    return torch.Generator(device=device).manual_seed(seed)
+
+
+def fpd(real, gen, min_samples=20_000, max_samples=50_000, num_batches=20, num_points=10, normalise=True, seed=42):
+    """Frechet physics distance (arXiv:2211.10295, JetNet's ``fpd``) of two [n, d] f32 CUDA feature samples -> (value, error).
+    For each of ``num_points`` sample sizes N = int(1 / linspace(1 / min_samples, 1 / max_samples)), ``num_batches`` draws with
+    replacement of N rows of each sample (seeded device generator); the Frechet distances are averaged per size and
+    ``a + b / N`` (a, b >= 0) is fitted; the value is ``a`` and the error the fit's standard error of ``a``.  The host waits only
+    to drop non-finite rows and for the 10 averages (the eigendecompositions of all draws run in one batch)."""
+    from scipy.optimize import curve_fit
+    real, gen, scale = _finite_rows_and_scale(real, gen, normalise)
+    sizes = (1 / np.linspace(1.0 / min_samples, 1.0 / max_samples, num_points)).astype("int32")
+    g = _generator(real.device, seed)
+    mom = []
+    for N in sizes:
+        N = int(N)
+        ir = torch.randint(len(real), (num_batches, N), generator=g, device=real.device, dtype=torch.int32)
+        ig = torch.randint(len(gen), (num_batches, N), generator=g, device=real.device, dtype=torch.int32)
+        mom.append(_mean_cov(*sampled_moments(real, ir, scale), N) + _mean_cov(*sampled_moments(gen, ig, scale), N))
+    m1, c1, m2, c2 = [torch.cat([p[i] for p in mom]) for i in range(4)]
+    vals = _frechet(m1, c1, m2, c2).reshape(num_points, num_batches).mean(1).cpu().numpy()
+    params, covs = curve_fit(lambda x, a, b: a + b * x, 1 / sizes, vals, bounds=([0, 0], [np.inf, np.inf]))
+    return float(params[0]), float(np.sqrt(np.diag(covs)[0]))
+
+
+def kpd(real, gen, num_batches=10, batch_size=5000, degree=KPD_DEGREE, normalise=True, seed=42):
+    """Kernel physics distance (arXiv:2211.10295, JetNet's ``kpd``) of two [n, d] f32 CUDA feature samples -> (median, error):
+    the unbiased MMD^2 with the polynomial kernel over ``num_batches`` draws with replacement of ``batch_size`` rows of each
+    sample (seeded device generator), its median and half of its KPD_ERROR_RANGE percentile range."""
+    real, gen, scale = _finite_rows_and_scale(real, gen, normalise)
+    g = _generator(real.device, seed)
+    ir = torch.randint(len(real), (num_batches, batch_size), generator=g, device=real.device, dtype=torch.int32)
+    ig = torch.randint(len(gen), (num_batches, batch_size), generator=g, device=real.device, dtype=torch.int32)
+    vals = kpd_mmd(real, gen, ir, ig, scale, degree).cpu().numpy()
+    lo, hi = np.percentile(vals, KPD_ERROR_RANGE)
+    return float(np.median(vals)), float((hi - lo) / 2)
 
 
 class ParticleClouds:
@@ -181,6 +333,17 @@ class JetClassHighLevelFeatures:
         out = out[keep].to(c.continuous.device)
         for name in ("tau1", "tau2", "tau3", "tau21", "tau32", "d2"):
             setattr(self, name, out[:, SUBSTRUCTURE_COLUMNS.index(name)])
+
+    def compute_efps(self, beta=EFP_BETA):
+        """Energy flow polynomials on the device (``energy_flow_polynomials``) from the physical constituents: sets the six
+        attributes of ``EFP_COLUMNS`` over the jets with at least one used particle, so that
+        ``wasserstein1d(reference, EFP_COLUMNS[1:])`` is W1-EFP and ``Wassertein1D("efp4_square", other)`` compares one."""
+        c = self.constituents
+        dev = c.continuous.device if c.continuous.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        out = energy_flow_polynomials(c.continuous.to(dev, torch.float32).contiguous(), as_u8(c.mask.to(dev)), None, beta)
+        out = out[~torch.isnan(out[:, 0])].to(c.continuous.device)
+        for i, name in enumerate(EFP_COLUMNS):
+            setattr(self, name, out[:, i])
 
     def wasserstein1d(self, reference, features=("pt", "m", "eta", "phi", "multiplicity", "Q_total", "Q_jet")):
         """{feature: W1 between this sample and ``reference``} on the device (``wasserstein1d``), one host synchronisation;

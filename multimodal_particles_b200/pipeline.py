@@ -11,7 +11,9 @@ on a side stream under the next micro-batch's generation — pushed over NVLink 
 jet-observable sums at the end.  With ``substructure=True`` the side stream also runs ``mmb_jet_substructure`` on every micro-batch
 and histograms tau21, tau32 and D2 into int64 counts of their own (SUBSTRUCTURE_BINS).  With ``w1_reference`` the side stream
 keeps the W1_COLUMNS of every jet; after the timed window they are all-gathered and scored against the reference with
-``mmb_wasserstein1d`` (``reference_observables`` builds an independent reference sample).  The reference has no multi-GPU code
+``mmb_wasserstein1d`` (``reference_observables`` builds an independent reference sample).  With ``efp=True`` the side stream
+also runs ``mmb_energy_flow_polynomials``; their columns join the W1 columns, and with a reference the five d = 4 EFPs are also
+scored by FPD and KPD (``observables.fpd`` / ``kpd``) after the timed window.  The reference has no multi-GPU code
 (SURVEY.md §2.1); ``tools/million_jets.py`` and the multi-GPU arms of ``bench.py`` call this.
 """
 import hashlib
@@ -21,7 +23,8 @@ import torch
 import torch.distributed as dist
 
 from . import sharding
-from .observables import JET_COLUMNS, SUBSTRUCTURE_COLUMNS, jet_observables, jet_substructure, wasserstein1d
+from .observables import (EFP_COLUMNS, JET_COLUMNS, SUBSTRUCTURE_COLUMNS, energy_flow_polynomials, fpd, jet_observables, jet_substructure,
+                          kpd, wasserstein1d)
 from .source import sample_source_state
 
 STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisation to a jet-like scale (pT > 0)
@@ -29,13 +32,14 @@ STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisatio
 # where the observable is undefined (NaN); counts layout [3][101]
 SUBSTRUCTURE_HISTS = (("tau21", 0.0, 1.0), ("tau32", 0.0, 1.0), ("d2", 0.0, 10.0))
 SUBSTRUCTURE_BINS = 100
-# jet-level columns scored by W1 against a reference sample; with substructure, W1_SUBSTRUCTURE_COLUMNS follow
+# jet-level columns scored by W1 against a reference sample; with substructure, W1_SUBSTRUCTURE_COLUMNS follow, then with efp
+# EFP_COLUMNS (FPD and KPD score EFP_COLUMNS[1:], the five d = 4 EFPs)
 W1_COLUMNS = ("pt", "m", "eta", "phi", "multiplicity", "Q_total", "Q_jet")
 W1_SUBSTRUCTURE_COLUMNS = ("tau21", "tau32", "d2")
 
 
-def w1_columns(substructure=False):
-    return W1_COLUMNS + (W1_SUBSTRUCTURE_COLUMNS if substructure else ())
+def w1_columns(substructure=False, efp=False):
+    return W1_COLUMNS + (W1_SUBSTRUCTURE_COLUMNS if substructure else ()) + (EFP_COLUMNS if efp else ())
 
 
 def _w1_index(device):
@@ -45,10 +49,11 @@ def _w1_index(device):
             torch.tensor([SUBSTRUCTURE_COLUMNS.index(c) for c in W1_SUBSTRUCTURE_COLUMNS], device=device))
 
 
-def _w1_rows(jets, sub, index):
-    """[B, K] f32: the W1 columns of one micro-batch from its jet_observables (and jet_substructure) rows."""
-    rows = jets.index_select(1, index[0])
-    return rows if sub is None else torch.cat([rows, sub.index_select(1, index[1])], 1)
+def _w1_rows(jets, sub, index, efps=None):
+    """[B, K] f32: the W1 columns of one micro-batch from its jet_observables (and jet_substructure, energy_flow_polynomials)
+    rows."""
+    rows = [jets.index_select(1, index[0])] + ([sub.index_select(1, index[1])] if sub is not None else []) + ([efps] if efps is not None else [])
+    return rows[0] if len(rows) == 1 else torch.cat(rows, 1)
 
 
 def _target_multiplicity(N):
@@ -84,13 +89,16 @@ class SubstructureHistograms:
 
 
 def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_batch=4096, n_particles=128, precision="auto",
-                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None):
+                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None, efp=False):
     """-> dict (rank 0: the C5 record; other ranks: None).  Device time by CUDA events around the whole slice incl. the final
     all-reduce, max over ranks.  ``substructure``: also histogram tau21, tau32 and D2 of every jet (``substructure_sha1``,
     ``substructure_counts`` and the means of the defined values join the record).  ``w1_reference``: [m, K] f32 device tensor
     of reference values of ``w1_columns(substructure)``; after the timed window the generated values of every jet are gathered
     in jet order and ``w1`` ({column: W1}), ``w1_used`` ({column: [finite generated, finite reference]}),
-    ``w1_reference_jets`` and ``w1_seconds`` (CUDA events around the W1 call) join the record."""
+    ``w1_reference_jets`` and ``w1_seconds`` (CUDA events around the W1 call) join the record.  ``efp``: also compute the
+    energy flow polynomials of every jet (the means of the defined values join the record as ``mean_efp1`` ...); their
+    columns follow in ``w1_columns(substructure, efp)``, and with a reference ``fpd`` and ``kpd`` ([value, error] of the five
+    d = 4 EFPs against the reference's) and ``jet_metrics_seconds`` (CUDA events around both) join the record too."""
     native = model.encoder.native_model(device)
     table = model.step_table()
     lo, hi = sharding.shard_range(total_jets, rank, world)
@@ -100,7 +108,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     counts = torch.zeros(hist.size, dtype=torch.int64, device=device)
     jet_sums = torch.zeros(11, dtype=torch.float64, device=device)
     sub_hist = SubstructureHistograms(device) if substructure else None
-    w1_cols = w1_columns(substructure)
+    efp_sums = torch.zeros(len(EFP_COLUMNS) + 1, dtype=torch.float64, device=device) if efp else None   # sums, then defined jets
+    w1_cols = w1_columns(substructure, efp)
     if w1_reference is not None:
         if w1_reference.dim() != 2 or w1_reference.shape[1] != len(w1_cols):
             raise ValueError(f"w1_reference must be [m, {len(w1_cols)}] ({', '.join(w1_cols)}), got {tuple(w1_reference.shape)}")
@@ -135,8 +144,12 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
                 sub = jet_substructure(x, m, STATS) if substructure else None
                 if substructure:
                     sub_hist.add(sub)
+                efps = energy_flow_polynomials(x, m, STATS) if efp else None
+                if efp:
+                    defined = ~torch.isnan(efps[:, :1])
+                    efp_sums.add_(torch.cat([torch.where(defined, efps, 0.0).double().sum(0), defined.double().sum(0)]))
                 if w1_reference is not None:
-                    w1_buf[start - lo:start - lo + B].copy_(_w1_rows(jets, sub, w1_index))
+                    w1_buf[start - lo:start - lo + B].copy_(_w1_rows(jets, sub, w1_index, efps))
                 if world > 1 and B == MB:
                     recv[i & 1].gather(pk)          # the packed micro-batch to every rank (copy-engine push, or one all-gather)
                 for t in (x, k, m):
@@ -150,6 +163,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     jet_sums.zero_()
     if substructure:
         sub_hist.zero_()
+    if efp:
+        efp_sums.zero_()
     torch.cuda.synchronize(device)
     if world > 1:
         dist.barrier()
@@ -162,6 +177,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         if substructure:
             dist.all_reduce(sub_hist.counts)
             dist.all_reduce(sub_hist.sums)
+        if efp:
+            dist.all_reduce(efp_sums)
     e.record(main_s)
     torch.cuda.synchronize(device)
     t = torch.tensor([s.elapsed_time(e)], dtype=torch.float64, device=device)
@@ -193,8 +210,15 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
             defined = int(per[i, :SUBSTRUCTURE_BINS].sum())
             rec[f"mean_{name}"] = float(sums[i] / defined) if defined else float("nan")
         rec["substructure_sha1"] = hashlib.sha1(sc.tobytes()).hexdigest()
+    if efp:
+        es = efp_sums.tolist()
+        for name, v in zip(EFP_COLUMNS, es):
+            rec[f"mean_{name}"] = v / es[-1] if es[-1] else float("nan")
     if w1_reference is not None:
-        rec.update(_score_w1(w1_all, w1_reference.to(device, torch.float32), w1_cols))
+        reference = w1_reference.to(device, torch.float32)
+        rec.update(_score_w1(w1_all, reference, w1_cols))
+        if efp:
+            rec.update(_score_efp_metrics(w1_all, reference, w1_cols))
     return rec
 
 
@@ -221,9 +245,24 @@ def _score_w1(values, reference, cols):
             "w1_reference_jets": int(reference.shape[0]), "w1_seconds": s.elapsed_time(e) * 1e-3}
 
 
+def _score_efp_metrics(values, reference, cols):
+    """FPD and KPD (observables.fpd / kpd at their defaults) of the five d = 4 EFP columns of the gathered rows against the
+    reference's, timed by CUDA events around both."""
+    pick = [cols.index(c) for c in EFP_COLUMNS[1:]]
+    gen, real = values[:, pick], reference[:, pick]
+    stream = torch.cuda.current_stream(values.device)
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record(stream)
+    f = fpd(real, gen)
+    k = kpd(real, gen)
+    e.record(stream)
+    torch.cuda.synchronize(values.device)
+    return {"fpd": list(f), "kpd": list(k), "jet_metrics_seconds": s.elapsed_time(e) * 1e-3}
+
+
 def reference_observables(model, cfg, n_jets, device, n_particles=128, substructure=False, jet_offset=1 << 40, micro_batch=16384,
-                          precision="auto", stats=STATS):
-    """[n_jets, K] f32 on ``device``: the ``w1_columns(substructure)`` of ``n_jets`` jets made as ``sharded_generation_run`` makes
+                          precision="auto", stats=STATS, efp=False):
+    """[n_jets, K] f32 on ``device``: the ``w1_columns(substructure, efp)`` of ``n_jets`` jets made as ``sharded_generation_run`` makes
     them (same model, source, solver, observables) but from the Philox jet offsets ``jet_offset + j``, disjoint from any run's
     [0, total), so the sample is independent of it.  W1 between two such samples is the seed-to-seed noise floor.  ``stats``:
     the de-standardisation of the observables."""
@@ -231,7 +270,7 @@ def reference_observables(model, cfg, n_jets, device, n_particles=128, substruct
     table = model.step_table()
     N = n_particles
     mult_hist = _target_multiplicity(N)
-    out = torch.empty(n_jets, len(w1_columns(substructure)), dtype=torch.float32, device=device)
+    out = torch.empty(n_jets, len(w1_columns(substructure, efp)), dtype=torch.float32, device=device)
     index = _w1_index(device)
     for start in range(0, n_jets, micro_batch):
         B = min(micro_batch, n_jets - start)
@@ -239,5 +278,6 @@ def reference_observables(model, cfg, n_jets, device, n_particles=128, substruct
                                       jet_offset=jet_offset + start, compact=True)
         native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start, precision=precision)
         _, _, jets = jet_observables(x, k, m, stats, want_particles=False)
-        out[start:start + B] = _w1_rows(jets, jet_substructure(x, m, stats) if substructure else None, index)
+        out[start:start + B] = _w1_rows(jets, jet_substructure(x, m, stats) if substructure else None, index,
+                                        energy_flow_polynomials(x, m, stats) if efp else None)
     return out

@@ -1,11 +1,12 @@
 """BASELINE config 5: a 1 M-jet generation run sharded over the GPUs of one box (multimodal_particles_b200/pipeline.py).
 
-    python tools/million_jets.py [--jets 1048576] [--substructure] [--w1-reference-jets M | --w1-reference FILE.npz] [--out F]
+    python tools/million_jets.py [--jets 1048576] [--substructure] [--efp] [--w1-reference-jets M | --w1-reference FILE.npz] [--out F]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/million_jets.py
 
 Prints one JSON line on rank 0 (device time by CUDA events, max over ranks; `histogram_sha1` is the same for every GPU count).
 With a W1 reference — M jets built by `pipeline.reference_observables` from disjoint Philox streams, or one array per column
-of `pipeline.w1_columns` in an .npz file — the record also holds the W1 of every column against it (`w1`, `w1_seconds`)."""
+of `pipeline.w1_columns` in an .npz file — the record also holds the W1 of every column against it (`w1`, `w1_seconds`), and with
+`--efp` also W1-EFP (the efp4_* entries of `w1`), `fpd` and `kpd` of the five d = 4 EFPs."""
 import argparse
 import json
 import os
@@ -28,6 +29,7 @@ def main():
     ap.add_argument("--micro-batch", type=int, default=16384)
     ap.add_argument("--precision", default="auto")
     ap.add_argument("--substructure", action="store_true", help="also histogram tau21, tau32 and D2 of every jet on the device")
+    ap.add_argument("--efp", action="store_true", help="also compute the energy flow polynomials of every jet (W1-EFP, FPD, KPD)")
     ap.add_argument("--w1-reference-jets", type=int, default=0, help="score W1 against an independent reference sample of this size")
     ap.add_argument("--w1-reference", default=None, help="score W1 against this .npz (one array per column name)")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
@@ -41,12 +43,14 @@ def main():
     reference = None
     if args.w1_reference:
         with np.load(args.w1_reference) as f:
-            reference = torch.from_numpy(np.stack([f[c].astype(np.float32).reshape(-1) for c in w1_columns(args.substructure)], 1)).to(dev)
+            reference = torch.from_numpy(np.stack([f[c].astype(np.float32).reshape(-1) for c in w1_columns(args.substructure, args.efp)], 1)).to(dev)
     elif args.w1_reference_jets > 0:
         reference = reference_observables(model, cfg, args.w1_reference_jets, dev, n_particles=bench.N_PART,
-                                          substructure=args.substructure, micro_batch=args.micro_batch, precision=args.precision)
+                                          substructure=args.substructure, micro_batch=args.micro_batch, precision=args.precision,
+                                          efp=args.efp)
     rec = sharded_generation_run(model, cfg, args.jets, rank, world, dev, micro_batch=args.micro_batch, n_particles=bench.N_PART,
-                                 precision=args.precision, substructure=args.substructure, w1_reference=reference)
+                                 precision=args.precision, substructure=args.substructure, w1_reference=reference,
+                                 efp=args.efp)
     if rank == 0:
         line = json.dumps(rec)
         print(line)
