@@ -522,6 +522,26 @@ int mmb_wasserstein1d(const float* x, int64_t ldx, int n, const float* y, int64_
                       double* out, int64_t* n_used, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * The same W1 per draw and feature over the used slots of drawn jets (JetNet's W1-P, and with P = 1 and no masks its W1-M and
+ * W1-EFP draws, arXiv:2211.10295), with no host copy of the drawn samples and no host synchronisation:
+ *   value of jet j, slot p, feature c: x[j*ldx_jet + p*ldx_slot + c]; the slot is used iff mask_x == NULL || mask_x[j*ldmx + p];
+ *   the sample of draw t is the used slots of the jets idx_x[t][0..rows), in draw order and within a jet in slot order (a jet
+ *   drawn k times contributes k times); y, mask_y, idx_y likewise;
+ *   out [draws][F] f64 (device): out[t][c] is bit-identical to mmb_wasserstein1d on the two samples of draw t gathered into
+ *   rows (non-finite values dropped, NaN when a sample has no finite value); n_used [2][draws][F] int64 (device, nullable):
+ *   finite x values, then finite y values.
+ * 0 < F <= MMB_W1_MAX_K, P >= 1, draws >= 1, rows >= 1, rows * P <= 2^31 - 1, 2 * draws * F <= 2^31 - 1, n, m >= 1, ldx_slot >= F (P > 1),
+ * ldx_jet >= (P - 1) * ldx_slot + F, ldmx >= P with a mask (y likewise), else MMB_EINVAL.  Jet indices are device int32
+ * [draws][rows] in [0, n) / [0, m) (not checked).  workspace: 256-byte aligned, mmb_wasserstein1d_drawn_workspace_bytes(draws,
+ * rows, P, F) bytes (0 for invalid sizes), else MMB_ENOMEM.  Stream-ordered, allocates nothing, bit-identical from call to call.
+ */
+size_t mmb_wasserstein1d_drawn_workspace_bytes(int draws, int rows, int P, int F);
+int mmb_wasserstein1d_drawn(const float* x, int64_t ldx_jet, int64_t ldx_slot, const uint8_t* mask_x, int64_t ldmx, int n,
+                            const float* y, int64_t ldy_jet, int64_t ldy_slot, const uint8_t* mask_y, int64_t ldmy, int m,
+                            int P, int F, const int32_t* idx_x, const int32_t* idx_y, int draws, int rows,
+                            double* out, int64_t* n_used, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * Energy flow polynomials of a generated batch (the features of the W1-EFP, FPD and KPD metrics, arXiv:2211.10295, as JetNet
  * computes them with energyflow: hadronic measure, kappa = 1, normalised energies):
  *   constituents as for mmb_jet_substructure ((x * std + mean) in fp32, massless, y = eta; used iff mask != 0 && pt > 0);

@@ -804,6 +804,38 @@ int mmb_wasserstein1d(const float* x, int64_t ldx, int n, const float* y, int64_
                                 static_cast<cudaStream_t>(stream));
 }
 
+static bool drawn_sizes_ok(int draws, int rows, int P, int F) {
+    return F >= 1 && F <= MMB_W1_MAX_K && P >= 1 && draws >= 1 && rows >= 1 && (long long)rows * P <= 0x7FFFFFFFLL &&
+           2LL * draws * F <= 0x7FFFFFFFLL;   // segments (sample, draw, feature) are counted in int
+}
+
+size_t mmb_wasserstein1d_drawn_workspace_bytes(int draws, int rows, int P, int F) {
+    return drawn_sizes_ok(draws, rows, P, F) ? wasserstein1d_drawn_workspace_bytes(draws, rows, P, F) : 0;
+}
+
+static bool drawn_strides_ok(int64_t ld_jet, int64_t ld_slot, const uint8_t* mask, int64_t ldm, int P, int F) {
+    return (P == 1 || ld_slot >= F) && ld_jet >= (int64_t)(P - 1) * ld_slot + F && (!mask || ldm >= P);
+}
+
+int mmb_wasserstein1d_drawn(const float* x, int64_t ldx_jet, int64_t ldx_slot, const uint8_t* mask_x, int64_t ldmx, int n,
+                            const float* y, int64_t ldy_jet, int64_t ldy_slot, const uint8_t* mask_y, int64_t ldmy, int m,
+                            int P, int F, const int32_t* idx_x, const int32_t* idx_y, int draws, int rows,
+                            double* out, int64_t* n_used, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!drawn_sizes_ok(draws, rows, P, F))
+        return fail(MMB_EINVAL, "mmb_wasserstein1d_drawn: draws = %d, rows = %d, P = %d, F = %d (need >= 1, >= 1, rows * P and 2 * draws * F <= 2^31 - 1, F in 1..%d)",
+                    draws, rows, P, F, MMB_W1_MAX_K);
+    if (n < 1 || m < 1) return fail(MMB_EINVAL, "mmb_wasserstein1d_drawn: n and m must be positive");
+    if (!drawn_strides_ok(ldx_jet, ldx_slot, mask_x, ldmx, P, F) || !drawn_strides_ok(ldy_jet, ldy_slot, mask_y, ldmy, P, F))
+        return fail(MMB_EINVAL, "mmb_wasserstein1d_drawn: strides overlap for P = %d, F = %d", P, F);
+    if (!x || !y || !idx_x || !idx_y || !out || !workspace) return fail(MMB_EINVAL, "mmb_wasserstein1d_drawn: null argument");
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(MMB_EINVAL, "mmb_wasserstein1d_drawn: workspace not 256-byte aligned");
+    const size_t need = wasserstein1d_drawn_workspace_bytes(draws, rows, P, F);
+    if (need == 0) return MMB_ECUDA;   // a size query failed and set the error text
+    if (workspace_bytes < need) return fail(MMB_ENOMEM, "mmb_wasserstein1d_drawn: workspace %zu B, needs %zu B", workspace_bytes, need);
+    return launch_wasserstein1d_drawn(x, ldx_jet, ldx_slot, mask_x, ldmx, y, ldy_jet, ldy_slot, mask_y, ldmy, P, F, idx_x, idx_y, draws, rows,
+                                      out, reinterpret_cast<long long*>(n_used), workspace, static_cast<cudaStream_t>(stream));
+}
+
 int mmb_energy_flow_polynomials(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N, float beta,
                                 float* out, void* stream) {
     if (!x || !mask || !out) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials: null argument");

@@ -112,6 +112,12 @@ int launch_jet_substructure(const float* x, const uint8_t* mask, const float* me
 size_t wasserstein1d_workspace_bytes(int n, int m, int K);   // 0 when the CUB size query fails
 int launch_wasserstein1d(const float* x, long long ldx, int n, const float* y, long long ldy, int m, int K, double* out, long long* n_used,
                          void* workspace, cudaStream_t stream);
+// the same per draw and feature over the used slots of drawn jets: key expansion into segments of capacity rows * P, one sort each
+size_t wasserstein1d_drawn_workspace_bytes(int draws, int rows, int P, int F);   // 0 when a CUB size query fails
+int launch_wasserstein1d_drawn(const float* x, long long ldx_jet, long long ldx_slot, const uint8_t* mask_x, long long ldmx, const float* y,
+                               long long ldy_jet, long long ldy_slot, const uint8_t* mask_y, long long ldmy, int P, int F, const int32_t* idx_x,
+                               const int32_t* idx_y, int draws, int rows, double* out, long long* n_used, void* workspace,
+                               cudaStream_t stream);
 
 // efp.cu — energy flow polynomials, one block per jet, Theta as an upper triangle of 32 x 32 blocks in shared memory
 int launch_energy_flow_polynomials(const float* x, const uint8_t* mask, const float* mean, const float* sd, int B, int N, float beta,

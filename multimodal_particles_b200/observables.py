@@ -8,7 +8,8 @@ N-subjettiness on exclusive kt / WTA axes and D2, jets.py:204-240) is a second k
 reference scores with (scipy.stats.wasserstein_distance, jets.py:329-332) is a third (``mmb_wasserstein1d``, ``wasserstein1d``,
 ``JetClassHighLevelFeatures.wasserstein1d``).  The energy flow polynomials of the JetNet metrics (arXiv:2211.10295) are a fourth
 (``mmb_energy_flow_polynomials``, ``energy_flow_polynomials``, ``JetClassHighLevelFeatures.compute_efps``); ``fpd`` and ``kpd``
-score them with the sample statistics of ``mmb_sampled_moments`` and ``mmb_kpd_mmd``.
+score them with the sample statistics of ``mmb_sampled_moments`` and ``mmb_kpd_mmd``.  JetNet's W1-M, W1-P and W1-EFP (``w1m``,
+``w1p``, ``w1efp``) score seeded draws of jets with ``mmb_wasserstein1d_drawn`` (``wasserstein1d_drawn``).
 """
 import ctypes
 
@@ -93,6 +94,53 @@ def wasserstein1d(x, y, return_counts=False):
                                             _native._ptr(out), _native._ptr(used), _native._ptr(ws), ws.numel(), _native._stream()))
     if one:
         out, used = out[0], used[:, 0]
+    return (out, used) if return_counts else out
+
+
+def _jets(t, mask, name):
+    """[n, P, F] or [n, F] f32 CUDA tensor (+ [n, P] mask) -> (tensor, ld_jet, ld_slot, P, mask u8 or None, ldm)."""
+    if t.dtype != torch.float32 or not t.is_cuda or t.dim() not in (2, 3):
+        raise _native.MmbError(f"wasserstein1d_drawn: {name} must be a [n, P, F] or [n, F] float32 CUDA tensor; there is no CPU path")
+    if t.stride(-1) != 1:
+        t = t.contiguous()
+    P = t.shape[1] if t.dim() == 3 else 1
+    ld_jet, ld_slot = t.stride(0), (t.stride(1) if t.dim() == 3 else t.shape[1])
+    if t.shape[0] == 1:
+        ld_jet = max(ld_jet, P * t.shape[-1])
+    if mask is not None:
+        if not mask.is_cuda or mask.numel() != t.shape[0] * P:
+            raise _native.MmbError(f"wasserstein1d_drawn: mask of {name} must be a [{t.shape[0]}, {P}] CUDA tensor")
+        mask = as_u8(mask).contiguous()
+    return t, ld_jet, ld_slot, P, mask, P
+
+
+def wasserstein1d_drawn(x, idx_x, y, idx_y, mask_x=None, mask_y=None, return_counts=False):
+    """Per draw t and feature c: the W1 (``wasserstein1d``) between the used slots of the jets x[idx_x[t]] and those of
+    y[idx_y[t]], each taken in draw order and slot order (a jet drawn k times counts k times), without gathering them.
+    x [n, P, F] or [n, F] (P = 1), y likewise, f32 on the GPU; masks [n, P] (None: every slot used); indices [draws, rows]
+    -> [draws, F] f64 on the device, bit-identical to ``wasserstein1d`` on the gathered samples (DESIGN.md §4.6e).
+    ``return_counts``: also the finite counts [2, draws, F] int64."""
+    x, ldxj, ldxs, P, mx, ldmx = _jets(x, mask_x, "x")
+    y, ldyj, ldys, Py, my, ldmy = _jets(y, mask_y, "y")
+    if x.device != y.device or P != Py or x.shape[-1] != y.shape[-1] or idx_x.dim() != 2 or idx_x.shape != idx_y.shape:
+        raise _native.MmbError(f"wasserstein1d_drawn: x {tuple(x.shape)}, y {tuple(y.shape)}, indices {tuple(idx_x.shape)} / "
+                               f"{tuple(idx_y.shape)} do not match")
+    if not idx_x.is_cuda or not idx_y.is_cuda:
+        raise _native.MmbError("wasserstein1d_drawn: indices must be CUDA tensors; there is no CPU path")
+    F = x.shape[-1]
+    draws, rows = idx_x.shape
+    ix, iy = _index(idx_x), _index(idx_y)
+    dev = x.device
+    lib = _native.load()
+    with torch.cuda.device(dev):
+        need = lib.mmb_wasserstein1d_drawn_workspace_bytes(draws, rows, P, F)
+        ws = torch.empty(max(need, 256), dtype=torch.uint8, device=dev)
+        out = torch.empty(draws, F, dtype=torch.float64, device=dev)
+        used = torch.empty(2, draws, F, dtype=torch.int64, device=dev)
+        _native.check(lib.mmb_wasserstein1d_drawn(_native._ptr(x), ldxj, ldxs, _native._ptr(mx), ldmx, x.shape[0],
+                                                  _native._ptr(y), ldyj, ldys, _native._ptr(my), ldmy, y.shape[0], P, F,
+                                                  _native._ptr(ix), _native._ptr(iy), draws, rows, _native._ptr(out), _native._ptr(used),
+                                                  _native._ptr(ws), ws.numel(), _native._stream()))
     return (out, used) if return_counts else out
 
 
@@ -244,6 +292,65 @@ def kpd(real, gen, num_batches=10, batch_size=5000, degree=KPD_DEGREE, normalise
     vals = kpd_mmd(real, gen, ir, ig, scale, degree).cpu().numpy()
     lo, hi = np.percentile(vals, KPD_ERROR_RANGE)
     return float(np.median(vals)), float((hi - lo) / 2)
+
+
+# JetNet's W1-M, W1-P and W1-EFP (arXiv:2211.10295): each W1 is the mean +- std over W1_NUM_BATCHES draws of
+# W1_NUM_EVAL_SAMPLES jets from each sample.  Conventions as remembered, not checked against JetNet (DESIGN.md §4.6e):
+W1_NUM_EVAL_SAMPLES = 50_000
+W1_NUM_BATCHES = 5
+W1_STD_DDOF = 0                              # np.std over the batches
+PARTICLE_COLUMNS = ("pt", "eta_rel", "phi_rel")   # W1-P features: ParticleClouds.continuous after postprocess (JetNet: pt_rel)
+
+
+def jetnet_draws(n_real, n_gen, num_eval_samples=W1_NUM_EVAL_SAMPLES, num_batches=W1_NUM_BATCHES, seed=42, device=None):
+    """The draws of w1m / w1p / w1efp, with replacement, from one seeded device generator: [num_batches, num_eval_samples]
+    int32 indices into the real sample, then into the generated one."""
+    g = _generator(device, seed)
+    ir = torch.randint(n_real, (num_batches, num_eval_samples), generator=g, device=device, dtype=torch.int32)
+    ig = torch.randint(n_gen, (num_batches, num_eval_samples), generator=g, device=device, dtype=torch.int32)
+    return ir, ig
+
+
+def w1_summary(values, average=True):
+    """[batches, F] per-draw W1 values (host array) -> (mean, std): with ``average`` the mean over features of the per-feature
+    means and sqrt(sum_c std_c^2) (np.linalg.norm), else the per-feature arrays.  A draw where a sample has no used particle
+    is NaN (JetNet: inf) and makes its feature's mean and std NaN."""
+    values = np.asarray(values, dtype=np.float64)
+    means, stds = values.mean(0), values.std(0, ddof=W1_STD_DDOF)
+    if average:
+        return float(means.mean()), float(np.linalg.norm(stds))
+    return means, stds
+
+
+def _jet_level(t, name):
+    if t.dim() not in (1, 2):
+        raise _native.MmbError(f"{name} takes [n] or [n, d] float32 CUDA tensors")
+    return t.reshape(t.shape[0], -1)
+
+
+def w1m(real, gen, num_eval_samples=W1_NUM_EVAL_SAMPLES, num_batches=W1_NUM_BATCHES, seed=42):
+    """JetNet's W1-M of two [n] f32 CUDA jet-mass samples -> (mean, std) over the draws (``jetnet_draws``); one host wait."""
+    real, gen = _jet_level(real, "w1m"), _jet_level(gen, "w1m")
+    ir, ig = jetnet_draws(len(real), len(gen), num_eval_samples, num_batches, seed, real.device)
+    return w1_summary(wasserstein1d_drawn(real, ir, gen, ig).cpu().numpy())
+
+
+def w1efp(real, gen, num_eval_samples=W1_NUM_EVAL_SAMPLES, num_batches=W1_NUM_BATCHES, average_over_efps=True, seed=42):
+    """JetNet's W1-EFP of two [n, d] f32 CUDA EFP samples -> (mean, std) averaged over the EFPs (``w1_summary``), or per-EFP
+    arrays with ``average_over_efps=False``; one host wait."""
+    real, gen = _jet_level(real, "w1efp"), _jet_level(gen, "w1efp")
+    ir, ig = jetnet_draws(len(real), len(gen), num_eval_samples, num_batches, seed, real.device)
+    return w1_summary(wasserstein1d_drawn(real, ir, gen, ig).cpu().numpy(), average_over_efps)
+
+
+def w1p(real, gen, mask_real=None, mask_gen=None, num_eval_samples=W1_NUM_EVAL_SAMPLES, num_batches=W1_NUM_BATCHES,
+        average_over_features=True, seed=42):
+    """JetNet's W1-P of two [n, N, F] f32 CUDA samples of post-processed particle features (PARTICLE_COLUMNS), masks [n, N]
+    (None: every slot used) -> (mean, std) averaged over the features (``w1_summary``), or per-feature arrays with
+    ``average_over_features=False``.  Per draw, the sample is the used particles of the drawn jets; one host wait."""
+    ir, ig = jetnet_draws(len(real), len(gen), num_eval_samples, num_batches, seed, real.device)
+    vals = wasserstein1d_drawn(real, ir, gen, ig, mask_real, mask_gen)
+    return w1_summary(vals.cpu().numpy(), average_over_features)
 
 
 class ParticleClouds:

@@ -13,7 +13,10 @@ and histograms tau21, tau32 and D2 into int64 counts of their own (SUBSTRUCTURE_
 keeps the W1_COLUMNS of every jet; after the timed window they are all-gathered and scored against the reference with
 ``mmb_wasserstein1d`` (``reference_observables`` builds an independent reference sample).  With ``efp=True`` the side stream
 also runs ``mmb_energy_flow_polynomials``; their columns join the W1 columns, and with a reference the five d = 4 EFPs are also
-scored by FPD and KPD (``observables.fpd`` / ``kpd``) after the timed window.  The reference has no multi-GPU code
+scored by FPD and KPD (``observables.fpd`` / ``kpd``) after the timed window.  With ``particle_reference`` the side stream copies the
+post-processed particles of the jets JetNet's W1-P draws (``observables.jetnet_draws``, made before the window) into one buffer;
+after the window the buffers of the ranks are summed and scored with ``observables.w1p`` (``reference_particles`` builds the
+reference), and with ``w1_reference`` W1-M and W1-EFP are scored from the gathered jet columns.  The reference has no multi-GPU code
 (SURVEY.md §2.1); ``tools/million_jets.py`` and the multi-GPU arms of ``bench.py`` call this.
 """
 import hashlib
@@ -23,8 +26,8 @@ import torch
 import torch.distributed as dist
 
 from . import sharding
-from .observables import (EFP_COLUMNS, JET_COLUMNS, SUBSTRUCTURE_COLUMNS, energy_flow_polynomials, fpd, jet_observables, jet_substructure,
-                          kpd, wasserstein1d)
+from .observables import (EFP_COLUMNS, JET_COLUMNS, PARTICLE_COLUMNS, SUBSTRUCTURE_COLUMNS, energy_flow_polynomials, fpd, jet_observables,
+                          jet_substructure, jetnet_draws, kpd, w1_summary, w1efp, w1m, wasserstein1d, wasserstein1d_drawn)
 from .source import sample_source_state
 
 STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisation to a jet-like scale (pT > 0)
@@ -89,7 +92,7 @@ class SubstructureHistograms:
 
 
 def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_batch=4096, n_particles=128, precision="auto",
-                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None, efp=False):
+                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None, efp=False, particle_reference=None):
     """-> dict (rank 0: the C5 record; other ranks: None).  Device time by CUDA events around the whole slice incl. the final
     all-reduce, max over ranks.  ``substructure``: also histogram tau21, tau32 and D2 of every jet (``substructure_sha1``,
     ``substructure_counts`` and the means of the defined values join the record).  ``w1_reference``: [m, K] f32 device tensor
@@ -98,7 +101,11 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     ``w1_reference_jets`` and ``w1_seconds`` (CUDA events around the W1 call) join the record.  ``efp``: also compute the
     energy flow polynomials of every jet (the means of the defined values join the record as ``mean_efp1`` ...); their
     columns follow in ``w1_columns(substructure, efp)``, and with a reference ``fpd`` and ``kpd`` ([value, error] of the five
-    d = 4 EFPs against the reference's) and ``jet_metrics_seconds`` (CUDA events around both) join the record too."""
+    d = 4 EFPs against the reference's) and ``jet_metrics_seconds`` (CUDA events around both) join the record too.
+    ``particle_reference``: (x [m, N, 3] f32, mask [m, N] u8) device tensors of post-processed reference particles
+    (``reference_particles``); ``w1p`` ([mean, std]), ``w1p_features`` ({column: [mean, std]}), with ``w1_reference`` also ``w1m``
+    and with ``efp`` ``w1efp`` (JetNet's defaults, ``observables.w1p`` / ``w1m`` / ``w1efp``), and ``jetnet_w1_seconds`` (CUDA
+    events around the whole scoring, so it includes its host waits for the per-draw values) join the record."""
     native = model.encoder.native_model(device)
     table = model.step_table()
     lo, hi = sharding.shard_range(total_jets, rank, world)
@@ -115,6 +122,13 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
             raise ValueError(f"w1_reference must be [m, {len(w1_cols)}] ({', '.join(w1_cols)}), got {tuple(w1_reference.shape)}")
         w1_buf = torch.empty(hi - lo, len(w1_cols), dtype=torch.float32, device=device)   # this rank's jets, in jet order
         w1_index = _w1_index(device)
+    if particle_reference is not None:
+        p_ref_x, p_ref_m = particle_reference
+        if p_ref_x.dim() != 3 or tuple(p_ref_x.shape[1:]) != (N, 3) or p_ref_m.shape[:2] != p_ref_x.shape[:2]:
+            raise ValueError(f"particle_reference must be (x [m, {N}, 3], mask [m, {N}]), got {tuple(p_ref_x.shape)}, {tuple(p_ref_m.shape)}")
+        p_plan = _particle_plan(len(p_ref_x), total_jets, lo, hi, MB, device)
+        p_x = torch.zeros(p_plan["slots"], N, 3, dtype=torch.float32, device=device)   # the drawn jets' particles, by draw slot
+        p_m = torch.zeros(p_plan["slots"], N, dtype=torch.uint8, device=device)
     packs = [sharding.PackedJets(MB, N, 3, device) for _ in range(3)]      # state of a micro-batch: [x | tokens | mask], one allocation
     recv = [sharding.make_gather(MB, N, 3, world, device, mode=gather) for _ in range(2)] if world > 1 else None
     side = torch.cuda.Stream(device=device)
@@ -138,7 +152,7 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
             ev.record(main_s)
             with torch.cuda.stream(side):
                 side.wait_event(ev)
-                _, _, jets = jet_observables(x, k, m, STATS, want_particles=False)
+                x_phys, _, jets = jet_observables(x, k, m, STATS, want_particles=particle_reference is not None)
                 counts.add_(hist.accumulate(x, k, m))
                 jet_sums.add_(torch.nan_to_num(jets.double()).sum(0))
                 sub = jet_substructure(x, m, STATS) if substructure else None
@@ -150,6 +164,12 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
                     efp_sums.add_(torch.cat([torch.where(defined, efps, 0.0).double().sum(0), defined.double().sum(0)]))
                 if w1_reference is not None:
                     w1_buf[start - lo:start - lo + B].copy_(_w1_rows(jets, sub, w1_index, efps))
+                if particle_reference is not None:
+                    a, b = p_plan["ranges"][start]
+                    if b > a:   # the draw slots of this micro-batch's jets (ranges made on the host before the window)
+                        sel, jet = p_plan["slot"][a:b], p_plan["jet"][a:b] - start
+                        p_x.index_copy_(0, sel, x_phys.index_select(0, jet))
+                        p_m.index_copy_(0, sel, m.index_select(0, jet))
                 if world > 1 and B == MB:
                     recv[i & 1].gather(pk)          # the packed micro-batch to every rank (copy-engine push, or one all-gather)
                 for t in (x, k, m):
@@ -186,6 +206,9 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     if w1_reference is not None:
         w1_all = _gather_rows(w1_buf, total_jets, world, device) if world > 1 else w1_buf
+    if particle_reference is not None and world > 1:   # every draw slot has one owner; the other ranks hold zeros
+        dist.all_reduce(p_x)
+        dist.all_reduce(p_m)
     if rank != 0:
         return None
     ms = float(t.item())
@@ -219,6 +242,44 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         rec.update(_score_w1(w1_all, reference, w1_cols))
         if efp:
             rec.update(_score_efp_metrics(w1_all, reference, w1_cols))
+    if particle_reference is not None:
+        rec.update(_score_jetnet_w1(p_ref_x.to(device, torch.float32), p_ref_m.to(device), p_x, p_m, p_plan["idx_real"],
+                                    w1_all if w1_reference is not None else None,
+                                    w1_reference.to(device, torch.float32) if w1_reference is not None else None, w1_cols, efp))
+    return rec
+
+
+def _particle_plan(n_reference, total, lo, hi, micro_batch, device):
+    """JetNet's W1-P draws over the global jets [0, total) (``jetnet_draws``: the same on every rank), sorted by jet, and the
+    range of that order each micro-batch of this rank's [lo, hi) owns (one host read, before the timed window)."""
+    idx_real, idx_gen = jetnet_draws(n_reference, total, device=device)
+    jet, slot = torch.sort(idx_gen.reshape(-1).long(), stable=True)
+    starts = torch.arange(lo, hi + micro_batch, micro_batch, device=device).clamp_(max=hi)
+    cut = torch.searchsorted(jet, starts).tolist()
+    return {"idx_real": idx_real, "slots": idx_gen.numel(), "jet": jet, "slot": slot,
+            "ranges": {int(a): (cut[i], cut[i + 1]) for i, a in enumerate(starts[:-1].tolist())}}
+
+
+def _score_jetnet_w1(ref_x, ref_m, gen_x, gen_m, idx_real, jet_values, jet_reference, cols, efp):
+    """W1-P of the gathered draw slots against the reference particles (``observables.w1p`` with the run's draws), and with jet
+    columns W1-M and W1-EFP (``observables.w1m`` / ``w1efp``).  The CUDA events span all of them, including the host reading
+    each call's per-draw values and the numpy aggregation between the calls, so the time is that of the whole scoring."""
+    stream = torch.cuda.current_stream(gen_x.device)
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record(stream)
+    slots = torch.arange(gen_x.shape[0], dtype=torch.int32, device=gen_x.device).reshape(idx_real.shape)
+    vals = wasserstein1d_drawn(ref_x, idx_real, gen_x, slots, ref_m, gen_m).cpu().numpy()
+    rec = {"w1p": list(w1_summary(vals)),
+           "w1p_features": {c: [float(a), float(b)] for c, a, b in zip(PARTICLE_COLUMNS, *w1_summary(vals, average=False))}}
+    if jet_values is not None:
+        m = cols.index("m")
+        rec["w1m"] = list(w1m(jet_reference[:, m], jet_values[:, m]))
+        if efp:
+            pick = [cols.index(c) for c in EFP_COLUMNS[1:]]
+            rec["w1efp"] = list(w1efp(jet_reference[:, pick], jet_values[:, pick]))
+    e.record(stream)
+    torch.cuda.synchronize(gen_x.device)
+    rec["jetnet_w1_seconds"] = s.elapsed_time(e) * 1e-3
     return rec
 
 
@@ -281,3 +342,25 @@ def reference_observables(model, cfg, n_jets, device, n_particles=128, substruct
         out[start:start + B] = _w1_rows(jets, jet_substructure(x, m, stats) if substructure else None, index,
                                         energy_flow_polynomials(x, m, stats) if efp else None)
     return out
+
+
+def reference_particles(model, cfg, n_jets, device, n_particles=128, jet_offset=1 << 40, micro_batch=16384, precision="auto", stats=STATS):
+    """(x [n_jets, N, 3] f32, mask [n_jets, N] u8) on ``device``: the post-processed particles (PARTICLE_COLUMNS) and masks of
+    ``n_jets`` jets made as ``reference_observables`` makes them (same model, source, solver, post-processing, Philox jet offsets
+    ``jet_offset + j``); the particle reference of ``sharded_generation_run(particle_reference=...)``.  ``jet_offset=0``
+    reproduces the run's own jets."""
+    native = model.encoder.native_model(device)
+    table = model.step_table()
+    N = n_particles
+    mult_hist = _target_multiplicity(N)
+    out_x = torch.empty(n_jets, N, 3, dtype=torch.float32, device=device)
+    out_m = torch.empty(n_jets, N, dtype=torch.uint8, device=device)
+    for start in range(0, n_jets, micro_batch):
+        B = min(micro_batch, n_jets - start)
+        x, k, m = sample_source_state(B, N, target_multiplicity=mult_hist, min_num_particles=0, device=device, seed=7,
+                                      jet_offset=jet_offset + start, compact=True)
+        native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start, precision=precision)
+        x_phys, _, _ = jet_observables(x, k, m, stats)
+        out_x[start:start + B] = x_phys
+        out_m[start:start + B] = m
+    return out_x, out_m
