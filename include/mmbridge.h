@@ -564,6 +564,52 @@ int mmb_energy_flow_polynomials(const float* x, const uint8_t* mask, const float
                                 float* out, void* stream);
 
 /*
+ * Every energy flow polynomial of degree (edge count) d <= 4: the feature set JetNet scores FPD and KPD on (efpset ("d<=", 4),
+ * 36 EFPs).  Constituents, z, theta and the index-tuple sum as for mmb_energy_flow_polynomials; in addition
+ *   c_i = sum_j z_j theta_ij^3, r_i = sum_j z_j theta_ij^4, u_i = sum_k theta_ik z_k s_k.
+ * The 20 connected loopless multigraphs with 1 <= d <= 4 (V vertices):
+ *   d = 1  EFPD4_1                  edge (V 2)                       sum_i z_i s_i
+ *   d = 2  EFPD4_2_DOUBLE           double edge (2)                  sum_i z_i q_i
+ *          EFPD4_2_PATH             2-edge path (3)                  sum_i z_i s_i^2
+ *   d = 3  EFPD4_3_TRIPLE           triple edge (2)                  sum_i z_i c_i
+ *          EFPD4_3_PATH_DOUBLE      2-edge path, one edge doubled (3) sum_i z_i q_i s_i
+ *          EFPD4_3_TRIANGLE         triangle (3)                     sum_{i,k} z_i z_k theta_ik M_ik
+ *          EFPD4_3_PATH             3-edge path (4)                  sum_i z_i s_i u_i
+ *          EFPD4_3_STAR             3-star (4)                       sum_i z_i s_i^3
+ *   d = 4  EFPD4_4_QUADRUPLE        quadruple edge (2)               sum_i z_i r_i
+ *          EFPD4_4_TRIPLE_SINGLE    triple edge + edge (3)           sum_i z_i c_i s_i
+ *          EFPD4_4_DOUBLE_DOUBLE    two doubled edges (3)            sum_i z_i q_i^2
+ *          EFPD4_4_TRIANGLE_DOUBLE  triangle, one edge doubled (3)   sum_{i,k} z_i z_k theta_ik^2 M_ik
+ *          EFPD4_4_SQUARE .. EFPD4_4_STAR2   the five 4-vertex graphs of mmb_energy_flow_polynomials, same formulas
+ *          EFPD4_4_PATH             4-edge path (5)                  sum_i z_i u_i^2
+ *          EFPD4_4_STAR             4-star (5)                       sum_i z_i s_i^4
+ *          EFPD4_4_FORK             3-star, one leg extended (5)     sum_i z_i s_i^2 u_i
+ * and the empty graph EFPD4_0 = 1 and the 15 disconnected graphs, whose EFP is the product of their components' (formed in
+ * fp64 from the fp64 sums, rounded once): EFPD4_1_1 is efp1^2, EFPD4_1_2_DOUBLE is efp1 * efp2_double, and so on; the
+ * columns are ordered by d, connected before disconnected.  EFPD4_1 and the five EFPD4_4_{SQUARE, PAW, PATH_MID2, PATH_END2,
+ * STAR2} are bit-identical to the columns of mmb_energy_flow_polynomials on the same input and beta.
+ * A jet with no used particle gets NaN in every column; one used particle: EFPD4_0 = 1, every other column 0.
+ * x [B,N,3] f32, mask [B,N] u8, N <= MMB_SUB_MAX_N (larger N: MMB_EINVAL); beta > 0.  out [B][MMB_EFPD4_OBS] f32.
+ * Stream-ordered, allocates nothing, bit-identical from call to call.
+ */
+enum {
+    MMB_EFPD4_0 = 0,
+    MMB_EFPD4_1,
+    MMB_EFPD4_2_DOUBLE, MMB_EFPD4_2_PATH, MMB_EFPD4_1_1,
+    MMB_EFPD4_3_TRIPLE, MMB_EFPD4_3_PATH_DOUBLE, MMB_EFPD4_3_TRIANGLE, MMB_EFPD4_3_PATH, MMB_EFPD4_3_STAR,
+    MMB_EFPD4_1_2_DOUBLE, MMB_EFPD4_1_2_PATH, MMB_EFPD4_1_1_1,
+    MMB_EFPD4_4_QUADRUPLE, MMB_EFPD4_4_TRIPLE_SINGLE, MMB_EFPD4_4_DOUBLE_DOUBLE, MMB_EFPD4_4_TRIANGLE_DOUBLE, MMB_EFPD4_4_SQUARE,
+    MMB_EFPD4_4_PAW, MMB_EFPD4_4_PATH_MID2, MMB_EFPD4_4_PATH_END2, MMB_EFPD4_4_STAR2, MMB_EFPD4_4_PATH, MMB_EFPD4_4_STAR,
+    MMB_EFPD4_4_FORK,
+    MMB_EFPD4_1_3_TRIPLE, MMB_EFPD4_1_3_PATH_DOUBLE, MMB_EFPD4_1_3_TRIANGLE, MMB_EFPD4_1_3_PATH, MMB_EFPD4_1_3_STAR,
+    MMB_EFPD4_2_DOUBLE_2_DOUBLE, MMB_EFPD4_2_DOUBLE_2_PATH, MMB_EFPD4_2_PATH_2_PATH, MMB_EFPD4_1_1_2_DOUBLE, MMB_EFPD4_1_1_2_PATH,
+    MMB_EFPD4_1_1_1_1,
+    MMB_EFPD4_OBS
+};
+int mmb_energy_flow_polynomials_d4(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N,
+                                   float beta, float* out, void* stream);
+
+/*
  * Sample statistics of the Frechet and kernel physics distances (FPD, KPD; arXiv:2211.10295) over rows the caller draws:
  * x: row r, column c at x[r*ldx + c] (ldx >= d), n rows, device f32; every value is used as x * scale[c] in fp64 (scale: device
  * f32 [d], NULL for 1).  Row indices are device int32 in [0, n) (not checked).  0 < d <= MMB_MET_MAX_D.

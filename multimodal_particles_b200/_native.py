@@ -113,6 +113,7 @@ SIGNATURES = {
     "mmb_wasserstein1d_drawn": (_i, [_vp, _i64, _i64, _vp, _i64, _i, _vp, _i64, _i64, _vp, _i64, _i, _i, _i, _vp, _vp, _i, _i,
                                      _vp, _vp, _vp, _sz, _vp]),
     "mmb_energy_flow_polynomials": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _vp, _vp]),
+    "mmb_energy_flow_polynomials_d4": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _vp, _vp]),
     "mmb_sampled_moments": (_i, [_vp, _i64, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "mmb_kpd_mmd_workspace_bytes": (_sz, [_i, _i, _i]),
     "mmb_kpd_mmd": (_i, [_vp, _i64, _i, _vp, _i64, _i, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _sz, _vp]),

@@ -847,6 +847,18 @@ int mmb_energy_flow_polynomials(const float* x, const uint8_t* mask, const float
     return launch_energy_flow_polynomials(x, mask, mean, std, B, N, beta, out, static_cast<cudaStream_t>(stream));
 }
 
+int mmb_energy_flow_polynomials_d4(const float* x, const uint8_t* mask, const float* mean, const float* std, int B, int N,
+                                   float beta, float* out, void* stream) {
+    if (!x || !mask || !out) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials_d4: null argument");
+    if ((mean == nullptr) != (std == nullptr)) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials_d4: mean and std go together");
+    if (B < 0 || N < 0) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials_d4: negative size");
+    if (N > MMB_SUB_MAX_N)
+        return fail(MMB_EINVAL, "mmb_energy_flow_polynomials_d4: N = %d exceeds %d particle slots", N, MMB_SUB_MAX_N);
+    if (!(beta > 0.0f)) return fail(MMB_EINVAL, "mmb_energy_flow_polynomials_d4: beta must be positive");
+    if (B == 0) return MMB_OK;
+    return launch_energy_flow_polynomials_d4(x, mask, mean, std, B, N, beta, out, static_cast<cudaStream_t>(stream));
+}
+
 int mmb_sampled_moments(const float* x, int64_t ldx, int n, int d, const float* scale, const int32_t* idx, int draws, int rows,
                         double* sum, double* sumsq, void* stream) {
     if (d < 1 || d > MMB_MET_MAX_D) return fail(MMB_EINVAL, "mmb_sampled_moments: d = %d outside 1..%d", d, MMB_MET_MAX_D);

@@ -122,6 +122,8 @@ int launch_wasserstein1d_drawn(const float* x, long long ldx_jet, long long ldx_
 // efp.cu — energy flow polynomials, one block per jet, Theta as an upper triangle of 32 x 32 blocks in shared memory
 int launch_energy_flow_polynomials(const float* x, const uint8_t* mask, const float* mean, const float* sd, int B, int N, float beta,
                                    float* out, cudaStream_t stream);
+int launch_energy_flow_polynomials_d4(const float* x, const uint8_t* mask, const float* mean, const float* sd, int B, int N,
+                                      float beta, float* out, cudaStream_t stream);
 
 // jet_metrics.cu — FPD moments over drawn rows, KPD unbiased MMD^2 over row strips with fixed-order partials
 int launch_sampled_moments(const float* x, long long ldx, int d, const float* scale, const int* idx, int draws, int rows, double* sum,

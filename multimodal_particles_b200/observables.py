@@ -8,7 +8,9 @@ N-subjettiness on exclusive kt / WTA axes and D2, jets.py:204-240) is a second k
 reference scores with (scipy.stats.wasserstein_distance, jets.py:329-332) is a third (``mmb_wasserstein1d``, ``wasserstein1d``,
 ``JetClassHighLevelFeatures.wasserstein1d``).  The energy flow polynomials of the JetNet metrics (arXiv:2211.10295) are a fourth
 (``mmb_energy_flow_polynomials``, ``energy_flow_polynomials``, ``JetClassHighLevelFeatures.compute_efps``); ``fpd`` and ``kpd``
-score them with the sample statistics of ``mmb_sampled_moments`` and ``mmb_kpd_mmd``.  JetNet's W1-M, W1-P and W1-EFP (``w1m``,
+score them with the sample statistics of ``mmb_sampled_moments`` and ``mmb_kpd_mmd``; every EFP of degree <= 4, the feature set
+JetNet scores FPD and KPD on, is a second instantiation of that kernel (``mmb_energy_flow_polynomials_d4``,
+``energy_flow_polynomials_d4``, ``jetnet_fpd_features``).  JetNet's W1-M, W1-P and W1-EFP (``w1m``,
 ``w1p``, ``w1efp``) score seeded draws of jets with ``mmb_wasserstein1d_drawn`` (``wasserstein1d_drawn``).
 """
 import ctypes
@@ -156,18 +158,61 @@ KPD_ERROR_RANGE = (16.275, 83.725)           # KPD error: half of this percentil
 def energy_flow_polynomials(x, mask_u8, stats=None, beta=EFP_BETA):
     """x [B,N,3] f32 (pt, eta, phi; standardised when ``stats`` is given), mask [B,N] u8 on the GPU, N <= 256 -> [B,6] f32 in the
     order of ``EFP_COLUMNS``.  Jets with no used particle (mask and pt > 0) are NaN; jets with one are 0."""
+    return _efp_call("mmb_energy_flow_polynomials", len(EFP_COLUMNS), x, mask_u8, stats, beta)
+
+
+def _efp_call(name, columns, x, mask_u8, stats, beta):
     _native._require_cuda(x, mask_u8)
     B, N, _ = x.shape
     dev = x.device
-    out = torch.empty(B, len(EFP_COLUMNS), dtype=torch.float32, device=dev)
+    out = torch.empty(B, columns, dtype=torch.float32, device=dev)
     mean = std = None
     if stats is not None:
         mean = (ctypes.c_float * 3)(*[float(v) for v in stats["mean"][:3]])
         std = (ctypes.c_float * 3)(*[float(v) for v in stats["std"][:3]])
     with torch.cuda.device(dev):
-        _native.check(_native.load().mmb_energy_flow_polynomials(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(beta),
-                                                                 _native._ptr(out), _native._stream()))
+        _native.check(getattr(_native.load(), name)(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(beta),
+                                                    _native._ptr(out), _native._stream()))
     return out
+
+
+# every EFP of degree d <= 4 (DESIGN.md §4.6f), the kernel's column order: by d, connected graphs before disconnected ones.  A
+# disconnected graph is named by its components (its EFP is their product); "^k" is k copies of one component.  energyflow
+# orders its graphs differently; FD and the polynomial-kernel MMD do not depend on the order of the features, and fpd / kpd
+# normalise each column on its own, so the order does not change FPD or KPD.
+EFP_D4_COLUMNS = ("efp0",
+                  "efp1",
+                  "efp2_double", "efp2_path", "efp1^2",
+                  "efp3_triple", "efp3_path_double", "efp3_triangle", "efp3_path", "efp3_star",
+                  "efp1*efp2_double", "efp1*efp2_path", "efp1^3",
+                  "efp4_quadruple", "efp4_triple_single", "efp4_double_double", "efp4_triangle_double", "efp4_square", "efp4_paw",
+                  "efp4_path_mid2", "efp4_path_end2", "efp4_star2", "efp4_path", "efp4_star", "efp4_fork",
+                  "efp1*efp3_triple", "efp1*efp3_path_double", "efp1*efp3_triangle", "efp1*efp3_path", "efp1*efp3_star",
+                  "efp2_double^2", "efp2_double*efp2_path", "efp2_path^2", "efp1^2*efp2_double", "efp1^2*efp2_path", "efp1^4")
+# the features FPD / KPD score, as remembered of JetNet's get_fpd_kpd_jet_features (efps(jets, efpset_args=[("d<=", 4)]), "36
+# EFPs"): every column, the empty graph and the disconnected graphs included.  The one place to change if the set turns out
+# to be the prime (connected) graphs or to exclude efp0.
+FPD_EFP_COLUMNS = EFP_D4_COLUMNS
+
+
+def energy_flow_polynomials_d4(x, mask_u8, stats=None, beta=EFP_BETA):
+    """Every EFP of degree <= 4 (``mmb_energy_flow_polynomials_d4``): x [B,N,3] f32 (pt, eta, phi; standardised when ``stats``
+    is given), mask [B,N] u8 on the GPU, N <= 256 -> [B,36] f32 in the order of ``EFP_D4_COLUMNS``.  Jets with no used particle
+    (mask and pt > 0) are NaN in every column; jets with one are 1 in efp0 and 0 elsewhere.  efp1 and the five efp4_* columns of
+    ``EFP_COLUMNS`` are bit-identical to ``energy_flow_polynomials``'."""
+    return _efp_call("mmb_energy_flow_polynomials_d4", len(EFP_D4_COLUMNS), x, mask_u8, stats, beta)
+
+
+_FPD_PICK = [EFP_D4_COLUMNS.index(c) for c in FPD_EFP_COLUMNS]
+
+
+def jetnet_fpd_features(x, mask_u8, stats=None):
+    """The features ``fpd`` / ``kpd`` score as JetNet does (``FPD_EFP_COLUMNS`` of ``energy_flow_polynomials_d4`` at EFP_BETA):
+    [B, len(FPD_EFP_COLUMNS)] f32 on the device."""
+    out = energy_flow_polynomials_d4(x, mask_u8, stats)
+    if _FPD_PICK == list(range(len(EFP_D4_COLUMNS))):
+        return out
+    return out[:, _FPD_PICK].contiguous()
 
 
 def _metric_rows(t, name):

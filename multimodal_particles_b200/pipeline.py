@@ -16,7 +16,10 @@ also runs ``mmb_energy_flow_polynomials``; their columns join the W1 columns, an
 scored by FPD and KPD (``observables.fpd`` / ``kpd``) after the timed window.  With ``particle_reference`` the side stream copies the
 post-processed particles of the jets JetNet's W1-P draws (``observables.jetnet_draws``, made before the window) into one buffer;
 after the window the buffers of the ranks are summed and scored with ``observables.w1p`` (``reference_particles`` builds the
-reference), and with ``w1_reference`` W1-M and W1-EFP are scored from the gathered jet columns.  The reference has no multi-GPU code
+reference), and with ``w1_reference`` W1-M and W1-EFP are scored from the gathered jet columns.  With ``fpd_reference`` the side
+stream also runs ``mmb_energy_flow_polynomials_d4`` and keeps JetNet's FPD / KPD features (``observables.jetnet_fpd_features``,
+every EFP of degree <= 4) of every jet; after the window they are gathered and scored with ``fpd`` and ``kpd``
+(``reference_fpd_features`` builds the reference).  The reference has no multi-GPU code
 (SURVEY.md §2.1); ``tools/million_jets.py`` and the multi-GPU arms of ``bench.py`` call this.
 """
 import hashlib
@@ -26,8 +29,9 @@ import torch
 import torch.distributed as dist
 
 from . import sharding
-from .observables import (EFP_COLUMNS, JET_COLUMNS, PARTICLE_COLUMNS, SUBSTRUCTURE_COLUMNS, energy_flow_polynomials, fpd, jet_observables,
-                          jet_substructure, jetnet_draws, kpd, w1_summary, w1efp, w1m, wasserstein1d, wasserstein1d_drawn)
+from .observables import (EFP_COLUMNS, FPD_EFP_COLUMNS, JET_COLUMNS, PARTICLE_COLUMNS, SUBSTRUCTURE_COLUMNS, energy_flow_polynomials, fpd,
+                          jet_observables, jet_substructure, jetnet_draws, jetnet_fpd_features, kpd, w1_summary, w1efp, w1m, wasserstein1d,
+                          wasserstein1d_drawn)
 from .source import sample_source_state
 
 STATS = {"mean": [1.2, 0.0, 0.0], "std": [0.35, 0.2, 0.2]}   # de-standardisation to a jet-like scale (pT > 0)
@@ -92,7 +96,8 @@ class SubstructureHistograms:
 
 
 def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_batch=4096, n_particles=128, precision="auto",
-                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None, efp=False, particle_reference=None):
+                           warmup_batches=2, gather="auto", substructure=False, w1_reference=None, efp=False, particle_reference=None,
+                           fpd_reference=None):
     """-> dict (rank 0: the C5 record; other ranks: None).  Device time by CUDA events around the whole slice incl. the final
     all-reduce, max over ranks.  ``substructure``: also histogram tau21, tau32 and D2 of every jet (``substructure_sha1``,
     ``substructure_counts`` and the means of the defined values join the record).  ``w1_reference``: [m, K] f32 device tensor
@@ -105,7 +110,11 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     ``particle_reference``: (x [m, N, 3] f32, mask [m, N] u8) device tensors of post-processed reference particles
     (``reference_particles``); ``w1p`` ([mean, std]), ``w1p_features`` ({column: [mean, std]}), with ``w1_reference`` also ``w1m``
     and with ``efp`` ``w1efp`` (JetNet's defaults, ``observables.w1p`` / ``w1m`` / ``w1efp``), and ``jetnet_w1_seconds`` (CUDA
-    events around the whole scoring, so it includes its host waits for the per-draw values) join the record."""
+    events around the whole scoring, so it includes its host waits for the per-draw values) join the record.
+    ``fpd_reference``: [m, len(FPD_EFP_COLUMNS)] f32 device tensor of reference ``observables.jetnet_fpd_features``
+    (``reference_fpd_features``); the side stream keeps those features of every jet (144 B per jet), and after the timed window
+    they are gathered in jet order and ``jetnet_fpd`` and ``jetnet_kpd`` ([value, error] of ``fpd`` / ``kpd`` at their
+    defaults), ``jetnet_fpd_reference_jets`` and ``jetnet_fpd_seconds`` (CUDA events around both calls) join the record."""
     native = model.encoder.native_model(device)
     table = model.step_table()
     lo, hi = sharding.shard_range(total_jets, rank, world)
@@ -129,6 +138,10 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         p_plan = _particle_plan(len(p_ref_x), total_jets, lo, hi, MB, device)
         p_x = torch.zeros(p_plan["slots"], N, 3, dtype=torch.float32, device=device)   # the drawn jets' particles, by draw slot
         p_m = torch.zeros(p_plan["slots"], N, dtype=torch.uint8, device=device)
+    if fpd_reference is not None:
+        if fpd_reference.dim() != 2 or fpd_reference.shape[1] != len(FPD_EFP_COLUMNS):
+            raise ValueError(f"fpd_reference must be [m, {len(FPD_EFP_COLUMNS)}] (FPD_EFP_COLUMNS), got {tuple(fpd_reference.shape)}")
+        fpd_buf = torch.empty(hi - lo, len(FPD_EFP_COLUMNS), dtype=torch.float32, device=device)   # this rank's jets, in jet order
     packs = [sharding.PackedJets(MB, N, 3, device) for _ in range(3)]      # state of a micro-batch: [x | tokens | mask], one allocation
     recv = [sharding.make_gather(MB, N, 3, world, device, mode=gather) for _ in range(2)] if world > 1 else None
     side = torch.cuda.Stream(device=device)
@@ -170,6 +183,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
                         sel, jet = p_plan["slot"][a:b], p_plan["jet"][a:b] - start
                         p_x.index_copy_(0, sel, x_phys.index_select(0, jet))
                         p_m.index_copy_(0, sel, m.index_select(0, jet))
+                if fpd_reference is not None:
+                    fpd_buf[start - lo:start - lo + B].copy_(jetnet_fpd_features(x, m, STATS))
                 if world > 1 and B == MB:
                     recv[i & 1].gather(pk)          # the packed micro-batch to every rank (copy-engine push, or one all-gather)
                 for t in (x, k, m):
@@ -206,6 +221,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     if w1_reference is not None:
         w1_all = _gather_rows(w1_buf, total_jets, world, device) if world > 1 else w1_buf
+    if fpd_reference is not None:
+        fpd_all = _gather_rows(fpd_buf, total_jets, world, device) if world > 1 else fpd_buf
     if particle_reference is not None and world > 1:   # every draw slot has one owner; the other ranks hold zeros
         dist.all_reduce(p_x)
         dist.all_reduce(p_m)
@@ -246,6 +263,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         rec.update(_score_jetnet_w1(p_ref_x.to(device, torch.float32), p_ref_m.to(device), p_x, p_m, p_plan["idx_real"],
                                     w1_all if w1_reference is not None else None,
                                     w1_reference.to(device, torch.float32) if w1_reference is not None else None, w1_cols, efp))
+    if fpd_reference is not None:
+        rec.update(_score_jetnet_fpd(fpd_all, fpd_reference.to(device, torch.float32)))
     return rec
 
 
@@ -321,23 +340,44 @@ def _score_efp_metrics(values, reference, cols):
     return {"fpd": list(f), "kpd": list(k), "jet_metrics_seconds": s.elapsed_time(e) * 1e-3}
 
 
+def _score_jetnet_fpd(values, reference):
+    """FPD and KPD (observables.fpd / kpd at their defaults) of the gathered FPD_EFP_COLUMNS rows against the reference's, timed
+    by CUDA events around both."""
+    stream = torch.cuda.current_stream(values.device)
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record(stream)
+    f = fpd(reference, values)
+    k = kpd(reference, values)
+    e.record(stream)
+    torch.cuda.synchronize(values.device)
+    return {"jetnet_fpd": list(f), "jetnet_kpd": list(k), "jetnet_fpd_reference_jets": int(reference.shape[0]),
+            "jetnet_fpd_seconds": s.elapsed_time(e) * 1e-3}
+
+
+def _reference_jets(model, n_jets, device, N, jet_offset, micro_batch, precision):
+    """Yields (start, x, k, mask) of the micro-batches of ``n_jets`` generated jets made as ``sharded_generation_run`` makes them
+    (same model, source, solver) from the Philox jet offsets ``jet_offset + start + j``."""
+    native = model.encoder.native_model(device)
+    table = model.step_table()
+    mult_hist = _target_multiplicity(N)
+    for start in range(0, n_jets, micro_batch):
+        B = min(micro_batch, n_jets - start)
+        x, k, m = sample_source_state(B, N, target_multiplicity=mult_hist, min_num_particles=0, device=device, seed=7,
+                                      jet_offset=jet_offset + start, compact=True)
+        native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start, precision=precision)
+        yield start, x, k, m
+
+
 def reference_observables(model, cfg, n_jets, device, n_particles=128, substructure=False, jet_offset=1 << 40, micro_batch=16384,
                           precision="auto", stats=STATS, efp=False):
     """[n_jets, K] f32 on ``device``: the ``w1_columns(substructure, efp)`` of ``n_jets`` jets made as ``sharded_generation_run`` makes
     them (same model, source, solver, observables) but from the Philox jet offsets ``jet_offset + j``, disjoint from any run's
     [0, total), so the sample is independent of it.  W1 between two such samples is the seed-to-seed noise floor.  ``stats``:
     the de-standardisation of the observables."""
-    native = model.encoder.native_model(device)
-    table = model.step_table()
-    N = n_particles
-    mult_hist = _target_multiplicity(N)
     out = torch.empty(n_jets, len(w1_columns(substructure, efp)), dtype=torch.float32, device=device)
     index = _w1_index(device)
-    for start in range(0, n_jets, micro_batch):
-        B = min(micro_batch, n_jets - start)
-        x, k, m = sample_source_state(B, N, target_multiplicity=mult_hist, min_num_particles=0, device=device, seed=7,
-                                      jet_offset=jet_offset + start, compact=True)
-        native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start, precision=precision)
+    for start, x, k, m in _reference_jets(model, n_jets, device, n_particles, jet_offset, micro_batch, precision):
+        B = x.shape[0]
         _, _, jets = jet_observables(x, k, m, stats, want_particles=False)
         out[start:start + B] = _w1_rows(jets, jet_substructure(x, m, stats) if substructure else None, index,
                                         energy_flow_polynomials(x, m, stats) if efp else None)
@@ -349,18 +389,23 @@ def reference_particles(model, cfg, n_jets, device, n_particles=128, jet_offset=
     ``n_jets`` jets made as ``reference_observables`` makes them (same model, source, solver, post-processing, Philox jet offsets
     ``jet_offset + j``); the particle reference of ``sharded_generation_run(particle_reference=...)``.  ``jet_offset=0``
     reproduces the run's own jets."""
-    native = model.encoder.native_model(device)
-    table = model.step_table()
     N = n_particles
-    mult_hist = _target_multiplicity(N)
     out_x = torch.empty(n_jets, N, 3, dtype=torch.float32, device=device)
     out_m = torch.empty(n_jets, N, dtype=torch.uint8, device=device)
-    for start in range(0, n_jets, micro_batch):
-        B = min(micro_batch, n_jets - start)
-        x, k, m = sample_source_state(B, N, target_multiplicity=mult_hist, min_num_particles=0, device=device, seed=7,
-                                      jet_offset=jet_offset + start, compact=True)
-        native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start, precision=precision)
+    for start, x, k, m in _reference_jets(model, n_jets, device, N, jet_offset, micro_batch, precision):
+        B = x.shape[0]
         x_phys, _, _ = jet_observables(x, k, m, stats)
         out_x[start:start + B] = x_phys
         out_m[start:start + B] = m
     return out_x, out_m
+
+
+def reference_fpd_features(model, cfg, n_jets, device, n_particles=128, jet_offset=1 << 40, micro_batch=16384, precision="auto",
+                           stats=STATS):
+    """[n_jets, len(FPD_EFP_COLUMNS)] f32 on ``device``: ``observables.jetnet_fpd_features`` of ``n_jets`` jets made as
+    ``reference_observables`` makes them (Philox jet offsets ``jet_offset + j``); the reference of
+    ``sharded_generation_run(fpd_reference=...)``.  ``jet_offset=0`` reproduces the run's own jets."""
+    out = torch.empty(n_jets, len(FPD_EFP_COLUMNS), dtype=torch.float32, device=device)
+    for start, x, _, m in _reference_jets(model, n_jets, device, n_particles, jet_offset, micro_batch, precision):
+        out[start:start + x.shape[0]] = jetnet_fpd_features(x, m, stats)
+    return out
