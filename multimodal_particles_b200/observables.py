@@ -24,6 +24,31 @@ from .epic import as_u8
 JET_COLUMNS = ("px", "py", "pz", "e", "pt", "m", "eta", "phi", "multiplicity", "Q_total", "Q_jet")
 
 
+def _stats_arrays(stats):
+    """{"mean": [...], "std": [...]} (the first three entries: pt, eta, phi) -> (mean, std) as ctypes float[3], or (None, None)."""
+    if stats is None:
+        return None, None
+    return tuple((ctypes.c_float * 3)(*[float(v) for v in stats[key][:3]]) for key in ("mean", "std"))
+
+
+def _cuda_device(t):
+    """The device of ``t`` when it is a CUDA device, else the current CUDA device."""
+    if t.is_cuda:
+        return t.device
+    if not torch.cuda.is_available():
+        raise _native.MmbError("libmmbridge has no CPU path: post-processing and the jet features need a CUDA device")
+    return torch.device("cuda", torch.cuda.current_device())
+
+
+def _rows(t, name):
+    """[n, K] f32 CUDA tensor -> ([n, K] view with unit column stride, row stride)."""
+    if t.dim() != 2 or t.dtype != torch.float32 or not t.is_cuda:
+        raise _native.MmbError(f"{name} takes [n, K] float32 CUDA tensors; there is no CPU path")
+    if t.stride(1) != 1 or (t.shape[0] > 1 and t.stride(0) < t.shape[1]):
+        t = t.contiguous()
+    return t, t.stride(0) if t.shape[0] > 1 else t.shape[1]
+
+
 def jet_observables(x, k_u8, mask_u8, stats=None, want_particles=True):
     """x [B,N,3] f32, k/mask [B,N] u8 on the GPU -> (x_phys [B,N,3] | None, flavor_charge [B,N,2] int8 | None, jets [B,11])."""
     _native._require_cuda(x, k_u8, mask_u8)
@@ -32,10 +57,7 @@ def jet_observables(x, k_u8, mask_u8, stats=None, want_particles=True):
     x_phys = torch.empty_like(x) if want_particles else None
     fc = torch.empty(B, N, 2, dtype=torch.int8, device=dev) if want_particles else None
     jets = torch.empty(B, len(JET_COLUMNS), dtype=torch.float32, device=dev)
-    mean = std = None
-    if stats is not None:
-        mean = (ctypes.c_float * 3)(*[float(v) for v in stats["mean"][:3]])
-        std = (ctypes.c_float * 3)(*[float(v) for v in stats["std"][:3]])
+    mean, std = _stats_arrays(stats)
     with torch.cuda.device(dev):
         _native.check(_native.load().mmb_jet_observables(_native._ptr(x), _native._ptr(k_u8), _native._ptr(mask_u8), mean, std, B, N,
                                                          _native._ptr(x_phys), _native._ptr(fc), _native._ptr(jets), _native._stream()))
@@ -55,24 +77,11 @@ def jet_substructure(x, mask_u8, stats=None, R=0.8, beta=1.0, want_axes=False):
     dev = x.device
     out = torch.empty(B, len(SUBSTRUCTURE_COLUMNS), dtype=torch.float32, device=dev)
     axes = torch.empty(B, 6, dtype=torch.int16, device=dev) if want_axes else None
-    mean = std = None
-    if stats is not None:
-        mean = (ctypes.c_float * 3)(*[float(v) for v in stats["mean"][:3]])
-        std = (ctypes.c_float * 3)(*[float(v) for v in stats["std"][:3]])
+    mean, std = _stats_arrays(stats)
     with torch.cuda.device(dev):
         _native.check(_native.load().mmb_jet_substructure(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(R), float(beta),
                                                           _native._ptr(out), _native._ptr(axes), _native._stream()))
     return (out, axes) if want_axes else out
-
-
-def _rows(t):
-    """[n] or [n, K] f32 CUDA tensor -> ([n, K] view with unit column stride, row stride)."""
-    if t.dtype != torch.float32 or not t.is_cuda:
-        raise _native.MmbError("wasserstein1d takes float32 CUDA tensors; there is no CPU path")
-    t = t.reshape(-1, 1) if t.dim() == 1 else t
-    if t.stride(1) != 1 or (t.shape[0] > 1 and t.stride(0) < t.shape[1]):
-        t = t.contiguous()
-    return t, t.stride(0) if t.shape[0] > 1 else t.shape[1]
 
 
 def wasserstein1d(x, y, return_counts=False):
@@ -80,8 +89,8 @@ def wasserstein1d(x, y, return_counts=False):
     scipy.stats.wasserstein_distance of the finite values of each column, NaN when a sample has none (DESIGN.md §4.6c).
     ``return_counts``: also the numbers of finite x and y values, [2, K] int64 ([2] for 1-D inputs)."""
     one = x.dim() == 1
-    x2, ldx = _rows(x)
-    y2, ldy = _rows(y)
+    x2, ldx = _rows(x.reshape(-1, 1) if one else x, "wasserstein1d")
+    y2, ldy = _rows(y.reshape(-1, 1) if y.dim() == 1 else y, "wasserstein1d")
     if x2.device != y2.device or x2.shape[1] != y2.shape[1]:
         raise _native.MmbError(f"wasserstein1d: x {tuple(x.shape)} on {x.device} and y {tuple(y.shape)} on {y.device} do not match")
     (n, K), m = x2.shape, y2.shape[0]
@@ -166,10 +175,7 @@ def _efp_call(name, columns, x, mask_u8, stats, beta):
     B, N, _ = x.shape
     dev = x.device
     out = torch.empty(B, columns, dtype=torch.float32, device=dev)
-    mean = std = None
-    if stats is not None:
-        mean = (ctypes.c_float * 3)(*[float(v) for v in stats["mean"][:3]])
-        std = (ctypes.c_float * 3)(*[float(v) for v in stats["std"][:3]])
+    mean, std = _stats_arrays(stats)
     with torch.cuda.device(dev):
         _native.check(getattr(_native.load(), name)(_native._ptr(x), _native._ptr(mask_u8), mean, std, B, N, float(beta),
                                                     _native._ptr(out), _native._stream()))
@@ -215,16 +221,6 @@ def jetnet_fpd_features(x, mask_u8, stats=None):
     return out[:, _FPD_PICK].contiguous()
 
 
-def _metric_rows(t, name):
-    if t.dim() != 2 or t.dtype != torch.float32 or not t.is_cuda:
-        raise _native.MmbError(f"{name} takes [n, d] float32 CUDA tensors; there is no CPU path")
-    if t.shape[1] > 64:
-        raise _native.MmbError(f"{name}: d = {t.shape[1]} exceeds 64 features")
-    if t.stride(1) != 1 or (t.shape[0] > 1 and t.stride(0) < t.shape[1]):
-        t = t.contiguous()
-    return t, t.stride(0) if t.shape[0] > 1 else t.shape[1]
-
-
 def _index(idx):
     return idx.to(torch.int32).contiguous()
 
@@ -232,7 +228,7 @@ def _index(idx):
 def sampled_moments(x, idx, scale=None):
     """x [n, d] f32, idx [draws, rows] (row indices) on the GPU -> (sum [draws, d], sum of x x^T [draws, d, d]) in f64 on the
     device, every value taken as x * scale (``scale`` [d] f32, None for 1; the product is exact in fp64)."""
-    x2, ldx = _metric_rows(x, "sampled_moments")
+    x2, ldx = _rows(x, "sampled_moments")
     (n, d), (draws, rows) = x2.shape, idx.shape
     idx = _index(idx)
     sums = torch.empty(draws, d, dtype=torch.float64, device=x2.device)
@@ -268,8 +264,8 @@ def _frechet(m1, c1, m2, c2):
 def kpd_mmd(real, gen, idx_real, idx_gen, scale=None, degree=KPD_DEGREE):
     """Per batch t: the unbiased MMD^2 between real[idx_real[t]] and gen[idx_gen[t]] (B rows each) with the polynomial kernel
     k(x, y) = (x . y / d + 1)^degree, in fp64 -> [batches] f64 on the device."""
-    r2, ldr = _metric_rows(real, "kpd_mmd")
-    g2, ldg = _metric_rows(gen, "kpd_mmd")
+    r2, ldr = _rows(real, "kpd_mmd")
+    g2, ldg = _rows(gen, "kpd_mmd")
     if r2.shape[1] != g2.shape[1] or r2.device != g2.device or idx_real.shape != idx_gen.shape:
         raise _native.MmbError(f"kpd_mmd: real {tuple(real.shape)}, gen {tuple(gen.shape)}, indices {tuple(idx_real.shape)} / "
                                f"{tuple(idx_gen.shape)} do not match")
@@ -419,11 +415,7 @@ class ParticleClouds:
         return self.continuous.shape[0]
 
     def _run(self, stats):
-        dev = self.continuous.device
-        if dev.type != "cuda":
-            if not torch.cuda.is_available():
-                raise _native.MmbError("post-processing needs a CUDA device: libmmbridge has no CPU path")
-            dev = torch.device("cuda", torch.cuda.current_device())
+        dev = _cuda_device(self.continuous)
         x = self.continuous.to(dev, torch.float32).contiguous()
         return jet_observables(x, as_u8(self.discrete.to(dev)), as_u8(self.mask.to(dev)), stats)
 
@@ -459,7 +451,7 @@ class JetClassHighLevelFeatures:
         jets = constituents._jets
         if jets is None:   # constituents already in physical units (no postprocess call): one pass without de-standardisation
             c = constituents
-            dev = c.continuous.device if c.continuous.is_cuda else torch.device("cuda", torch.cuda.current_device())
+            dev = _cuda_device(c.continuous)
             tokens = c.discrete if c.discrete.shape[-1] == 1 else None
             if tokens is None:
                 raise NotImplementedError("construct from token-valued clouds or call postprocess() first")
@@ -478,7 +470,7 @@ class JetClassHighLevelFeatures:
         ``tau3``, ``tau21``, ``tau32`` and ``d2`` over the jets with at least 3 used particles (the others are dropped, as
         the reference drops them), so that ``Wassertein1D("tau21", other)`` compares them."""
         c = self.constituents
-        dev = c.continuous.device if c.continuous.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        dev = _cuda_device(c.continuous)
         out, axes = jet_substructure(c.continuous.to(dev, torch.float32).contiguous(), as_u8(c.mask.to(dev)), None, R, beta,
                                      want_axes=True)
         keep = axes[:, 0] >= 0
@@ -491,7 +483,7 @@ class JetClassHighLevelFeatures:
         attributes of ``EFP_COLUMNS`` over the jets with at least one used particle, so that
         ``wasserstein1d(reference, EFP_COLUMNS[1:])`` is W1-EFP and ``Wassertein1D("efp4_square", other)`` compares one."""
         c = self.constituents
-        dev = c.continuous.device if c.continuous.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        dev = _cuda_device(c.continuous)
         out = energy_flow_polynomials(c.continuous.to(dev, torch.float32).contiguous(), as_u8(c.mask.to(dev)), None, beta)
         out = out[~torch.isnan(out[:, 0])].to(c.continuous.device)
         for i, name in enumerate(EFP_COLUMNS):
@@ -501,7 +493,7 @@ class JetClassHighLevelFeatures:
         """{feature: W1 between this sample and ``reference``} on the device (``wasserstein1d``), one host synchronisation;
         the same values as ``Wassertein1D(feature, reference)``.  tau1, tau2, tau3, tau21, tau32 and d2 need
         ``compute_substructure`` on both objects; they cover fewer jets, so features are grouped by length (one call each)."""
-        dev = self.pt.device if self.pt.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        dev = _cuda_device(self.pt)
         col = lambda obj, f: getattr(obj, f).reshape(-1).to(dev, torch.float32)
         groups = {}
         for f in features:

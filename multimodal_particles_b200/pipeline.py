@@ -8,19 +8,21 @@ particles.py:85-89,124-156, jets.py:90-107) and the validation histograms (``mmb
 per-GPU int64 counts.  Exchanges (SURVEY.md §8e): the packed micro-batch (1 792 B / jet) goes to every rank once per micro-batch,
 on a side stream under the next micro-batch's generation — pushed over NVLink peer memory by the copy engines
 (``sharding.PeerGather``; one NCCL all-gather where peer memory is unavailable) — and one all-reduce of the histograms and of the
-jet-observable sums at the end.  With ``substructure=True`` the side stream also runs ``mmb_jet_substructure`` on every micro-batch
-and histograms tau21, tau32 and D2 into int64 counts of their own (SUBSTRUCTURE_BINS).  With ``w1_reference`` the side stream
-keeps the W1_COLUMNS of every jet; after the timed window they are all-gathered and scored against the reference with
-``mmb_wasserstein1d`` (``reference_observables`` builds an independent reference sample).  With ``efp=True`` the side stream
-also runs ``mmb_energy_flow_polynomials``; their columns join the W1 columns, and with a reference the five d = 4 EFPs are also
-scored by FPD and KPD (``observables.fpd`` / ``kpd``) after the timed window.  With ``particle_reference`` the side stream copies the
-post-processed particles of the jets JetNet's W1-P draws (``observables.jetnet_draws``, made before the window) into one buffer;
-after the window the buffers of the ranks are summed and scored with ``observables.w1p`` (``reference_particles`` builds the
-reference), and with ``w1_reference`` W1-M and W1-EFP are scored from the gathered jet columns.  With ``fpd_reference`` the side
-stream also runs ``mmb_energy_flow_polynomials_d4`` and keeps JetNet's FPD / KPD features (``observables.jetnet_fpd_features``,
-every EFP of degree <= 4) of every jet; after the window they are gathered and scored with ``fpd`` and ``kpd``
-(``reference_fpd_features`` builds the reference).  The reference has no multi-GPU code
-(SURVEY.md §2.1); ``tools/million_jets.py`` and the multi-GPU arms of ``bench.py`` call this.
+jet-observable sums at the end.  ``_jet_features`` runs the per-jet kernels of a micro-batch for the side stream and the
+reference builders alike; its outputs feed additive sums (zeroed after the warm-up and all-reduced in the timed window as one
+list), one per-jet row buffer in jet order (gathered after the window by ``_gather_rows``) or the particle draw buffers.  With
+``substructure=True`` the side stream also runs ``mmb_jet_substructure`` on every micro-batch and histograms tau21, tau32 and D2
+into int64 counts of their own (SUBSTRUCTURE_BINS).  With ``w1_reference`` the row buffer holds the W1_COLUMNS of every jet;
+after the timed window they are scored against the reference with ``mmb_wasserstein1d`` (``reference_observables`` builds an
+independent reference sample).  With ``efp=True`` the side stream also runs ``mmb_energy_flow_polynomials``; their columns join
+the W1 columns, and with a reference the five d = 4 EFPs are also scored by FPD and KPD (``observables.fpd`` / ``kpd``) after the
+timed window.  With ``particle_reference`` the side stream copies the post-processed particles of the jets JetNet's W1-P draws
+(``observables.jetnet_draws``, made before the window) into one buffer; after the window the buffers of the ranks are summed and
+scored with ``observables.w1p`` (``reference_particles`` builds the reference), and with ``w1_reference`` W1-M and W1-EFP are
+scored from the gathered jet columns.  With ``fpd_reference`` the side stream also runs ``mmb_energy_flow_polynomials_d4`` and
+JetNet's FPD / KPD features (``observables.jetnet_fpd_features``, every EFP of degree <= 4) of every jet follow the W1 columns in
+the row buffer; after the window they are scored with ``fpd`` and ``kpd`` (``reference_fpd_features`` builds the reference).  The
+reference has no multi-GPU code (SURVEY.md §2.1); ``tools/million_jets.py`` and the multi-GPU arms of ``bench.py`` call this.
 """
 import hashlib
 
@@ -56,10 +58,24 @@ def _w1_index(device):
             torch.tensor([SUBSTRUCTURE_COLUMNS.index(c) for c in W1_SUBSTRUCTURE_COLUMNS], device=device))
 
 
-def _w1_rows(jets, sub, index, efps=None):
-    """[B, K] f32: the W1 columns of one micro-batch from its jet_observables (and jet_substructure, energy_flow_polynomials)
-    rows."""
-    rows = [jets.index_select(1, index[0])] + ([sub.index_select(1, index[1])] if sub is not None else []) + ([efps] if efps is not None else [])
+def _jet_features(x, k, m, stats, particles=False, substructure=False, efp=False, fpd=False):
+    """The per-jet kernels on one micro-batch, each only when wanted: (x_phys [B,N,3] | None, jets [B,11], sub [B,8] | None,
+    efps [B,6] | None, fpd [B, len(FPD_EFP_COLUMNS)] | None) from ``jet_observables`` (post-processed particles with
+    ``particles``), ``jet_substructure``, ``energy_flow_polynomials`` and ``jetnet_fpd_features``."""
+    x_phys, _, jets = jet_observables(x, k, m, stats, want_particles=particles)
+    return (x_phys, jets, jet_substructure(x, m, stats) if substructure else None, energy_flow_polynomials(x, m, stats) if efp else None,
+            jetnet_fpd_features(x, m, stats) if fpd else None)
+
+
+def _rows(features, index, w1=True):
+    """[B, K] f32: one micro-batch's per-jet rows from its ``_jet_features``: with ``w1`` the W1 columns (those computed of
+    ``w1_columns``), then FPD_EFP_COLUMNS when they were computed."""
+    _, jets, sub, efps, fpd_features = features
+    rows = []
+    if w1:
+        rows += [jets.index_select(1, index[0])] + ([sub.index_select(1, index[1])] if sub is not None else []) + ([efps] if efps is not None else [])
+    if fpd_features is not None:
+        rows.append(fpd_features)
     return rows[0] if len(rows) == 1 else torch.cat(rows, 1)
 
 
@@ -89,10 +105,6 @@ class SubstructureHistograms:
         b = torch.where(undefined, float(nb), b).long() + self.offset
         self.counts.scatter_add_(0, b.reshape(-1), torch.ones(b.numel(), dtype=torch.int64, device=sub.device))
         self.sums.add_(torch.where(undefined, 0.0, v).double().sum(0))
-
-    def zero_(self):
-        self.counts.zero_()
-        self.sums.zero_()
 
 
 def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_batch=4096, n_particles=128, precision="auto",
@@ -125,12 +137,12 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     jet_sums = torch.zeros(11, dtype=torch.float64, device=device)
     sub_hist = SubstructureHistograms(device) if substructure else None
     efp_sums = torch.zeros(len(EFP_COLUMNS) + 1, dtype=torch.float64, device=device) if efp else None   # sums, then defined jets
+    # the additive accumulators: zeroed after the warm-up, all-reduced inside the timed window
+    additive = [counts, jet_sums] + ([sub_hist.counts, sub_hist.sums] if substructure else []) + ([efp_sums] if efp else [])
     w1_cols = w1_columns(substructure, efp)
-    if w1_reference is not None:
-        if w1_reference.dim() != 2 or w1_reference.shape[1] != len(w1_cols):
-            raise ValueError(f"w1_reference must be [m, {len(w1_cols)}] ({', '.join(w1_cols)}), got {tuple(w1_reference.shape)}")
-        w1_buf = torch.empty(hi - lo, len(w1_cols), dtype=torch.float32, device=device)   # this rank's jets, in jet order
-        w1_index = _w1_index(device)
+    n_w1 = len(w1_cols) if w1_reference is not None else 0
+    if w1_reference is not None and (w1_reference.dim() != 2 or w1_reference.shape[1] != len(w1_cols)):
+        raise ValueError(f"w1_reference must be [m, {len(w1_cols)}] ({', '.join(w1_cols)}), got {tuple(w1_reference.shape)}")
     if particle_reference is not None:
         p_ref_x, p_ref_m = particle_reference
         if p_ref_x.dim() != 3 or tuple(p_ref_x.shape[1:]) != (N, 3) or p_ref_m.shape[:2] != p_ref_x.shape[:2]:
@@ -141,7 +153,11 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     if fpd_reference is not None:
         if fpd_reference.dim() != 2 or fpd_reference.shape[1] != len(FPD_EFP_COLUMNS):
             raise ValueError(f"fpd_reference must be [m, {len(FPD_EFP_COLUMNS)}] (FPD_EFP_COLUMNS), got {tuple(fpd_reference.shape)}")
-        fpd_buf = torch.empty(hi - lo, len(FPD_EFP_COLUMNS), dtype=torch.float32, device=device)   # this rank's jets, in jet order
+    # per-jet rows of this rank's jets in jet order: the W1 columns (with w1_reference), then FPD_EFP_COLUMNS (with fpd_reference)
+    n_rows = n_w1 + (len(FPD_EFP_COLUMNS) if fpd_reference is not None else 0)
+    rows = torch.empty(hi - lo, n_rows, dtype=torch.float32, device=device) if n_rows else None
+    w1_index = _w1_index(device)
+    want = dict(particles=particle_reference is not None, substructure=substructure, efp=efp, fpd=fpd_reference is not None)
     packs = [sharding.PackedJets(MB, N, 3, device) for _ in range(3)]      # state of a micro-batch: [x | tokens | mask], one allocation
     recv = [sharding.make_gather(MB, N, 3, world, device, mode=gather) for _ in range(2)] if world > 1 else None
     side = torch.cuda.Stream(device=device)
@@ -165,26 +181,23 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
             ev.record(main_s)
             with torch.cuda.stream(side):
                 side.wait_event(ev)
-                x_phys, _, jets = jet_observables(x, k, m, STATS, want_particles=particle_reference is not None)
+                features = _jet_features(x, k, m, STATS, **want)
+                x_phys, jets, sub, efps, _ = features
                 counts.add_(hist.accumulate(x, k, m))
                 jet_sums.add_(torch.nan_to_num(jets.double()).sum(0))
-                sub = jet_substructure(x, m, STATS) if substructure else None
                 if substructure:
                     sub_hist.add(sub)
-                efps = energy_flow_polynomials(x, m, STATS) if efp else None
                 if efp:
                     defined = ~torch.isnan(efps[:, :1])
                     efp_sums.add_(torch.cat([torch.where(defined, efps, 0.0).double().sum(0), defined.double().sum(0)]))
-                if w1_reference is not None:
-                    w1_buf[start - lo:start - lo + B].copy_(_w1_rows(jets, sub, w1_index, efps))
+                if rows is not None:
+                    rows[start - lo:start - lo + B].copy_(_rows(features, w1_index, w1=w1_reference is not None))
                 if particle_reference is not None:
                     a, b = p_plan["ranges"][start]
                     if b > a:   # the draw slots of this micro-batch's jets (ranges made on the host before the window)
                         sel, jet = p_plan["slot"][a:b], p_plan["jet"][a:b] - start
                         p_x.index_copy_(0, sel, x_phys.index_select(0, jet))
                         p_m.index_copy_(0, sel, m.index_select(0, jet))
-                if fpd_reference is not None:
-                    fpd_buf[start - lo:start - lo + B].copy_(jetnet_fpd_features(x, m, STATS))
                 if world > 1 and B == MB:
                     recv[i & 1].gather(pk)          # the packed micro-batch to every rank (copy-engine push, or one all-gather)
                 for t in (x, k, m):
@@ -194,12 +207,8 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         main_s.wait_stream(side)
 
     run(lo, min(hi, lo + warmup_batches * MB))       # warm-up, then reset the accumulators
-    counts.zero_()
-    jet_sums.zero_()
-    if substructure:
-        sub_hist.zero_()
-    if efp:
-        efp_sums.zero_()
+    for acc in additive:
+        acc.zero_()
     torch.cuda.synchronize(device)
     if world > 1:
         dist.barrier()
@@ -207,22 +216,14 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
     s.record(main_s)
     run(lo, hi)
     if world > 1:
-        dist.all_reduce(counts)
-        dist.all_reduce(jet_sums)
-        if substructure:
-            dist.all_reduce(sub_hist.counts)
-            dist.all_reduce(sub_hist.sums)
-        if efp:
-            dist.all_reduce(efp_sums)
+        for acc in additive:
+            dist.all_reduce(acc)
     e.record(main_s)
     torch.cuda.synchronize(device)
     t = torch.tensor([s.elapsed_time(e)], dtype=torch.float64, device=device)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    if w1_reference is not None:
-        w1_all = _gather_rows(w1_buf, total_jets, world, device) if world > 1 else w1_buf
-    if fpd_reference is not None:
-        fpd_all = _gather_rows(fpd_buf, total_jets, world, device) if world > 1 else fpd_buf
+    all_rows = _gather_rows(rows, total_jets, world, device) if rows is not None and world > 1 else rows
     if particle_reference is not None and world > 1:   # every draw slot has one owner; the other ranks hold zeros
         dist.all_reduce(p_x)
         dist.all_reduce(p_m)
@@ -254,17 +255,20 @@ def sharded_generation_run(model, cfg, total_jets, rank, world, device, micro_ba
         es = efp_sums.tolist()
         for name, v in zip(EFP_COLUMNS, es):
             rec[f"mean_{name}"] = v / es[-1] if es[-1] else float("nan")
+    w1_all, w1_ref = None, None
     if w1_reference is not None:
-        reference = w1_reference.to(device, torch.float32)
-        rec.update(_score_w1(w1_all, reference, w1_cols))
-        if efp:
-            rec.update(_score_efp_metrics(w1_all, reference, w1_cols))
+        w1_all, w1_ref = all_rows[:, :n_w1], w1_reference.to(device, torch.float32)
+        rec.update(_score_w1(w1_all, w1_ref, w1_cols))
+        if efp:   # the five d = 4 EFPs
+            pick = [w1_cols.index(c) for c in EFP_COLUMNS[1:]]
+            rec.update(_score_fpd_kpd(w1_all[:, pick], w1_ref[:, pick], "fpd", "kpd", "jet_metrics_seconds"))
     if particle_reference is not None:
-        rec.update(_score_jetnet_w1(p_ref_x.to(device, torch.float32), p_ref_m.to(device), p_x, p_m, p_plan["idx_real"],
-                                    w1_all if w1_reference is not None else None,
-                                    w1_reference.to(device, torch.float32) if w1_reference is not None else None, w1_cols, efp))
+        rec.update(_score_jetnet_w1(p_ref_x.to(device, torch.float32), p_ref_m.to(device), p_x, p_m, p_plan["idx_real"], w1_all, w1_ref,
+                                    w1_cols, efp))
     if fpd_reference is not None:
-        rec.update(_score_jetnet_fpd(fpd_all, fpd_reference.to(device, torch.float32)))
+        rec.update(_score_fpd_kpd(all_rows[:, n_w1:], fpd_reference.to(device, torch.float32), "jetnet_fpd", "jetnet_kpd",
+                                  "jetnet_fpd_seconds"))
+        rec["jetnet_fpd_reference_jets"] = int(fpd_reference.shape[0])
     return rec
 
 
@@ -279,27 +283,36 @@ def _particle_plan(n_reference, total, lo, hi, micro_batch, device):
             "ranges": {int(a): (cut[i], cut[i + 1]) for i, a in enumerate(starts[:-1].tolist())}}
 
 
+def _timed(device, fn):
+    """(fn(), seconds between CUDA events recorded on the current stream around it); ends in a synchronise."""
+    stream = torch.cuda.current_stream(device)
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record(stream)
+    out = fn()
+    e.record(stream)
+    torch.cuda.synchronize(device)
+    return out, s.elapsed_time(e) * 1e-3
+
+
 def _score_jetnet_w1(ref_x, ref_m, gen_x, gen_m, idx_real, jet_values, jet_reference, cols, efp):
     """W1-P of the gathered draw slots against the reference particles (``observables.w1p`` with the run's draws), and with jet
     columns W1-M and W1-EFP (``observables.w1m`` / ``w1efp``).  The CUDA events span all of them, including the host reading
     each call's per-draw values and the numpy aggregation between the calls, so the time is that of the whole scoring."""
-    stream = torch.cuda.current_stream(gen_x.device)
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record(stream)
-    slots = torch.arange(gen_x.shape[0], dtype=torch.int32, device=gen_x.device).reshape(idx_real.shape)
-    vals = wasserstein1d_drawn(ref_x, idx_real, gen_x, slots, ref_m, gen_m).cpu().numpy()
-    rec = {"w1p": list(w1_summary(vals)),
-           "w1p_features": {c: [float(a), float(b)] for c, a, b in zip(PARTICLE_COLUMNS, *w1_summary(vals, average=False))}}
-    if jet_values is not None:
-        m = cols.index("m")
-        rec["w1m"] = list(w1m(jet_reference[:, m], jet_values[:, m]))
-        if efp:
-            pick = [cols.index(c) for c in EFP_COLUMNS[1:]]
-            rec["w1efp"] = list(w1efp(jet_reference[:, pick], jet_values[:, pick]))
-    e.record(stream)
-    torch.cuda.synchronize(gen_x.device)
-    rec["jetnet_w1_seconds"] = s.elapsed_time(e) * 1e-3
-    return rec
+    def score():
+        slots = torch.arange(gen_x.shape[0], dtype=torch.int32, device=gen_x.device).reshape(idx_real.shape)
+        vals = wasserstein1d_drawn(ref_x, idx_real, gen_x, slots, ref_m, gen_m).cpu().numpy()
+        rec = {"w1p": list(w1_summary(vals)),
+               "w1p_features": {c: [float(a), float(b)] for c, a, b in zip(PARTICLE_COLUMNS, *w1_summary(vals, average=False))}}
+        if jet_values is not None:
+            m = cols.index("m")
+            rec["w1m"] = list(w1m(jet_reference[:, m], jet_values[:, m]))
+            if efp:
+                pick = [cols.index(c) for c in EFP_COLUMNS[1:]]
+                rec["w1efp"] = list(w1efp(jet_reference[:, pick], jet_values[:, pick]))
+        return rec
+
+    rec, seconds = _timed(gen_x.device, score)
+    return dict(rec, jetnet_w1_seconds=seconds)
 
 
 def _gather_rows(buf, total, world, device):
@@ -314,44 +327,17 @@ def _gather_rows(buf, total, world, device):
 
 
 def _score_w1(values, reference, cols):
-    stream = torch.cuda.current_stream(values.device)
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record(stream)
-    w1, used = wasserstein1d(values, reference, return_counts=True)
-    e.record(stream)
-    torch.cuda.synchronize(values.device)
+    (w1, used), seconds = _timed(values.device, lambda: wasserstein1d(values, reference, return_counts=True))
     w1, used = w1.tolist(), used.tolist()
     return {"w1": dict(zip(cols, w1)), "w1_used": {c: [used[0][i], used[1][i]] for i, c in enumerate(cols)},
-            "w1_reference_jets": int(reference.shape[0]), "w1_seconds": s.elapsed_time(e) * 1e-3}
+            "w1_reference_jets": int(reference.shape[0]), "w1_seconds": seconds}
 
 
-def _score_efp_metrics(values, reference, cols):
-    """FPD and KPD (observables.fpd / kpd at their defaults) of the five d = 4 EFP columns of the gathered rows against the
-    reference's, timed by CUDA events around both."""
-    pick = [cols.index(c) for c in EFP_COLUMNS[1:]]
-    gen, real = values[:, pick], reference[:, pick]
-    stream = torch.cuda.current_stream(values.device)
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record(stream)
-    f = fpd(real, gen)
-    k = kpd(real, gen)
-    e.record(stream)
-    torch.cuda.synchronize(values.device)
-    return {"fpd": list(f), "kpd": list(k), "jet_metrics_seconds": s.elapsed_time(e) * 1e-3}
-
-
-def _score_jetnet_fpd(values, reference):
-    """FPD and KPD (observables.fpd / kpd at their defaults) of the gathered FPD_EFP_COLUMNS rows against the reference's, timed
-    by CUDA events around both."""
-    stream = torch.cuda.current_stream(values.device)
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record(stream)
-    f = fpd(reference, values)
-    k = kpd(reference, values)
-    e.record(stream)
-    torch.cuda.synchronize(values.device)
-    return {"jetnet_fpd": list(f), "jetnet_kpd": list(k), "jetnet_fpd_reference_jets": int(reference.shape[0]),
-            "jetnet_fpd_seconds": s.elapsed_time(e) * 1e-3}
+def _score_fpd_kpd(values, reference, fpd_key, kpd_key, seconds_key):
+    """FPD and KPD (observables.fpd / kpd at their defaults) of the gathered rows against the reference's, timed by CUDA events
+    around both."""
+    (f, k), seconds = _timed(values.device, lambda: (fpd(reference, values), kpd(reference, values)))
+    return {fpd_key: list(f), kpd_key: list(k), seconds_key: seconds}
 
 
 def _reference_jets(model, n_jets, device, N, jet_offset, micro_batch, precision):
@@ -368,6 +354,15 @@ def _reference_jets(model, n_jets, device, N, jet_offset, micro_batch, precision
         yield start, x, k, m
 
 
+def _reference(model, n_jets, device, n_particles, jet_offset, micro_batch, precision, stats, outs, pick, **want):
+    """Fills ``outs`` ([n_jets, ...] tensors) in jet order with ``pick(features, mask)`` of each micro-batch of ``_reference_jets``,
+    ``features`` being its ``_jet_features(**want)``, so that a reference is made as the run makes its own values."""
+    for start, x, k, m in _reference_jets(model, n_jets, device, n_particles, jet_offset, micro_batch, precision):
+        for out, v in zip(outs, pick(_jet_features(x, k, m, stats, **want), m)):
+            out[start:start + x.shape[0]] = v
+    return outs
+
+
 def reference_observables(model, cfg, n_jets, device, n_particles=128, substructure=False, jet_offset=1 << 40, micro_batch=16384,
                           precision="auto", stats=STATS, efp=False):
     """[n_jets, K] f32 on ``device``: the ``w1_columns(substructure, efp)`` of ``n_jets`` jets made as ``sharded_generation_run`` makes
@@ -376,11 +371,8 @@ def reference_observables(model, cfg, n_jets, device, n_particles=128, substruct
     the de-standardisation of the observables."""
     out = torch.empty(n_jets, len(w1_columns(substructure, efp)), dtype=torch.float32, device=device)
     index = _w1_index(device)
-    for start, x, k, m in _reference_jets(model, n_jets, device, n_particles, jet_offset, micro_batch, precision):
-        B = x.shape[0]
-        _, _, jets = jet_observables(x, k, m, stats, want_particles=False)
-        out[start:start + B] = _w1_rows(jets, jet_substructure(x, m, stats) if substructure else None, index,
-                                        energy_flow_polynomials(x, m, stats) if efp else None)
+    _reference(model, n_jets, device, n_particles, jet_offset, micro_batch, precision, stats, [out], lambda f, m: [_rows(f, index)],
+               substructure=substructure, efp=efp)
     return out
 
 
@@ -390,14 +382,9 @@ def reference_particles(model, cfg, n_jets, device, n_particles=128, jet_offset=
     ``jet_offset + j``); the particle reference of ``sharded_generation_run(particle_reference=...)``.  ``jet_offset=0``
     reproduces the run's own jets."""
     N = n_particles
-    out_x = torch.empty(n_jets, N, 3, dtype=torch.float32, device=device)
-    out_m = torch.empty(n_jets, N, dtype=torch.uint8, device=device)
-    for start, x, k, m in _reference_jets(model, n_jets, device, N, jet_offset, micro_batch, precision):
-        B = x.shape[0]
-        x_phys, _, _ = jet_observables(x, k, m, stats)
-        out_x[start:start + B] = x_phys
-        out_m[start:start + B] = m
-    return out_x, out_m
+    outs = [torch.empty(n_jets, N, 3, dtype=torch.float32, device=device), torch.empty(n_jets, N, dtype=torch.uint8, device=device)]
+    return tuple(_reference(model, n_jets, device, N, jet_offset, micro_batch, precision, stats, outs, lambda f, m: [f[0], m],
+                            particles=True))
 
 
 def reference_fpd_features(model, cfg, n_jets, device, n_particles=128, jet_offset=1 << 40, micro_batch=16384, precision="auto",
@@ -406,6 +393,5 @@ def reference_fpd_features(model, cfg, n_jets, device, n_particles=128, jet_offs
     ``reference_observables`` makes them (Philox jet offsets ``jet_offset + j``); the reference of
     ``sharded_generation_run(fpd_reference=...)``.  ``jet_offset=0`` reproduces the run's own jets."""
     out = torch.empty(n_jets, len(FPD_EFP_COLUMNS), dtype=torch.float32, device=device)
-    for start, x, _, m in _reference_jets(model, n_jets, device, n_particles, jet_offset, micro_batch, precision):
-        out[start:start + x.shape[0]] = jetnet_fpd_features(x, m, stats)
+    _reference(model, n_jets, device, n_particles, jet_offset, micro_batch, precision, stats, [out], lambda f, m: [f[4]], fpd=True)
     return out

@@ -2,17 +2,13 @@
 tests/efp_d4_oracle.py, bit-identity of the columns it shares with mmb_energy_flow_polynomials, special jets, the stats path,
 determinism, argument errors, and JetNet's FPD / KPD on these features in the sharded generation run."""
 import ctypes
-import json
-import os
-import socket
 
 import numpy as np
 import pytest
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
 
 import efp_d4_oracle as do
+from pipeline_lib import one_gpu_run, two_gpu_run
 
 DEV = "cuda:0"
 REL = 1e-5
@@ -117,13 +113,6 @@ TOTAL, REF_JETS = 3 * 16384, 20000
 NEW_KEYS = {"jetnet_fpd", "jetnet_kpd", "jetnet_fpd_reference_jets", "jetnet_fpd_seconds"}
 
 
-def _run(model, cfg, total, micro_batch, **kw):
-    import bench
-    from multimodal_particles_b200.pipeline import sharded_generation_run
-    return sharded_generation_run(model, cfg, total, 0, 1, torch.device(DEV), micro_batch=micro_batch, n_particles=bench.N_PART,
-                                  warmup_batches=1, **kw)
-
-
 def _same_except_time(a, b):
     assert set(a) == set(b)
     for key, val in a.items():
@@ -141,9 +130,9 @@ def test_sharded_run_jetnet_fpd_kpd():
     cfg, model = bench.build_model(dev_)
     ref = reference_fpd_features(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART)
     assert ref.shape == (REF_JETS, len(FPD_EFP_COLUMNS)) and ref.dtype == torch.float32
-    base = _run(model, cfg, TOTAL, 16384)
-    big = _run(model, cfg, TOTAL, 16384, fpd_reference=ref)
-    small = _run(model, cfg, TOTAL, 4096, fpd_reference=ref)
+    base = one_gpu_run(model, cfg, TOTAL, 16384)
+    big = one_gpu_run(model, cfg, TOTAL, 16384, fpd_reference=ref)
+    small = one_gpu_run(model, cfg, TOTAL, 4096, fpd_reference=ref)
     assert set(big) - set(base) == NEW_KEYS
     _same_except_time(base, {k: v for k, v in big.items() if k not in NEW_KEYS})      # the d <= 4 pass changes nothing else
     for key in ("jetnet_fpd", "jetnet_kpd"):
@@ -154,8 +143,8 @@ def test_sharded_run_jetnet_fpd_kpd():
     assert list(fpd(ref, same)) == big["jetnet_fpd"] and list(kpd(ref, same)) == big["jetnet_kpd"]
     # the existing EFP metrics are the same with and without the d <= 4 features
     w1_ref = reference_observables(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, efp=True)
-    efp_plain = _run(model, cfg, TOTAL, 16384, w1_reference=w1_ref, efp=True)
-    efp_both = _run(model, cfg, TOTAL, 16384, w1_reference=w1_ref, efp=True, fpd_reference=ref)
+    efp_plain = one_gpu_run(model, cfg, TOTAL, 16384, w1_reference=w1_ref, efp=True)
+    efp_both = one_gpu_run(model, cfg, TOTAL, 16384, w1_reference=w1_ref, efp=True, fpd_reference=ref)
     _same_except_time(efp_plain, {k: v for k, v in efp_both.items() if k not in NEW_KEYS})
     assert efp_both["jetnet_fpd"] == big["jetnet_fpd"] and efp_both["jetnet_kpd"] == big["jetnet_kpd"]
     # an independent reference of the same model is within a few errors of 0; one with 25 % wider jets is far
@@ -163,34 +152,15 @@ def test_sharded_run_jetnet_fpd_kpd():
     assert fv <= 5 * fe + 1e-9 and abs(kv) <= 5 * ke + 1e-9, (big["jetnet_fpd"], big["jetnet_kpd"])
     shifted = dict(PIPE_STATS, std=[PIPE_STATS["std"][0], 0.25, 0.25])
     ref_shift = reference_fpd_features(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, stats=shifted)
-    far = _run(model, cfg, TOTAL, 16384, fpd_reference=ref_shift)
+    far = one_gpu_run(model, cfg, TOTAL, 16384, fpd_reference=ref_shift)
     assert far["jetnet_fpd"][0] > 10 * (fv + fe), (far["jetnet_fpd"], big["jetnet_fpd"])
     assert far["jetnet_kpd"][0] > 10 * (abs(kv) + ke), (far["jetnet_kpd"], big["jetnet_kpd"])
 
 
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
-def _two_gpu_worker(rank, world, port, out_path):
+def _two_gpu_kwargs(model, cfg, dev_):
     import bench
-    from multimodal_particles_b200.pipeline import reference_fpd_features, sharded_generation_run
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    torch.cuda.set_device(rank)
-    dev_ = torch.device("cuda", rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev_)
-    try:
-        cfg, model = bench.build_model(dev_)
-        ref = reference_fpd_features(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART)
-        rec = sharded_generation_run(model, cfg, TOTAL + 5, rank, world, dev_, micro_batch=16384, n_particles=bench.N_PART,
-                                     warmup_batches=1, fpd_reference=ref)
-        if rank == 0:
-            with open(out_path, "w") as f:
-                json.dump({k: rec[k] for k in ("jetnet_fpd", "jetnet_kpd")}, f)
-    finally:
-        dist.destroy_process_group()
+    from multimodal_particles_b200.pipeline import reference_fpd_features
+    return dict(fpd_reference=reference_fpd_features(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART))
 
 
 @pytest.mark.gpu
@@ -199,12 +169,8 @@ def test_two_gpu_jetnet_fpd_kpd_equal_one_gpu(tmp_path):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
     import bench
-    from multimodal_particles_b200.pipeline import reference_fpd_features
-    out = str(tmp_path / "metrics.json")
-    mp.spawn(_two_gpu_worker, args=(2, _free_port(), out), nprocs=2, join=True)
-    two = json.load(open(out))
+    two = two_gpu_run(tmp_path, TOTAL + 5, _two_gpu_kwargs, ("jetnet_fpd", "jetnet_kpd"))
     dev_ = torch.device(DEV)
     cfg, model = bench.build_model(dev_)
-    ref = reference_fpd_features(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART)
-    one = _run(model, cfg, TOTAL + 5, 16384, fpd_reference=ref)
+    one = one_gpu_run(model, cfg, TOTAL + 5, 16384, **_two_gpu_kwargs(model, cfg, dev_))
     assert two["jetnet_fpd"] == one["jetnet_fpd"] and two["jetnet_kpd"] == one["jetnet_kpd"]

@@ -1,16 +1,11 @@
 """FPD and KPD on the device: mmb_sampled_moments / mmb_kpd_mmd against the numpy statements of tests/efp_oracle.py on the same
 injected draws, determinism, the metrics' sensitivity, and the EFP metrics of the sharded generation run."""
-import json
-import os
-import socket
-
 import numpy as np
 import pytest
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
 
 import efp_oracle as eo
+from pipeline_lib import one_gpu_run, two_gpu_run
 
 DEV = "cuda:0"
 
@@ -128,13 +123,6 @@ TOTAL, REF_JETS = 3 * 16384, 20000
 METRIC_KEYS = ("w1", "w1_used", "fpd", "kpd")
 
 
-def _run(model, cfg, total, micro_batch, **kw):
-    import bench
-    from multimodal_particles_b200.pipeline import sharded_generation_run
-    return sharded_generation_run(model, cfg, total, 0, 1, torch.device(DEV), micro_batch=micro_batch, n_particles=bench.N_PART,
-                                  warmup_batches=1, **kw)
-
-
 @pytest.mark.gpu
 def test_sharded_run_efp_metrics():
     import bench
@@ -145,10 +133,10 @@ def test_sharded_run_efp_metrics():
     ref = reference_observables(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, efp=True)
     cols = w1_columns(False, True)
     assert ref.shape == (REF_JETS, len(cols)) and cols[-6:] == EFP_COLUMNS
-    base = _run(model, cfg, TOTAL, 16384)
-    plain = _run(model, cfg, TOTAL, 16384, w1_reference=ref[:, :len(w1_columns())])
-    big = _run(model, cfg, TOTAL, 16384, w1_reference=ref, efp=True)
-    small = _run(model, cfg, TOTAL, 4096, w1_reference=ref, efp=True)
+    base = one_gpu_run(model, cfg, TOTAL, 16384)
+    plain = one_gpu_run(model, cfg, TOTAL, 16384, w1_reference=ref[:, :len(w1_columns())])
+    big = one_gpu_run(model, cfg, TOTAL, 16384, w1_reference=ref, efp=True)
+    small = one_gpu_run(model, cfg, TOTAL, 4096, w1_reference=ref, efp=True)
     for key, val in base.items():                                    # the EFP pass changes nothing else
         if key not in ("seconds", "value"):
             assert big[key] == val, key
@@ -165,34 +153,15 @@ def test_sharded_run_efp_metrics():
     from multimodal_particles_b200.pipeline import STATS
     shifted = dict(STATS, std=[STATS["std"][0], 0.25, 0.25])
     ref_shift = reference_observables(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, stats=shifted, efp=True)
-    far = _run(model, cfg, TOTAL, 16384, w1_reference=ref_shift, efp=True)
+    far = one_gpu_run(model, cfg, TOTAL, 16384, w1_reference=ref_shift, efp=True)
     assert far["fpd"][0] > 10 * (big["fpd"][0] + big["fpd"][1]), (far["fpd"], big["fpd"])
     assert far["kpd"][0] > 10 * (abs(big["kpd"][0]) + big["kpd"][1]), (far["kpd"], big["kpd"])
 
 
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
-def _two_gpu_worker(rank, world, port, out_path):
+def _two_gpu_kwargs(model, cfg, dev_):
     import bench
-    from multimodal_particles_b200.pipeline import reference_observables, sharded_generation_run
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    torch.cuda.set_device(rank)
-    dev_ = torch.device("cuda", rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev_)
-    try:
-        cfg, model = bench.build_model(dev_)
-        ref = reference_observables(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, efp=True)
-        rec = sharded_generation_run(model, cfg, TOTAL + 5, rank, world, dev_, micro_batch=16384, n_particles=bench.N_PART,
-                                     warmup_batches=1, w1_reference=ref, efp=True)
-        if rank == 0:
-            with open(out_path, "w") as f:
-                json.dump({k: rec[k] for k in METRIC_KEYS}, f)
-    finally:
-        dist.destroy_process_group()
+    from multimodal_particles_b200.pipeline import reference_observables
+    return dict(w1_reference=reference_observables(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, efp=True), efp=True)
 
 
 @pytest.mark.gpu
@@ -201,13 +170,9 @@ def test_two_gpu_efp_metrics_equal_one_gpu(tmp_path):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
     import bench
-    from multimodal_particles_b200.pipeline import reference_observables
-    out = str(tmp_path / "metrics.json")
-    mp.spawn(_two_gpu_worker, args=(2, _free_port(), out), nprocs=2, join=True)
-    two = json.load(open(out))
+    two = two_gpu_run(tmp_path, TOTAL + 5, _two_gpu_kwargs, METRIC_KEYS)
     dev_ = torch.device(DEV)
     cfg, model = bench.build_model(dev_)
-    ref = reference_observables(model, cfg, REF_JETS, dev_, n_particles=bench.N_PART, efp=True)
-    one = _run(model, cfg, TOTAL + 5, 16384, w1_reference=ref, efp=True)
+    one = one_gpu_run(model, cfg, TOTAL + 5, 16384, **_two_gpu_kwargs(model, cfg, dev_))
     assert two["w1"] == one["w1"] and two["w1_used"] == {c: list(v) for c, v in one["w1_used"].items()}
     assert two["fpd"] == one["fpd"] and two["kpd"] == one["kpd"]

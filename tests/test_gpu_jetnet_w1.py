@@ -3,7 +3,6 @@ drawn sample, agreement with scipy, determinism under repeats and permutations, 
 and W1-P, W1-M and W1-EFP of the sharded generation run."""
 import json
 import os
-import socket
 import subprocess
 import sys
 
@@ -11,8 +10,8 @@ import numpy as np
 import pytest
 import scipy.stats
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
+
+from pipeline_lib import one_gpu_run, two_gpu_run
 
 DEV = "cuda:0"
 
@@ -227,13 +226,6 @@ def test_jetnet_functions_aggregate_the_draws():
 TOTAL, REF_JETS = 3 * 16384, 20000
 
 
-def _run(model, cfg, total, micro_batch, **kw):
-    import bench
-    from multimodal_particles_b200.pipeline import sharded_generation_run
-    return sharded_generation_run(model, cfg, total, 0, 1, torch.device(DEV), micro_batch=micro_batch, n_particles=bench.N_PART,
-                                  warmup_batches=1, **kw)
-
-
 def _references(model, cfg, dev):
     import bench
     from multimodal_particles_b200.pipeline import reference_observables, reference_particles
@@ -250,9 +242,9 @@ def test_sharded_run_jetnet_w1():
     cfg, model = bench.build_model(dev)
     ref_jets, ref_parts = _references(model, cfg, dev)
     assert ref_parts[0].shape == (REF_JETS, bench.N_PART, 3) and ref_parts[1].shape == (REF_JETS, bench.N_PART)
-    base = _run(model, cfg, TOTAL, 16384, efp=True, w1_reference=ref_jets)
-    big = _run(model, cfg, TOTAL, 16384, efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
-    small = _run(model, cfg, TOTAL, 4096, efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
+    base = one_gpu_run(model, cfg, TOTAL, 16384, efp=True, w1_reference=ref_jets)
+    big = one_gpu_run(model, cfg, TOTAL, 16384, efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
+    small = one_gpu_run(model, cfg, TOTAL, 4096, efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
     new = {"w1p", "w1p_features", "w1m", "w1efp", "jetnet_w1_seconds"}
     assert set(big) == set(base) | new and not new & set(base)
     for key, val in base.items():                                   # the particle collection changes nothing else
@@ -277,7 +269,7 @@ def test_sharded_run_jetnet_w1():
         v = x[..., i][msk]
         assert big["w1p_features"][c][0] < 0.05 * (np.quantile(v, 0.9) - np.quantile(v, 0.1)), c
     # without a W1 reference only W1-P joins
-    only = _run(model, cfg, TOTAL, 16384, particle_reference=ref_parts)
+    only = one_gpu_run(model, cfg, TOTAL, 16384, particle_reference=ref_parts)
     assert "w1m" not in only and "w1efp" not in only and only["w1p"] == big["w1p"]
 
 
@@ -295,29 +287,9 @@ def test_million_jets_tool_with_both_references(tmp_path):
     assert all(np.isfinite(rec[k]).all() for k in ("w1p", "w1m", "w1efp"))
 
 
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
-def _two_gpu_worker(rank, world, port, out_path):
-    import bench
-    from multimodal_particles_b200.pipeline import sharded_generation_run
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    torch.cuda.set_device(rank)
-    dev = torch.device("cuda", rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
-    try:
-        cfg, model = bench.build_model(dev)
-        ref_jets, ref_parts = _references(model, cfg, dev)
-        rec = sharded_generation_run(model, cfg, TOTAL + 5, rank, world, dev, micro_batch=16384, n_particles=bench.N_PART,
-                                     warmup_batches=1, efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
-        if rank == 0:
-            with open(out_path, "w") as f:
-                json.dump({k: rec[k] for k in ("w1p", "w1p_features", "w1m", "w1efp")}, f)
-    finally:
-        dist.destroy_process_group()
+def _two_gpu_kwargs(model, cfg, dev):
+    ref_jets, ref_parts = _references(model, cfg, dev)
+    return dict(efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
 
 
 @pytest.mark.gpu
@@ -326,11 +298,9 @@ def test_two_gpu_jetnet_w1_equals_one_gpu(tmp_path):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
     import bench
-    out = str(tmp_path / "jetnet_w1.json")
-    mp.spawn(_two_gpu_worker, args=(2, _free_port(), out), nprocs=2, join=True)
-    two = json.load(open(out))
+    keys = ("w1p", "w1p_features", "w1m", "w1efp")
+    two = two_gpu_run(tmp_path, TOTAL + 5, _two_gpu_kwargs, keys)
     dev = torch.device(DEV)
     cfg, model = bench.build_model(dev)
-    ref_jets, ref_parts = _references(model, cfg, dev)
-    one = _run(model, cfg, TOTAL + 5, 16384, efp=True, w1_reference=ref_jets, particle_reference=ref_parts)
-    assert two == json.loads(json.dumps({k: one[k] for k in ("w1p", "w1p_features", "w1m", "w1efp")}))
+    one = one_gpu_run(model, cfg, TOTAL + 5, 16384, **_two_gpu_kwargs(model, cfg, dev))
+    assert two == json.loads(json.dumps({k: one[k] for k in keys}))

@@ -2,16 +2,13 @@
 against scipy on the same float32 data, determinism, argument errors, the JetClassHighLevelFeatures mirror and the W1 of the
 sharded generation run (GPU)."""
 import ctypes
-import json
-import os
-import socket
 
 import numpy as np
 import pytest
 import scipy.stats
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
+
+from pipeline_lib import one_gpu_run, two_gpu_run
 
 DEV = "cuda:0"
 REL, ABS = 1e-9, 1e-12
@@ -201,13 +198,6 @@ def test_mirror_class_equals_wassertein1d():
     assert a.wasserstein1d(a, ("pt", "tau21")) == {"pt": 0.0, "tau21": 0.0}
 
 
-def _run(model, cfg, total, micro_batch, **kw):
-    import bench
-    from multimodal_particles_b200.pipeline import sharded_generation_run
-    return sharded_generation_run(model, cfg, total, 0, 1, torch.device(DEV), micro_batch=micro_batch, n_particles=bench.N_PART,
-                                  warmup_batches=1, **kw)
-
-
 TOTAL, REF_JETS = 3 * 16384, 20000
 
 
@@ -221,9 +211,9 @@ def test_sharded_run_w1():
     ref = reference_observables(model, cfg, REF_JETS, dev, n_particles=bench.N_PART, substructure=True)
     cols = w1_columns(True)
     assert ref.shape == (REF_JETS, len(cols))
-    base = _run(model, cfg, TOTAL, 16384, substructure=True)
-    big = _run(model, cfg, TOTAL, 16384, substructure=True, w1_reference=ref)
-    small = _run(model, cfg, TOTAL, 4096, substructure=True, w1_reference=ref)
+    base = one_gpu_run(model, cfg, TOTAL, 16384, substructure=True)
+    big = one_gpu_run(model, cfg, TOTAL, 16384, substructure=True, w1_reference=ref)
+    small = one_gpu_run(model, cfg, TOTAL, 4096, substructure=True, w1_reference=ref)
     for key, val in base.items():                                   # the W1 collection changes nothing else
         if key not in ("seconds", "value"):
             assert big[key] == val, key
@@ -244,33 +234,14 @@ def test_sharded_run_w1():
     # a reference with a harder particle pT scale is far away in jet pT
     shifted = dict(STATS, mean=[STATS["mean"][0] + 0.3] + STATS["mean"][1:])
     ref_shift = reference_observables(model, cfg, REF_JETS, dev, n_particles=bench.N_PART, stats=shifted)
-    far = _run(model, cfg, TOTAL, 16384, w1_reference=ref_shift)
+    far = one_gpu_run(model, cfg, TOTAL, 16384, w1_reference=ref_shift)
     assert far["w1"]["pt"] > 10 * big["w1"]["pt"]
 
 
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
-def _two_gpu_worker(rank, world, port, out_path):
+def _two_gpu_kwargs(model, cfg, dev):
     import bench
-    from multimodal_particles_b200.pipeline import reference_observables, sharded_generation_run
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    torch.cuda.set_device(rank)
-    dev = torch.device("cuda", rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
-    try:
-        cfg, model = bench.build_model(dev)
-        ref = reference_observables(model, cfg, REF_JETS, dev, n_particles=bench.N_PART, substructure=True)
-        rec = sharded_generation_run(model, cfg, TOTAL + 5, rank, world, dev, micro_batch=16384, n_particles=bench.N_PART,
-                                     warmup_batches=1, substructure=True, w1_reference=ref)
-        if rank == 0:
-            with open(out_path, "w") as f:
-                json.dump({"w1": rec["w1"], "w1_used": rec["w1_used"]}, f)
-    finally:
-        dist.destroy_process_group()
+    from multimodal_particles_b200.pipeline import reference_observables
+    return dict(substructure=True, w1_reference=reference_observables(model, cfg, REF_JETS, dev, n_particles=bench.N_PART, substructure=True))
 
 
 @pytest.mark.gpu
@@ -279,12 +250,8 @@ def test_two_gpu_w1_equals_one_gpu(tmp_path):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
     import bench
-    from multimodal_particles_b200.pipeline import reference_observables
-    out = str(tmp_path / "w1.json")
-    mp.spawn(_two_gpu_worker, args=(2, _free_port(), out), nprocs=2, join=True)
-    two = json.load(open(out))
+    two = two_gpu_run(tmp_path, TOTAL + 5, _two_gpu_kwargs, ("w1", "w1_used"))
     dev = torch.device(DEV)
     cfg, model = bench.build_model(dev)
-    ref = reference_observables(model, cfg, REF_JETS, dev, n_particles=bench.N_PART, substructure=True)
-    one = _run(model, cfg, TOTAL + 5, 16384, substructure=True, w1_reference=ref)
+    one = one_gpu_run(model, cfg, TOTAL + 5, 16384, **_two_gpu_kwargs(model, cfg, dev))
     assert two["w1"] == one["w1"] and two["w1_used"] == {c: list(v) for c, v in one["w1_used"].items()}

@@ -24,9 +24,8 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
-from multimodal_particles_b200.observables import jet_observables, wasserstein1d  # noqa: E402
-from multimodal_particles_b200.pipeline import STATS, _target_multiplicity, reference_observables, w1_columns  # noqa: E402
-from multimodal_particles_b200.source import sample_source_state  # noqa: E402
+from multimodal_particles_b200.observables import wasserstein1d  # noqa: E402
+from multimodal_particles_b200.pipeline import reference_observables, reference_particles, w1_columns  # noqa: E402
 
 REF_OFFSET = 1 << 40
 
@@ -41,19 +40,10 @@ def card():
     return name, q
 
 
-def particles(model, n_jets, dev, jet_offset, micro_batch=16384):
+def particles(model, cfg, n_jets, dev, jet_offset):
     """[live particles, 3] f32 (pt, eta, phi in physical units) of the jets generated as reference_observables makes them."""
-    native, table, N = model.encoder.native_model(dev), model.step_table(), bench.N_PART
-    mult_hist = _target_multiplicity(N)
-    parts = []
-    for start in range(0, n_jets, micro_batch):
-        B = min(micro_batch, n_jets - start)
-        x, k, m = sample_source_state(B, N, target_multiplicity=mult_hist, min_num_particles=0, device=dev, seed=7,
-                                      jet_offset=jet_offset + start, compact=True)
-        native.generate(x, k, m, table, seed=11, jet_offset=jet_offset + start)
-        x_phys, _, _ = jet_observables(x, k, m, STATS)
-        parts.append(x_phys[m.bool()])
-    return torch.cat(parts)
+    x, m = reference_particles(model, cfg, n_jets, dev, n_particles=bench.N_PART, jet_offset=jet_offset)
+    return x[m.bool()]
 
 
 def device_time(x, y, iters):
@@ -121,7 +111,7 @@ def main():
                  "device_ms_by_kernel": split})
     del gen, ref
 
-    pg, pr = particles(model, args.jets, dev, 0), particles(model, args.jets, dev, REF_OFFSET)
+    pg, pr = particles(model, cfg, args.jets, dev, 0), particles(model, cfg, args.jets, dev, REF_OFFSET)
     dev_s, got = device_time(pg, pr, args.iters)
     cpu_s, want = scipy_time(pg[:, :1].cpu().numpy(), pr[:, :1].cpu().numpy(), [0])
     rows.append({"level": "particle", "columns": ["pt", "eta", "phi"], "n": pg.shape[0], "m": pr.shape[0], "device_s": dev_s,
