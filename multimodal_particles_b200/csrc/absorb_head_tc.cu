@@ -42,84 +42,14 @@
 
 #include "mmb_device.cuh"
 #include "mmb_internal.h"
+#include "tcgen05.cuh"
 
 namespace mmb {
 namespace {
 
 constexpr int kC = 128;            // transformer width this kernel is built for
 constexpr int kHeads = 2;            // 64 channels per head
-constexpr int kSlot = 36864;       // bytes per streamed matrix: 32 KB weight tile + 4 KB bias tile
 constexpr int kMaxBlocks = 4;
-
-// ---- PTX wrappers (same conventions as epic_tc.cu) ----------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t slot_smem, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot_smem), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// one lane of a converged warp
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// 32 consecutive fp32 columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-    uint32_t r[32];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr) : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46);
-}
-__host__ __device__ constexpr uint32_t instr_desc(int M, int N, bool b_mn) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | (b_mn ? (1u << 16) : 0u) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-    __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&h);
-}
 
 // fp32 side table (floats), per block then the per-particle output vector
 struct HeadTable {
@@ -269,50 +199,6 @@ __device__ __forceinline__ float tanh_fast(float a) {
     asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(a));
     return t;
 }
-__device__ __forceinline__ float ex2_fast(float a) {
-    float t;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(a));
-    return t;
-}
-
-// Sum `vals[0..CNT)` over the 32 lanes of a warp by recursive halving: each stage exchanges half of the values a lane still
-// holds (CNT-1 shuffles in total instead of 5*CNT).  On return lane l holds, in vals[0], the warp total of the value whose index
-// has bit log2(CNT/2) = lane bit 4, ..., i.e. idx = sum_k ((l >> (4-k)) & 1) * (CNT >> (k+1)); CNT <= 32, a power of two.
-template <int CNT>
-__device__ __forceinline__ void warp_halving_sum(float (&vals)[CNT], int lane) {
-    int off = 16;
-#pragma unroll
-    for (int cnt = CNT; cnt > 1; cnt >>= 1, off >>= 1) {
-        const bool upper = (lane & off) != 0;
-#pragma unroll
-        for (int i = 0; i < cnt / 2; ++i) {
-            const float keep = upper ? vals[cnt / 2 + i] : vals[i];
-            const float send = upper ? vals[i] : vals[cnt / 2 + i];
-            vals[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-        }
-    }
-    for (; off >= 1; off >>= 1) vals[0] += __shfl_xor_sync(0xffffffffu, vals[0], off);
-}
-template <int CNT>
-__device__ __forceinline__ int warp_halving_index(int lane) {
-    int idx = 0, off = 16;
-#pragma unroll
-    for (int cnt = CNT; cnt > 1; cnt >>= 1, off >>= 1) idx += (lane & off) ? cnt / 2 : 0;
-    return idx;
-}
-
-__device__ __forceinline__ void tmem_ldw(uint32_t taddr, float (&v)[32]) { tmem_ld32(taddr, v); }
-// [128 rows x 128 k] bf16 tile, K-major canonical: 8-row groups 2048 B apart (SBO), 16-byte k-chunks 128 B apart (LBO).
-// thread `row` stores columns [col, col + CW) of its row
-template <int CW>
-__device__ __forceinline__ void store_row(uint8_t* tile, int row, int col, const float (&v)[CW]) {
-    uint8_t* p = tile + (row >> 3) * 2048 + (row & 7) * 16 + (col >> 3) * 128;
-#pragma unroll
-    for (int c = 0; c < CW / 8; ++c)
-        *reinterpret_cast<uint4*>(p + c * 128) = make_uint4(pack_bf16(v[8 * c], v[8 * c + 1]), pack_bf16(v[8 * c + 2], v[8 * c + 3]),
-                                                            pack_bf16(v[8 * c + 4], v[8 * c + 5]), pack_bf16(v[8 * c + 6], v[8 * c + 7]));
-}
-__device__ __forceinline__ void named_bar(int id, int threads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
 
 // One CTA owns one TILE at a time: 128 rows = up to four jets in 32-row quarters (see the header).  Thread (r, cq): row r = TMEM
 // lane r (warp & 3 selects the lane quarter the warp may touch), channel slice cq = warp >> 2 -> kCW consecutive accumulator
@@ -379,14 +265,14 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
     const uint32_t wbase = smem_u32(smem);
     // Ring slot 0 = [bias tile | weight tile], slot 1 = [weight tile | bias tile]: the two weight tiles are adjacent in shared
     // memory, so a pair of streamed matrices can be consumed as ONE [256 x 128] B operand (the fused q/k GEMM).
-    auto w_addr = [&](uint32_t slot) { return wbase + (slot ? kSlot : 4096u); };
-    auto b_addr = [&](uint32_t slot) { return wbase + (slot ? kSlot + 32768u : 0u); };
+    auto w_addr = [&](uint32_t slot) { return wbase + (slot ? kSlot : kSlot - kSlotBias); };
+    auto b_addr = [&](uint32_t slot) { return wbase + (slot ? kSlot + kSlotBias : 0u); };
     auto issue_load = [&](uint32_t i) {  // thread 0 only
         const uint32_t bar = (i & 1) ? bar_full1 : bar_full0;
         const uint8_t* src = p.image + (size_t)(i % n_seq) * kSlot;
         mbar_expect_tx(bar, kSlot);
-        bulk_g2s(w_addr(i & 1), src, 32768, bar);
-        bulk_g2s(b_addr(i & 1), src + 32768, 4096, bar);
+        bulk_g2s(w_addr(i & 1), src, kSlotBias, bar);
+        bulk_g2s(b_addr(i & 1), src + kSlotBias, kSlot - kSlotBias, bar);
     };
     if (tid == 0) {
         if (total_mats > 0) issue_load(0);
@@ -454,7 +340,7 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
     auto group_norm_to_A = [&](uint32_t d_src, const float* bias /*nullable, smem, per segment*/, const float* gamma, const float* beta,
                                bool swish) {
         float v[CW];
-        tmem_ldw(d_src + lane_off + col0, v);
+        tmem_ld32(d_src + lane_off + col0, v);
         if (bias) {
 #pragma unroll
             for (int j = 0; j < CW; j += 4) {
@@ -746,9 +632,9 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
             if (blk == 0) STK_TRACE(8);
             {   // both tiles in one epilogue phase
                 float v[CW];
-                tmem_ldw(dACC + q_half * 128 + lane_off + col0, v);
+                tmem_ld32(dACC + q_half * 128 + lane_off + col0, v);
                 store_row<CW>(sQ, r, col0, v);
-                tmem_ldw(dACC + (q_half ^ 1) * 128 + lane_off + col0, v);
+                tmem_ld32(dACC + (q_half ^ 1) * 128 + lane_off + col0, v);
                 store_row<CW>(sK, r, col0, v);
                 tc_fence_before();
                 fence_proxy_async();
@@ -788,7 +674,7 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
 #pragma unroll 1
                 for (int c = 0; c < 2; ++c) {
                     if (!((mine >> c) & 1u)) continue;
-                    tmem_ldw(dS + c * CW, v);
+                    tmem_ld32(dS + c * CW, v);
                     if ((weighted >> c) & 1u) {   // keys of weight 0 (unused rows) leave the maximum: + (-3e38)
 #pragma unroll
                         for (int j = 0; j < CW; j += 4) {
@@ -812,7 +698,7 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
 #pragma unroll 1
                 for (int c = 0; c < 2; ++c) {
                     if ((mine >> c) & 1u) {
-                        tmem_ldw(dS + c * CW, v);
+                        tmem_ld32(dS + c * CW, v);
                         if ((weighted >> c) & 1u) {   // P_j = w_j exp(.) = exp2(. + log2 w_j); w_j = 0 -> exp2(-inf) = 0
 #pragma unroll
                             for (int j = 0; j < CW; j += 4) {
@@ -845,7 +731,7 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
                 tc_fence_after();
                 if (tid == 0 && wseq + 2 < total_mats) issue_load(wseq + 2);
                 ++wseq;
-                tmem_ldw(dACC + lane_off + col0, v);
+                tmem_ld32(dACC + lane_off + col0, v);
                 if (seg < 0) {
 #pragma unroll
                     for (int j = 0; j < CW; ++j) v[j] = 0.0f;     // V rows of an empty quarter meet zero columns of P, but 0 x NaN is NaN
@@ -879,7 +765,7 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
 #pragma unroll
                 for (int i = 0; i < HQ; ++i) tot += s_sum[h * HQ + i][r];
                 const float rinv = tot > 0.0f ? 1.0f / tot : 0.0f;    // empty quarter: no keys
-                tmem_ldw(dACC + lane_off + col0, v);
+                tmem_ld32(dACC + lane_off + col0, v);
 #pragma unroll
                 for (int j = 0; j < CW; j += 2) fmul2(v[j], v[j + 1], v[j], v[j + 1], rinv, rinv);
                 store_row<CW>(sA, r, col0, v);
@@ -899,7 +785,7 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
         {
             const float* w = sTab + HeadTable::rate_w(nblk);
             float v[CW], a0 = 0.0f, a1 = 0.0f;
-            tmem_ldw(dX + lane_off + col0, v);
+            tmem_ld32(dX + lane_off + col0, v);
 #pragma unroll
             for (int j = 0; j < CW; j += 4) {
                 const float4 w4 = *reinterpret_cast<const float4*>(w + col0 + j);
@@ -949,9 +835,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
     if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-// element (row o, k) of a K-major tile with 8-row groups `sbo` bytes apart -> bf16 index
-inline size_t tile_index(int o, int k, int sbo) { return ((size_t)(o / 8) * sbo + (size_t)(k / 8) * 128 + (o % 8) * 16 + (k % 8) * 2) / 2; }
-
 }  // namespace
 
 // ---- host side: one transformer stack = operand image + side table (+ optional per-jet head) --------------------------
@@ -977,14 +860,10 @@ int tf_stack_build(TfStack* st, const float* proj_in, int Cin, const float* bloc
     std::vector<float> tab((size_t)HeadTable::floats(n_blocks), 0.0f);
     auto put_matrix = [&](int slot, const float* Wm, int in_dim) {
         for (int o = 0; o < C; ++o)
-            for (int k = 0; k < in_dim; ++k) img[(size_t)slot * kSlot / 2 + tile_index(o, k, 2048)] = __float2bfloat16(Wm[(size_t)o * in_dim + k]);
+            for (int k = 0; k < in_dim; ++k) slot_put_weight(img, slot, o, k, Wm[(size_t)o * in_dim + k]);
     };
     auto put_bias = [&](int slot, const float* b) {
-        for (int o = 0; o < C; ++o) {
-            const __nv_bfloat16 hi = __float2bfloat16(b[o]);
-            img[(size_t)slot * kSlot / 2 + 32768 / 2 + tile_index(o, 0, 256)] = hi;
-            img[(size_t)slot * kSlot / 2 + 32768 / 2 + tile_index(o, 1, 256)] = __float2bfloat16(b[o] - __bfloat162float(hi));
-        }
+        for (int o = 0; o < C; ++o) slot_put_bias(img, slot, o, b[o]);
     };
     put_matrix(0, proj_in, Cin);
     put_bias(0, proj_in + (size_t)C * Cin);

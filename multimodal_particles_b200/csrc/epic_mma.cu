@@ -83,12 +83,6 @@ struct Lay {
 };
 
 // ---- small PTX wrappers ---------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ uint32_t pack2(float lo, float hi) {
-    __half2 h = __floats2half2_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&h);
-}
 // D = A * B + C (m16n8k16, fp16 in, fp32 accumulate); D and C are separate registers, so a shared bias quad needs no copy
 __device__ __forceinline__ void mma(float (&d)[4], const uint32_t (&a)[4], const uint2 b, const float4 c) {
     asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%11,%12,%13};"
@@ -102,9 +96,7 @@ __device__ __forceinline__ void mma_acc(float (&d)[4], const uint32_t (&a)[4], c
 __device__ __forceinline__ void ldmatrix_x4(uint32_t (&a)[4], uint32_t addr) {
     asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(a[0]), "=r"(a[1]), "=r"(a[2]), "=r"(a[3]) : "r"(addr));
 }
-__device__ __forceinline__ void jet_bar(int id, int threads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
 
-__device__ __forceinline__ float lrelu_f(float a) { return fmaxf(a, 0.01f * a); }
 __device__ __forceinline__ void lrelu4(float (&c)[4]) {
     float t0, t1, t2, t3;
     fmul2(t0, t1, c[0], c[1], 0.01f, 0.01f);
@@ -167,8 +159,8 @@ struct MmaParams {
 // rows 0-7 carry the vector; rows 8-15 are zero (their outputs are never read) unless `dup`, which makes all 16 rows equal
 // so that the OUTPUT quad {c0, c1, c2, c3} = {y[2t], y[2t+1], y[2t], y[2t+1]} can serve as a C operand for 16 particle rows.
 __device__ __forceinline__ void vec_frag(uint32_t (&a)[4], float v00, float v01, float v10, float v11, bool dup = false) {
-    a[0] = pack2(v00, v01);
-    a[2] = pack2(v10, v11);
+    a[0] = pack_f16(v00, v01);
+    a[2] = pack_f16(v10, v11);
     a[1] = dup ? a[0] : 0u;
     a[3] = dup ? a[2] : 0u;
 }
@@ -277,10 +269,10 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
         auto pack_rows = [&](uint32_t (&a)[NMT][4], const float (&v)[NMT][2][4]) {
 #pragma unroll
             for (int mt = 0; mt < NMT; ++mt) {
-                a[mt][0] = pack2(v[mt][0][0], v[mt][0][1]);
-                a[mt][1] = pack2(v[mt][0][2], v[mt][0][3]);
-                a[mt][2] = pack2(v[mt][1][0], v[mt][1][1]);
-                a[mt][3] = pack2(v[mt][1][2], v[mt][1][3]);
+                a[mt][0] = pack_f16(v[mt][0][0], v[mt][0][1]);
+                a[mt][1] = pack_f16(v[mt][0][2], v[mt][0][3]);
+                a[mt][2] = pack_f16(v[mt][1][0], v[mt][1][1]);
+                a[mt][3] = pack_f16(v[mt][1][2], v[mt][1][3]);
             }
         };
         // masked column sums of xl over the jet: this warp's rows by multiply-adds + xor butterfly, then the jet's other warps
@@ -307,7 +299,7 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
             }
             if (cls > 1) {
                 if (g == 0) *reinterpret_cast<float4*>(pool_mine + pp * 16 + 4 * t) = make_float4(s[0][0], s[0][1], s[1][0], s[1][1]);
-                jet_bar(bar_id, bar_threads);
+                named_bar(bar_id, bar_threads);
                 float4 acc = *reinterpret_cast<const float4*>(pool_jet + pp * 16 + 4 * t);
                 for (int w = 1; w < cls; ++w) {
                     const float4 q = *reinterpret_cast<const float4*>(pool_jet + w * kPoolFloats + pp * 16 + 4 * t);
@@ -343,9 +335,9 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
                     const uint32_t sel = live ? (0x3C00u << (16 * (kk & 1))) : 0u;
                     const int kw = kk >> 1;
                     uint32_t w[8];
-                    w[0] = pack2(hi[0], hi[1]);     // xs == 0 on dead rows
-                    w[1] = pack2(hi[2], lo[0]);
-                    w[2] = pack2(lo[1], lo[2]);
+                    w[0] = pack_f16(hi[0], hi[1]);     // xs == 0 on dead rows
+                    w[1] = pack_f16(hi[2], lo[0]);
+                    w[2] = pack_f16(lo[1], lo[2]);
 #pragma unroll
                     for (int i = 0; i < 4; ++i) w[3 + i] = (i < S / 2 && kw == i) ? sel : 0u;
                     w[7] = 0u;
@@ -388,15 +380,15 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
                     mma(c[j], a_mean, tile(LY::t_g0 + j), ctx_quad(1, j));
                     mma_acc(c[j], a_sum, tile(LY::t_g0 + 2 + j));
                 }
-                vec_frag(a, lrelu_f(c[0][0]), lrelu_f(c[0][1]), lrelu_f(c[1][0]), lrelu_f(c[1][1]));
+                vec_frag(a, lrelu_fast(c[0][0]), lrelu_fast(c[0][1]), lrelu_fast(c[1][0]), lrelu_fast(c[1][1]));
 #pragma unroll
                 for (int j = 0; j < 2; ++j) mma(c[j], a, tile(LY::t_g1 + j), quad(LY::v_g1, j));
-                vec_frag(a, lrelu_f(c[0][0]), lrelu_f(c[0][1]), lrelu_f(c[1][0]), lrelu_f(c[1][1]));
+                vec_frag(a, lrelu_fast(c[0][0]), lrelu_fast(c[0][1]), lrelu_fast(c[1][0]), lrelu_fast(c[1][1]));
 #pragma unroll
                 for (int j = 0; j < 2 * GT; ++j) {
                     float d[4];
                     mma(d, a, tile(LY::t_g2 + j), quad(LY::v_g2 + (j >> 1), j & 1));
-                    xg[j][0] = lrelu_f(d[0]); xg[j][1] = lrelu_f(d[1]);
+                    xg[j][0] = lrelu_fast(d[0]); xg[j][1] = lrelu_fast(d[1]);
                     skg[j][0] = skip_on ? xg[j][0] : 0.0f; skg[j][1] = skip_on ? xg[j][1] : 0.0f;
                 }
             }
@@ -422,7 +414,7 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
 #pragma unroll
                         for (int j = 0; j < 2; ++j) mma_acc(c[j], a, tl[(LY::o_g1 + 4 + 2 * gt + j) * 32]);
                     }
-                    vec_frag(a, lrelu_f(c[0][0]), lrelu_f(c[0][1]), lrelu_f(c[1][0]), lrelu_f(c[1][1]));
+                    vec_frag(a, lrelu_fast(c[0][0]), lrelu_fast(c[0][1]), lrelu_fast(c[1][0]), lrelu_fast(c[1][1]));
                     // fc_global2 + residual (epic.py:231-232), trunk skip (epic.py:155)
                     float xm[2 * GT][2];
 #pragma unroll
@@ -431,7 +423,7 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
                         b.x += xg[j][0]; b.y += xg[j][1];
                         float d[4];
                         mma(d, a, tl[(LY::o_g2 + j) * 32], b);
-                        xm[j][0] = lrelu_f(d[0]); xm[j][1] = lrelu_f(d[1]);
+                        xm[j][0] = lrelu_fast(d[0]); xm[j][1] = lrelu_fast(d[1]);
                         xg[j][0] = xm[j][0] + skg[j][0]; xg[j][1] = xm[j][1] + skg[j][1];
                     }
                     // per-jet part of fc_local1: time vector + Wl1[:, H:H+G] xg   (epic.py:233-238); all 16 rows equal, so the
@@ -500,8 +492,8 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
                     mma(hv, af[mt], wv, bv);
                     if constexpr (SH > 0) {
                         uint32_t az[4];
-                        az[0] = pack2(selu_f(hz[0]), selu_f(hz[1]));
-                        az[1] = pack2(selu_f(hz[2]), selu_f(hz[3]));
+                        az[0] = pack_f16(selu_f(hz[0]), selu_f(hz[1]));
+                        az[1] = pack_f16(selu_f(hz[2]), selu_f(hz[3]));
                         az[2] = az[3] = 0u;
                         mma(hz, az, w2, b2);
                     }
@@ -694,9 +686,9 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
                 if (cls > 1 && lane == 0) s_claim[team * cls] = idx;
             }
             if (cls > 1) {
-                jet_bar(team_barrier(cls, team), 32 * cls);
+                named_bar(team_barrier(cls, team), 32 * cls);
                 idx = s_claim[team * cls];
-                jet_bar(team_barrier(cls, team), 32 * cls);   // everyone has read the claim before the leader overwrites it
+                named_bar(team_barrier(cls, team), 32 * cls);   // everyone has read the claim before the leader overwrites it
             }
             if (idx >= n_key) break;
             const int jet = __ldg(p.lists + (size_t)key * p.B + idx);

@@ -45,6 +45,7 @@
 
 #include "mmb_device.cuh"
 #include "mmb_internal.h"
+#include "tcgen05.cuh"
 
 namespace mmb {
 namespace {
@@ -112,44 +113,9 @@ TcLayout make_layout(const MmbEpicDims& d) {
 // element (row, k) of a [16 x 16] K-major operand -> index in bf16 units
 inline int bop_index(int row, int k) { return (row / 8) * 128 + (k / 8) * 64 + (row % 8) * 8 + (k % 8); }
 
-// ---- PTX wrappers --------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// named_bar(id, 128) with the thread count as an immediate (named_bar passes it in a register)
 __device__ __forceinline__ void group_bar(int id) { asm volatile("bar.sync %0, 128;" ::"r"(id) : "memory"); }
 
-__device__ __forceinline__ void tmem_alloc(uint32_t slot_smem, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot_smem), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-
-// D[tmem] (+)= A[smem] * B[smem]^T, kind::f16 (bf16 in, fp32 accumulate); one thread issues
-// one lane of a converged warp
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
 // The pooling GEMM: up to eight K-steps (B descriptor advances by 512 B = 32 address units per step) into one accumulator.
 // All descriptors are formed before the first MMA so their moves to uniform registers can overlap; K-steps whose bit in
 // `live` is clear are skipped (their rows are all zero); the first issued step overwrites, the rest accumulate.
@@ -180,9 +146,6 @@ __device__ __forceinline__ void umma_pool8(uint32_t d_tmem, uint64_t adesc, uint
         "}"
         ::"r"(d_tmem), "l"(adesc), "l"(bdesc0), "r"(idesc), "r"(live), "r"(first), "l"(adesc_hi) : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
 
 // 16 consecutive fp32 columns of this thread's TMEM lane
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
@@ -194,22 +157,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
     for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// shared-memory matrix descriptor, no swizzle (SURVEY/DESIGN: bits 0-13 addr>>4, 16-29 LBO>>4,
-// 32-45 SBO>>4, 46-47 version=1, 61-63 layout=0)
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46);
-}
-// instruction descriptor kind::f16: D fp32 (bit 4), A/B bf16 (bits 7,10), N>>3 at 17, M>>4 at 24; b_mn = B is MN-major
-__host__ __device__ constexpr uint32_t instr_desc(int M, int N, bool b_mn) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | (b_mn ? (1u << 16) : 0u) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-    __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&h);
 }
 
 // this thread's 16-wide row -> its slot of the A operand (two 16-byte chunks, K-major canonical)
@@ -259,7 +206,6 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
     for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-__device__ __forceinline__ float lrelu_fast(float a) { return fmaxf(a, 0.01f * a); }
 // init + sum_{k<K} w[k * wstride] * x(k) with four independent accumulators: the serial per-jet global MLP is a chain of such
 // dots on one warp, and a single accumulator makes every one of them K dependent FMAs long
 // init + sum_k w[k] x[k] over K contiguous floats (K % 4 == 0); w and x 16-byte aligned shared memory: 128-bit loads

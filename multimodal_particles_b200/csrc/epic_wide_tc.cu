@@ -36,73 +36,17 @@
 
 #include "mmb_device.cuh"
 #include "mmb_internal.h"
+#include "tcgen05.cuh"
 
 namespace mmb {
 namespace {
 
 constexpr int kH = 128;
-constexpr int kSlot = 36864;        // bytes per streamed matrix: 32 KB weight tile + 4 KB bias tile
 constexpr int kThreads = 512;
 constexpr int kCW = 32;             // accumulator columns per thread
 constexpr int kMaxL = 8;
 
-// ---- PTX wrappers (same conventions as absorb_head_tc.cu) ---------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t slot_smem, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot_smem), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// 32 consecutive fp32 columns of this thread's TMEM lane: load / store
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-    uint32_t r[32];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr) : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
+// 32 consecutive fp32 columns of this thread's TMEM lane: store
 __device__ __forceinline__ void tmem_st32(uint32_t taddr, const float (&v)[32]) {
     asm volatile(
         "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
@@ -118,54 +62,10 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const float (&v)[32]) 
         : "memory");
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 }
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46);
-}
-__host__ __device__ constexpr uint32_t instr_desc(int M, int N) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-    __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&h);
-}
-__device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
-    __half2 h = __floats2half2_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&h);
-}
-// [128 rows x 128 k] bf16 tile, K-major canonical: 8-row groups 2048 B apart (SBO), 16-byte k-chunks 128 B apart (LBO)
-__device__ __forceinline__ void store_row(uint8_t* tile, int row, int col, const float (&v)[32]) {
-    uint8_t* p = tile + (row >> 3) * 2048 + (row & 7) * 16 + (col >> 3) * 128;
-#pragma unroll
-    for (int c = 0; c < 4; ++c)
-        *reinterpret_cast<uint4*>(p + c * 128) = make_uint4(pack_bf16(v[8 * c], v[8 * c + 1]), pack_bf16(v[8 * c + 2], v[8 * c + 3]),
-                                                            pack_bf16(v[8 * c + 4], v[8 * c + 5]), pack_bf16(v[8 * c + 6], v[8 * c + 7]));
-}
 // skip tile: fp16 [128 rows][128 cols], 256 B per row, 16-byte chunks XOR-swizzled by the row so that a quarter-warp (8 rows,
 // same chunk number) touches 8 different bank groups
 __device__ __forceinline__ uint4* skip_chunk(uint8_t* tile, int row, int chunk) {
     return reinterpret_cast<uint4*>(tile + row * 256 + ((chunk ^ (row & 7)) << 4));
-}
-// column sums over the 32 rows of a warp (recursive halving, 31 shuffles): on return lane l holds in vals[0] the total of
-// column halving_index(l)
-__device__ __forceinline__ void warp_halving_sum32(float (&vals)[32], int lane) {
-    int off = 16;
-#pragma unroll
-    for (int cnt = 32; cnt > 1; cnt >>= 1, off >>= 1) {
-        const bool upper = (lane & off) != 0;
-#pragma unroll
-        for (int i = 0; i < cnt / 2; ++i) {
-            const float keep = upper ? vals[cnt / 2 + i] : vals[i];
-            const float send = upper ? vals[i] : vals[cnt / 2 + i];
-            vals[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-        }
-    }
-}
-__device__ __forceinline__ int halving_index32(int lane) {
-    int idx = 0, off = 16;
-#pragma unroll
-    for (int cnt = 32; cnt > 1; cnt >>= 1, off >>= 1) idx += (lane & off) ? cnt / 2 : 0;
-    return idx;
 }
 __device__ __forceinline__ float lrelu(float a) { return a > 0.0f ? a : 0.01f * a; }
 __device__ __forceinline__ float selu(float a) {
@@ -417,7 +317,7 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
                 const uint64_t ad = smem_desc(smem_u32(sA(t)), 128, 2048), wd = smem_desc(wb, 128, 2048);
 #pragma unroll 8
                 for (int j = 0; j < nk; ++j) umma(d, ad + (uint64_t)(j * 16), wd + (uint64_t)(j * 16), idesc, (accumulate || j > 0) ? 1u : 0u);
-                if (bias) umma(d, ones_desc, smem_desc(wb + 32768, 128, 256), idesc, 1u);
+                if (bias) umma(d, ones_desc, smem_desc(wb + kSlotBias, 128, 256), idesc, 1u);
                 umma_commit(bar_mma[t]);
             }
             __syncwarp();
@@ -654,8 +554,8 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
                 }
                 store_row(sA(t), r, col0, v);
                 if (kind != 1) {   // column sums for the next pooling (unused rows are zero already)
-                    warp_halving_sum32(v, lane);
-                    sv[Vec::part + t * 16 * 32 + warp * 32 + halving_index32(lane)] = v[0];
+                    warp_halving_sum(v, lane);
+                    sv[Vec::part + t * 16 * 32 + warp * 32 + warp_halving_index<32>(lane)] = v[0];
                 }
             } else if (kind != 1) {
                 sv[Vec::part + t * 16 * 32 + warp * 32 + lane] = 0.0f;
@@ -824,9 +724,6 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
 
 __device__ long long g_wide_trace[32];
 
-// element (row o, k) of a K-major tile with 8-row groups `sbo` bytes apart -> bf16 index
-inline size_t tile_index(int o, int k, int sbo) { return ((size_t)(o / 8) * sbo + (size_t)(k / 8) * 128 + (o % 8) * 16 + (k % 8) * 2) / 2; }
-
 inline uint32_t host_pack_bf16(float lo, float hi) {
     const __nv_bfloat16 a = __float2bfloat16(lo), b = __float2bfloat16(hi);
     return (uint32_t)(*reinterpret_cast<const uint16_t*>(&a)) | ((uint32_t)(*reinterpret_cast<const uint16_t*>(&b)) << 16);
@@ -881,12 +778,6 @@ int wide_build_image(EpicModel* m, const float* W) {
     std::vector<__nv_bfloat16> img((size_t)ly.n_seq * kSlot / 2, __float2bfloat16(0.0f));
     std::vector<float> tab((size_t)ly.tab_floats, 0.0f);
     std::vector<uint2> frag((size_t)ly.frag_elems, make_uint2(0u, 0u));
-    auto put = [&](int slot, int o, int k, double v) { img[(size_t)slot * kSlot / 2 + tile_index(o, k, 2048)] = __float2bfloat16((float)v); };
-    auto put_bias = [&](int slot, int o, float b) {
-        const __nv_bfloat16 hi = __float2bfloat16(b);
-        img[(size_t)slot * kSlot / 2 + 32768 / 2 + tile_index(o, 0, 256)] = hi;
-        img[(size_t)slot * kSlot / 2 + 32768 / 2 + tile_index(o, 1, 256)] = __float2bfloat16(b - __bfloat162float(hi));
-    };
     // local_0 with the embeddings folded in: operand columns [x_hi (3) | x_lo (3) | onehot (S)]; its time columns act on the
     // jet's context vector (whose first T entries are the time embedding)
     for (int o = 0; o < H; ++o) {
@@ -894,13 +785,13 @@ int wide_build_image(EpicModel* m, const float* W) {
         for (int j = 0; j < Dc; ++j) {
             double acc = 0;
             for (int c = 0; c < C; ++c) acc += (double)w0[T + c] * W[Lo.emb_cont_w + (size_t)c * Dc + j];
-            put(0, o, j, acc);
-            put(0, o, Dc + j, acc);
+            slot_put_weight(img, 0, o, j, acc);
+            slot_put_weight(img, 0, o, Dc + j, acc);
         }
         for (int s = 0; s < S; ++s) {
             double acc = 0;
             for (int dd = 0; dd < D; ++dd) acc += (double)w0[T + C + dd] * W[Lo.emb_disc + (size_t)s * D + dd];
-            put(0, o, 2 * Dc + s, acc);
+            slot_put_weight(img, 0, o, 2 * Dc + s, acc);
         }
         double c0 = W[Lo.local0_b + o];
         for (int c = 0; c < C; ++c) c0 += (double)w0[T + c] * W[Lo.emb_cont_b + c];
@@ -936,15 +827,15 @@ int wide_build_image(EpicModel* m, const float* W) {
         for (int o = 0; o < H; ++o) {
             tl[ly.o_blg1 + o] = Wl[Lo.l_g1_b + o];
             tl[ly.o_bl1 + o] = Wl[Lo.l_l1_b + o];
-            for (int k = 0; k < H; ++k) put(1 + 2 * l, o, k, Wl[Lo.l_l1_w + (size_t)o * Kl + k]);
-            for (int k = 0; k < H; ++k) put(2 + 2 * l, o, k, Wl[Lo.l_l2_w + (size_t)o * H + k]);
-            put_bias(2 + 2 * l, o, Wl[Lo.l_l2_b + o]);
+            for (int k = 0; k < H; ++k) slot_put_weight(img, 1 + 2 * l, o, k, Wl[Lo.l_l1_w + (size_t)o * Kl + k]);
+            for (int k = 0; k < H; ++k) slot_put_weight(img, 2 + 2 * l, o, k, Wl[Lo.l_l2_w + (size_t)o * H + k]);
+            slot_put_bias(img, 2 + 2 * l, o, Wl[Lo.l_l2_b + o]);
         }
         for (int o = 0; o < G; ++o) tl[ly.o_blg2 + o] = Wl[Lo.l_g2_b + o];
     }
     for (int o = 0; o < Dc + S; ++o) {
-        for (int k = 0; k < H; ++k) put(1 + 2 * L, o, k, W[Lo.out_w + (size_t)o * H + k]);
-        put_bias(1 + 2 * L, o, W[Lo.out_b + o]);
+        for (int k = 0; k < H; ++k) slot_put_weight(img, 1 + 2 * L, o, k, W[Lo.out_w + (size_t)o * H + k]);
+        slot_put_bias(img, 1 + 2 * L, o, W[Lo.out_b + o]);
     }
     if (Sh) {   // discrete head; a padded slot's logits are head(0) (the reference masks before the head, mbm.py:105-111)
         std::vector<double> z1(Sh);

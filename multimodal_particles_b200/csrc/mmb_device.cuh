@@ -5,10 +5,19 @@
 // bit-identical to oracle/mmb_oracle.c, which performs the same IEEE operations in the same order.
 #pragma once
 
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 namespace mmb {
+
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// named barrier `id` over `threads` threads (a multiple of 32)
+__device__ __forceinline__ void named_bar(int id, int threads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
+__device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
+    __half2 h = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&h);
+}
 
 // exp() from IEEE fp32 operations only (Cody-Waite + polynomial): the same function on CPU and GPU.
 __device__ __forceinline__ float expf_exact(float x) {
@@ -65,6 +74,8 @@ __device__ __forceinline__ void fmul2(float& d0, float& d1, float a0, float a1, 
 }
 
 __device__ __forceinline__ float lrelu(float a) { return a > 0.0f ? a : __fmul_rn(a, 0.01f); }
+// the tensor-core engines' branch-free form
+__device__ __forceinline__ float lrelu_fast(float a) { return fmaxf(a, 0.01f * a); }
 
 __device__ __forceinline__ float selu(float a) {
     const float scale = 1.0507009873554804934193349852946f;
