@@ -648,8 +648,8 @@ int mmb_sample_source(float* x, uint8_t* k, uint8_t* mask, int B, int N, float s
                       uint64_t seed, uint64_t jet_offset, void* stream);
 
 /*
- * Forward half of a training / validation step (SURVEY.md §8f N2) — bridge sampling and the masked losses; the backward pass
- * stays out of scope.
+ * Training step of MultiModalBridgeMatching (SURVEY.md §8f N2) — bridge sampling and the masked losses below, and the losses
+ * with their gradients with respect to every EPiC weight (mmb_epic_loss_grad, after mmb_bridge_losses).
  *
  * mmb_sample_bridges = MultiModalBridgeMatching.sample_bridges (mp/models/generative/multimodal_bridge_matching.py:148-165) given the
  * per-jet times t [B]:  xt = (t x1 + (1-t) x0) + sigma z  (LinearUniformBridge.sample, bridges.py:23-27);
@@ -673,6 +673,26 @@ int mmb_absorbing_sample(const float* sp, const uint8_t* target_mask, const floa
 size_t mmb_bridge_losses_workspace_bytes(int B, int N);
 int mmb_bridge_losses(const float* v, const float* logits, const float* x0, const float* x1, const uint8_t* k1, const uint8_t* mask,
                       int B, int N, int S, float* out, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * The two losses of mmb_bridge_losses on the heads of the fp32 network (mmb_epic_forward, MMB_PREC_FP32) and their gradients
+ * with respect to every float of the packed weight blob (mbm.py:167-197, 232-240): the backward pass of a training step.
+ *   dims, W: the network's shape and its weights as a DEVICE blob in mmb_epic_layout order (weight norm folded by the caller, so
+ *   the blob an autograd graph produced on the device is used as it is: no model handle, no host round trip per step);
+ *   x [B,N,Dc], k [B,N] u8 (< S), mask [B,N] u8, temb [B,T+X] (temb_stride = T+X) or one shared row (temb_stride = 0) as in
+ *   mmb_epic_forward; x0, x1 [B,N,Dc], k1 [B,N] u8 (< S): the bridge end points of mmb_bridge_losses.
+ *   losses [3] = { mse, ce, live particles } as mmb_bridge_losses defines them;
+ *   jac [2][layout.total] = d mse / dW, d ce / dW; NULL = losses only (no backward pass);
+ *   d_context [2][B][X] = d mse, d ce with respect to each jet's embedded context (the part of temb after the time embedding);
+ *   nullable, written only with jac and X > 0.
+ * Jets without a live particle contribute nothing.  Deterministic: CTA count and summation order depend on dims and B only.
+ * 1 <= N <= MMB_EPIC_GRAD_MAX_N.  workspace: mmb_epic_loss_grad_workspace_bytes(dims, B, N) bytes (0 for bad arguments).
+ */
+#define MMB_EPIC_GRAD_MAX_N 1024
+size_t mmb_epic_loss_grad_workspace_bytes(const MmbEpicDims* dims, int B, int N);
+int mmb_epic_loss_grad(const MmbEpicDims* dims, const float* W, const float* x, const uint8_t* k, const uint8_t* mask, const float* temb,
+                       int temb_stride, const float* x0, const float* x1, const uint8_t* k1, int B, int N, float* losses, float* jac,
+                       float* d_context, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -122,6 +122,9 @@ SIGNATURES = {
     "mmb_absorbing_sample": (_i, [_vp, _vp, _vp, _u64, _u64, _i, _i, _vp, _vp]),
     "mmb_bridge_losses_workspace_bytes": (_sz, [_i, _i]),
     "mmb_bridge_losses": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _sz, _vp]),
+    "mmb_epic_loss_grad_workspace_bytes": (_sz, [ctypes.POINTER(EpicDims), _i, _i]),
+    "mmb_epic_loss_grad": (_i, [ctypes.POINTER(EpicDims), _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _sz,
+                                _vp]),
     "mmb_trans_packed_floats": (_sz, [ctypes.POINTER(TransDims)]),
     "mmb_trans_create": (_i, [ctypes.POINTER(TransDims), _vp, _sz, _i, ctypes.POINTER(_vp)]),
     "mmb_trans_destroy": (None, [_vp]),
@@ -514,3 +517,28 @@ def bridge_losses(v, logits, x0, x1, k1_u8, mask_u8):
         check(lib.mmb_bridge_losses(_ptr(v), _ptr(logits), _ptr(x0), _ptr(x1), _ptr(k1_u8), _ptr(mask_u8), B, N, S, _ptr(out), _ptr(ws),
                                     ws.numel(), _stream()))
     return out
+
+
+def epic_loss_grad(dims: EpicDims, W, x, k_u8, mask_u8, rows, x0, x1, k1_u8, jacobian=True):
+    """Bridge-matching losses of the fp32 network with weights ``W`` (device blob in ``mmb_epic_layout`` order) and, with
+    ``jacobian``, their gradients: -> (losses [3] = (mse, ce, live), jac [2, total] or None, d_context [2, B, X] or None)."""
+    _require_cuda(W, x, k_u8, mask_u8, rows, x0, x1, k1_u8)
+    B, N, _ = x.shape
+    lib = load()
+    total = lib.mmb_epic_packed_floats(ctypes.byref(dims))
+    if W.dtype != torch.float32 or W.numel() != total:
+        raise MmbError(f"weight blob must hold {total} float32 values, got {W.numel()} {W.dtype}")
+    width = dims.dim_time_emb + dims.dim_context
+    if rows.shape[-1] != width:
+        raise MmbError(f"context rows must hold {dims.dim_time_emb} time + {dims.dim_context} context entries, got {rows.shape[-1]}")
+    stride = 0 if rows.shape[0] == 1 and B != 1 else width
+    dev = x.device
+    losses = torch.empty(3, device=dev, dtype=torch.float32)
+    jac = torch.empty(2, total, device=dev, dtype=torch.float32) if jacobian else None
+    d_context = torch.empty(2, B, dims.dim_context, device=dev, dtype=torch.float32) if jacobian and dims.dim_context else None
+    need = lib.mmb_epic_loss_grad_workspace_bytes(ctypes.byref(dims), B, N)
+    ws = torch.empty(max(need, 16), device=dev, dtype=torch.uint8)
+    with torch.cuda.device(dev):
+        check(lib.mmb_epic_loss_grad(ctypes.byref(dims), _ptr(W), _ptr(x), _ptr(k_u8), _ptr(mask_u8), _ptr(rows), stride, _ptr(x0), _ptr(x1),
+                                     _ptr(k1_u8), B, N, _ptr(losses), _ptr(jac), _ptr(d_context), _ptr(ws), ws.numel(), _stream()))
+    return losses, jac, d_context

@@ -785,6 +785,36 @@ int mmb_bridge_losses(const float* v, const float* logits, const float* x0, cons
                                 static_cast<cudaStream_t>(stream));
 }
 
+static int check_grad_shape(const MmbEpicDims* d, int B, int N) {
+    if (!d) return fail(MMB_EINVAL, "mmb_epic_loss_grad: null dims");
+    if (d->dim_continuous < 1 || d->dim_continuous > 8 || d->vocab_size < 1 || d->vocab_size > 32)
+        return fail(MMB_EINVAL, "mmb_epic_loss_grad: need 1 <= Dc <= 8 and 1 <= S <= 32 (got Dc=%d S=%d)", d->dim_continuous, d->vocab_size);
+    if (d->dim_hidden_local < 1 || d->dim_hidden_glob < 1 || d->dim_time_emb < 1 || d->dim_cont_emb < 0 || d->dim_disc_emb < 0 ||
+        d->num_blocks < 0 || d->dim_context < 0 || d->disc_head_hidden < 0)
+        return fail(MMB_EINVAL, "mmb_epic_loss_grad: bad EPiC widths");
+    if (B < 1 || N < 1 || N > MMB_EPIC_GRAD_MAX_N)
+        return fail(MMB_EINVAL, "mmb_epic_loss_grad: need B >= 1 and 1 <= N <= %d (got B=%d N=%d)", MMB_EPIC_GRAD_MAX_N, B, N);
+    return MMB_OK;
+}
+
+size_t mmb_epic_loss_grad_workspace_bytes(const MmbEpicDims* dims, int B, int N) {
+    if (check_grad_shape(dims, B, N)) return 0;
+    return epic_loss_grad_workspace_bytes(*dims, B, N);
+}
+
+int mmb_epic_loss_grad(const MmbEpicDims* dims, const float* W, const float* x, const uint8_t* k, const uint8_t* mask, const float* temb,
+                       int temb_stride, const float* x0, const float* x1, const uint8_t* k1, int B, int N, float* losses, float* jac,
+                       float* d_context, void* workspace, size_t workspace_bytes, void* stream) {
+    if (int rc = check_grad_shape(dims, B, N)) return rc;
+    if (!W || !x || !k || !mask || !temb || !x0 || !x1 || !k1 || !losses || !workspace)
+        return fail(MMB_EINVAL, "mmb_epic_loss_grad: null argument");
+    if (temb_stride < 0) return fail(MMB_EINVAL, "mmb_epic_loss_grad: negative temb_stride");
+    const size_t need = epic_loss_grad_workspace_bytes(*dims, B, N);
+    if (workspace_bytes < need) return fail(MMB_ENOMEM, "mmb_epic_loss_grad: workspace has %zu B, needs %zu B", workspace_bytes, need);
+    return launch_epic_loss_grad(*dims, W, x, k, mask, temb, temb_stride, x0, x1, k1, B, N, losses, jac, d_context, workspace,
+                                 static_cast<cudaStream_t>(stream));
+}
+
 size_t mmb_wasserstein1d_workspace_bytes(int n, int m, int K) {
     if (n < 0 || m < 0 || K < 1 || K > MMB_W1_MAX_K) return 0;
     return wasserstein1d_workspace_bytes(n, m, K);

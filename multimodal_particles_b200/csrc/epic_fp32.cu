@@ -64,12 +64,6 @@ __device__ inline Smem carve(float* base, const Fp32Dims& f, int N) {
     return s;
 }
 
-// acc + sum_i w[i]*in[i], ascending i, one fmaf per term
-__device__ __forceinline__ float dot_from(float acc, const float* __restrict__ w, const float* in, int n) {
-    for (int i = 0; i < n; ++i) acc = __fmaf_rn(__ldg(w + i), in[i], acc);
-    return acc;
-}
-
 // four output rows at once (same chains, inputs read once)
 __device__ __forceinline__ void dot4_from(float (&acc)[4], const float* __restrict__ w, int ldw, const float* in, int n) {
     const float *w0 = w, *w1 = w + ldw, *w2 = w + 2 * ldw, *w3 = w + 3 * ldw;

@@ -73,6 +73,12 @@ __device__ __forceinline__ void fmul2(float& d0, float& d1, float a0, float a1, 
         : "=f"(d0), "=f"(d1) : "f"(a0), "f"(a1), "f"(b0), "f"(b1));
 }
 
+// acc + sum_i w[i]*in[i], ascending i, one fmaf per term (the fp32 forward's dot product; epic_fp32.cu, epic_grad.cu)
+__device__ __forceinline__ float dot_from(float acc, const float* __restrict__ w, const float* in, int n) {
+    for (int i = 0; i < n; ++i) acc = __fmaf_rn(__ldg(w + i), in[i], acc);
+    return acc;
+}
+
 __device__ __forceinline__ float lrelu(float a) { return a > 0.0f ? a : __fmul_rn(a, 0.01f); }
 // the tensor-core engines' branch-free form
 __device__ __forceinline__ float lrelu_fast(float a) { return fmaxf(a, 0.01f * a); }

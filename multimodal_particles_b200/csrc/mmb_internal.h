@@ -154,6 +154,12 @@ int launch_generate_fp32(const EpicModel* m, float* x, uint8_t* k, const uint8_t
                          int n_steps, float dt, const float* u_jump, uint64_t seed, uint64_t jet_offset,
                          int B, int N, cudaStream_t stream);
 
+// epic_grad.cu — bridge-matching losses and their weight gradients, fp32 (arguments checked by the caller)
+size_t epic_loss_grad_workspace_bytes(const MmbEpicDims& d, int B, int N);
+int launch_epic_loss_grad(const MmbEpicDims& d, const float* W, const float* x, const uint8_t* k, const uint8_t* mask, const float* temb,
+                          int temb_stride, const float* x0, const float* x1, const uint8_t* k1, int B, int N, float* losses, float* jac,
+                          float* d_context, void* workspace, cudaStream_t stream);
+
 // epic_tc.cu — tcgen05 path
 bool tc_supported(const MmbEpicDims* d, int N);
 int tc_read_trace(long long* out, int n);

@@ -4,7 +4,8 @@ The reference builds the network from ``torch.nn`` layers and evaluates ~725 eag
 (mp/models/architectures/epic.py:10-241, utils.py:6-198).  Here the modules only *hold* the
 parameters (so checkpoints load unchanged: ``…weight_g [out,1]``, ``…weight_v [out,in]``, ``…bias``,
 SURVEY.md §A.6); evaluation folds the weight norm once, packs everything into the blob described in
-include/mmbridge.h and calls the sm_100a kernels.  No autograd: this is the generation path.
+include/mmbridge.h and calls the sm_100a kernels.  No autograd on this generation path; ``packed_parameters`` gives the same
+blob under autograd for the losses' backward pass (MultiModalBridgeMatching.bridge_matching_losses).
 """
 from typing import Optional
 
@@ -86,6 +87,10 @@ class InputEmbeddings(nn.Module):
     def context(self, context_continuous, context_discrete, device) -> Optional[torch.Tensor]:
         """The part of the reference's per-jet ``context`` vector behind the time embedding (utils.py:155-170): [B, dim_context]
         fp32 on ``device`` — a Linear / table lookup on a few numbers per jet, once per call."""
+        return self.embedded_context(context_continuous, context_discrete, device)
+
+    def embedded_context(self, context_continuous, context_discrete, device) -> Optional[torch.Tensor]:
+        """``context`` under the caller's grad mode: with gradients on, the result carries the graph of the context embedding."""
         if not self.dim_context:
             return None
         parts = []
@@ -165,24 +170,30 @@ class EPiCWrapper(nn.Module):
     def epic_dims(self, disc_head_hidden: int = 0) -> _native.EpicDims:
         return _native.EpicDims(**self._dims, disc_head_hidden=disc_head_hidden)
 
-    def pack_weights(self, head: Optional[nn.Sequential] = None) -> torch.Tensor:
-        """Flat fp32 blob in the order of ``mmb_epic_layout`` (include/mmbridge.h)."""
+    def _blob_parts(self, head: Optional[nn.Sequential], fold) -> list:
+        """The tensors of the blob in ``mmb_epic_layout`` order (include/mmbridge.h); ``fold`` gives a layer's folded weight."""
         emb, net = self.embedding, self.epic
         parts = [emb.embedding_continuous.weight, emb.embedding_continuous.bias, emb.embedding_discrete.weight]
-
-        def wn(layer: WeightNormLinear):
-            parts.extend([layer.folded(), layer.bias])
-
         proj = net.epic_proj
-        for layer in (proj.local_0, proj.global_0, proj.global_1, proj.global_2):
-            wn(layer)
+        layers = [proj.local_0, proj.global_0, proj.global_1, proj.global_2]
         for block in net.epic_layers:
-            for layer in (block.fc_global1, block.fc_global2, block.fc_local1, block.fc_local2):
-                wn(layer)
-        wn(net.output_layer)
+            layers += [block.fc_global1, block.fc_global2, block.fc_local1, block.fc_local2]
+        for layer in layers + [net.output_layer]:
+            parts.extend([fold(layer), layer.bias])
         if head is not None:
             parts.extend([head[0].weight, head[0].bias, head[2].weight, head[2].bias])
+        return parts
+
+    def pack_weights(self, head: Optional[nn.Sequential] = None) -> torch.Tensor:
+        """Flat fp32 blob in the order of ``mmb_epic_layout`` (include/mmbridge.h)."""
+        parts = self._blob_parts(head, WeightNormLinear.folded)
         return torch.cat([p.detach().to("cpu", torch.float32).reshape(-1) for p in parts])
+
+    def packed_parameters(self, head: Optional[nn.Sequential] = None) -> torch.Tensor:
+        """The blob of ``pack_weights`` as a differentiable fp32 tensor on the parameters' device: the weight norm is folded by
+        ``torch._weight_norm`` under autograd, so a gradient of the blob reaches ``weight_g`` and ``weight_v``."""
+        fold = lambda layer: torch._weight_norm(layer.weight_v.float(), layer.weight_g.float(), 0)
+        return torch.cat([p.float().reshape(-1) for p in self._blob_parts(head, fold)])
 
     def native_model(self, device, head: Optional[nn.Sequential] = None) -> _native.EpicModel:
         """Device-resident packed model; rebuilt when any parameter changed (optimizer step,

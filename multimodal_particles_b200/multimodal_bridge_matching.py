@@ -5,8 +5,9 @@ Same constructor argument (``MultimodalBridgeMatchingConfig``), same ``forward(s
 ``simulate_dynamics(state, batch)`` and ``predict_step(batch, batch_idx)`` signatures, same output
 containers and tensor layouts, same state-dict keys.  The compute is libmmbridge.so: the loop in
 ``simulate_dynamics`` is ONE call of ``mmb_generate`` with the state resident on the GPU, instead
-of ~725 eager ops and 4 host syncs per step (SURVEY.md §3.1).  Training methods
-(``sample_bridges``, losses, ``training_step``) are outside this path (SURVEY.md §8f N2) and raise.
+of ~725 eager ops and 4 host syncs per step (SURVEY.md §3.1).  Training: ``sample_bridges`` and
+``bridge_matching_losses`` (differentiable, native backward pass) make a training step in a user's loop; ``training_step`` and
+``configure_optimizers`` are not wired and raise (SURVEY.md §8f N2).
 """
 from types import SimpleNamespace
 
@@ -84,6 +85,24 @@ def to_host_async(t: torch.Tensor) -> torch.Tensor:
     out = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
     out.copy_(t, non_blocking=True)
     return out
+
+
+class _BridgeMatchingLosses(torch.autograd.Function):
+    """(blob, embedded context) -> (loss_continuous, loss_discrete): one call of the native loss / gradient kernels; backward
+    combines the two Jacobian rows with the incoming scalar gradients."""
+
+    @staticmethod
+    def forward(ctx, W, context, dims, x, k, mask, rows, x0, x1, k1):
+        losses, jac, d_context = _native.epic_loss_grad(dims, W.detach().contiguous(), x, k, mask, rows, x0, x1, k1)
+        ctx.save_for_backward(jac, d_context if d_context is not None else jac.new_empty(0))
+        return losses[0].clone(), losses[1].clone()
+
+    @staticmethod
+    def backward(ctx, g_mse, g_ce):
+        jac, d_context = ctx.saved_tensors
+        d_w = g_mse * jac[0] + g_ce * jac[1]
+        d_ctx = g_mse * d_context[0] + g_ce * d_context[1] if ctx.needs_input_grad[1] else None
+        return (d_w, d_ctx) + (None,) * 8
 
 
 class MultiModalBridgeMatching(_ModuleBase):
@@ -238,6 +257,42 @@ class MultiModalBridgeMatching(_ModuleBase):
         """masked cross entropy of the token classifier (mbm.py:185-197); forward value only (no autograd)"""
         return self._losses(heads, state, batch)[1]
 
+    def bridge_matching_losses(self, state: HybridState, batch):
+        """``(loss_continuous, loss_discrete)`` of the network on the bridge state (mbm.py:167-197), differentiable with respect
+        to every parameter of the encoder: ``backward()`` fills ``.grad`` under the reference's state-dict keys (``…weight_g``,
+        ``…weight_v``, ``…bias``, the embeddings, ``encoder.fc_layer.*``, ``embedding_continuous_context.*``).  The network,
+        both losses and both gradients are one pass of the native fp32 kernels (``mmb_epic_loss_grad``); torch adds the weight-norm
+        chain rule and the context embedding.  A user's loop does what the reference's ``training_step`` does (mbm.py:232-240)::
+
+            state = model.sample_bridges(batch)
+            l0, l1 = model.bridge_matching_losses(state, batch)
+            loss, _ = model.loss_multihead([l0, l1])
+            loss.backward()
+            opt.step()
+
+        ``training_step`` and ``configure_optimizers`` still raise: wiring the Lightning step, the optimiser and its gradient
+        clipping is separate work.  Under ``torch.no_grad()`` the same values come without building the Jacobian."""
+        epic = self.encoder.epic
+        head = self.encoder.fc_layer if self.encoder.add_discrete_head else None
+        dev = self._compute_device(SimpleNamespace(continuous=state.continuous))
+        dims = epic.epic_dims(head[0].out_features if head is not None else 0)
+        f32 = lambda a: a.to(dev, torch.float32).contiguous()
+        u8 = lambda a: as_u8(a.to(dev))
+        x, k, mask = f32(state.continuous), u8(state.discrete), u8(state.absorbing)
+        x0, x1, k1 = f32(batch.source_continuous), f32(batch.target_continuous), u8(batch.target_discrete)
+        cc, cd = getattr(batch, "context_continuous", None), getattr(batch, "context_discrete", None)
+        if not torch.is_grad_enabled():
+            rows = epic.context_rows(state.time, cc, cd, dev)
+            W = epic.packed_parameters(head).to(dev).contiguous()
+            losses, _, _ = _native.epic_loss_grad(dims, W, x, k, mask, rows, x0, x1, k1, jacobian=False)
+            return losses[0], losses[1]
+        context = epic.embedding.embedded_context(cc, cd, dev)   # under autograd: the context Linear gets its gradient
+        rows = epic.time_embedding(state.time).to(dev)
+        if context is not None:
+            rows = torch.cat([rows, context.detach()], dim=-1).contiguous()
+        W = epic.packed_parameters(head).to(dev)
+        return _BridgeMatchingLosses.apply(W, context, dims, x, k, mask, rows, x0, x1, k1)
+
     @torch.no_grad()
     def validation_step(self, batch, batch_idx=0) -> torch.Tensor:
         """mbm.py:241-250: bridges -> heads -> the two losses -> learnable multi-head weighting (forward only)."""
@@ -247,8 +302,9 @@ class MultiModalBridgeMatching(_ModuleBase):
         loss, _ = self.loss_multihead([both[0], both[1]])
         return loss
 
-    # ---- outside the generation path ----------------------------------------------------------
+    # ---- not wired yet: a user's loop over bridge_matching_losses does what training_step does ----------------
     def _training_not_in_scope(self, *args, **kwargs):
-        raise NotImplementedError("the backward pass / optimiser are outside the B200 hot path (SURVEY.md §8f N2: forward only)")
+        raise NotImplementedError("the Lightning training step / optimiser are not wired: call bridge_matching_losses, "
+                                  "loss_multihead and backward() in your own loop (SURVEY.md §8f N2)")
 
     training_step = configure_optimizers = _training_not_in_scope
