@@ -36,8 +36,6 @@
 // one particle, four.
 #include <cuda_bf16.h>
 
-#include <stdlib.h>
-
 #include <vector>
 
 #include "mmb_device.cuh"
@@ -77,7 +75,6 @@ struct HeadParams {
     int n_jet;               // > 0: also write the mean of X over the N slots
     float* jet_out;          // [B][128] slot means (the per-jet head consumes them)
     const int32_t* pack;     // PackScratch of this call (tf_pack_kernel), or null: one jet per tile, one row per slot
-    long long* trace;        // debug: clock64() stamps of the first jet of CTA 0 (tools/stack_trace.py); null in production
 };
 
 // ---- packing pre-pass ---------------------------------------------------------------------------------------------------------
@@ -203,7 +200,6 @@ __device__ __forceinline__ float tanh_fast(float a) {
 // One CTA owns one TILE at a time: 128 rows = up to four jets in 32-row quarters (see the header).  Thread (r, cq): row r = TMEM
 // lane r (warp & 3 selects the lane quarter the warp may touch), channel slice cq = warp >> 2 -> kCW consecutive accumulator
 // columns = one tcgen05.ld per pass.
-template <bool TRACE>
 __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     constexpr int CW = kCW, NQ = kNQ, G = CW / 4, HQ = NQ / 2;   // HQ: threads per (row, attention head)
@@ -407,7 +403,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
     };
     // q / k / v biases are handled algebraically: q rides on an extra K-step; k is a per-query constant in the logits
     // (softmax-invariant) and is dropped; v is folded into the proj_out bias because softmax rows sum to one.
-#define STK_TRACE(id) do { if constexpr (TRACE) { if (p.trace && blockIdx.x == 0 && tile == 0 && tid == 32) p.trace[id] = clock64(); } } while (0)
     // ---- preparation of a tile, in four steps that are spread over the phases of the previous tile -------------------------------
     float* sStage = reinterpret_cast<float*>(sV + 16384);    // [128 rows][32 floats]: hidden | onehot | x | x of the nearest particle
     float* sTbias = reinterpret_cast<float*>(sV + 8192);     // [segment][nblk][128] raw time terms (the proj_in operand sits below)
@@ -539,7 +534,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
         rows_prefetch(tn);
     }
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        STK_TRACE(0);
         asm volatile("cp.async.wait_all;" ::: "memory");
         __syncthreads();
         { TileState* tmp = ts; ts = tn; tn = tmp; }
@@ -601,35 +595,27 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
         tc_fence_before();
         fence_proxy_async();
         __syncthreads();
-        STK_TRACE(1);
         mma_issue([&](uint32_t ws) { gemm_w(ws, dX, smem_u32(sA0), 512, 2, false, true, bar_mma); });
         mma_done(1);
-        STK_TRACE(2);
         const float* bias2 = s_bias2 + (seg < 0 ? 0 : seg) * nblk * kC;
 
         for (int blk = 0; blk < nblk; ++blk) {
             const float* T = sTab + blk * HeadTable::kPerBlock;
             // ---- ResnetBlock (gsdm.py:54-66)
             group_norm_to_A(dX, nullptr, T + 0 * kC, T + 1 * kC, true);
-            if (blk == 0) STK_TRACE(3);
             mma_issue([&](uint32_t ws) { gemm_w(ws, dACC, aA, 2048, 8, false, false, bar_mma); });           // conv1
             if (blk == 0 && has_next) desc_commit(tn);       // next tile's preparation rides under the GEMM round trips
             mma_done(1);
-            if (blk == 0) STK_TRACE(4);
             group_norm_to_A(dACC, bias2 + blk * kC, T + 3 * kC, T + 4 * kC, true);
-            if (blk == 0) STK_TRACE(5);
             mma_issue([&](uint32_t ws) { gemm_w(ws, dX, aA, 2048, 8, true, true, bar_mma); });               // X += conv2(.) + b2
             if (blk == 0 && has_next) masks_issue(tn);
             mma_done(1);
-            if (blk == 0) STK_TRACE(6);
             // ---- AttnBlock (gsdm.py:142-168)
             group_norm_to_A(dX, nullptr, T + 5 * kC, T + 6 * kC, false);
-            if (blk == 0) STK_TRACE(7);
             const uint32_t q_half = wseq & 1;                                // q sits in ring slot wseq & 1
             mma_issue([&](uint32_t ws) { gemm_qk(ws, dACC, aA); });                                 // [q | k] (+ bq), one N = 256 GEMM into ACC | S0
             if (blk == 0 && has_next) rowmap_build(tn);
             mma_done(2);
-            if (blk == 0) STK_TRACE(8);
             {   // both tiles in one epilogue phase
                 float v[CW];
                 tmem_ld32(dACC + q_half * 128 + lane_off + col0, v);
@@ -640,7 +626,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
                 fence_proxy_async();
                 __syncthreads();
             }
-            if (blk == 0) STK_TRACE(9);
             mma_issue([&](uint32_t ws) {                                     // S_h = Q_h K_h^T, K = 64
                 tc_fence_after();
                 const uint64_t qd = smem_desc(aQ, 128, 2048), kd = smem_desc(aK, 128, 2048);
@@ -653,7 +638,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
                 gemm_w(ws, dACC, aA, 2048, 8, false, false, bar_mma2);        // v: runs under the softmax, its own barrier
             });
             mma_done(0);
-            if (blk == 0) STK_TRACE(11);
             // softmax over the keys of the query's OWN jet (block-diagonal): thread (r, cq) serves head cq / HQ and the two 32-key
             // chunks (= row quarters) 2 (cq % HQ), 2 (cq % HQ) + 1; a chunk of another jet contributes nothing, a key's column
             // of P carries the key's row weight (the representative dead row stands for n_dead identical keys).  The HQ threads
@@ -686,10 +670,8 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
 #pragma unroll
                     for (int j = 0; j < CW; j += 2) mx = fmaxf(mx, fmaxf(v[j], v[j + 1]));
                 }
-                if (blk == 0) STK_TRACE(30);
                 s_rowx[cq][r] = mx;
                 named_bar(1 + NQ + h, 128 * HQ);   // the key slices of a head
-                if (blk == 0) STK_TRACE(31);
 #pragma unroll
                 for (int i = 0; i < HQ; ++i) mx = fmaxf(mx, s_rowx[h * HQ + i][r]);
                 const float sc = 0.125f * 1.4426950408889634f;  // dh^-1/2 * log2(e)
@@ -725,7 +707,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
                     store_row<CW>(h ? sQ : sK, r, key0 + c * CW, v);
                 }
                 s_sum[cq][r] = s0 + s1;
-                if (blk == 0) STK_TRACE(32);
                 // the v GEMM finished long ago: its tile joins this phase's fence and barrier
                 mbar_wait(bar_mma2, mma2_phase); mma2_phase ^= 1;
                 tc_fence_after();
@@ -737,13 +718,10 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
                     for (int j = 0; j < CW; ++j) v[j] = 0.0f;     // V rows of an empty quarter meet zero columns of P, but 0 x NaN is NaN
                 }
                 store_row<CW>(sV, r, col0, v);
-                if (blk == 0) STK_TRACE(33);
             }
             tc_fence_before();
             fence_proxy_async();
-            if (blk == 0) STK_TRACE(34);
             __syncthreads();
-            if (blk == 0) STK_TRACE(12);
             mma_issue([&](uint32_t) {                                        // O_h = P_h V_h, K = 128 keys, N = 64
                 tc_fence_after();
                 const uint64_t vd = smem_desc(aV, 2048, 128);
@@ -757,7 +735,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
                 umma_commit(bar_mma);
             });
             mma_done(0);
-            if (blk == 0) STK_TRACE(13);
             if (blk == nblk - 1 && has_next) rows_prefetch(tn);   // V is dead now
             {
                 float v[CW];  // columns [col0, +CW) of O belong to head cq / HQ: normalised by that head's row sum
@@ -773,12 +750,9 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
             tc_fence_before();
             fence_proxy_async();
             __syncthreads();
-            if (blk == 0) STK_TRACE(14);
             mma_issue([&](uint32_t ws) { gemm_w(ws, dX, aA, 2048, 8, true, true, bar_mma); });               // X += proj_out(.) + (b_o + W_o b_v)
             mma_done(1);
-            if (blk == 0) STK_TRACE(15);
         }
-        STK_TRACE(16);
         // ---- per-slot output: one 128-vector against the residual stream (absorbing: post_rate_proj(pre_rate_proj(X))
         //      folded, absorbing_flows.py:127-131; trans: near_atom_proj / vec_weighting_proj) and, for the per-jet heads,
         //      the mean of X over the N slots (transdimensional_model.py:309-311,403-405; the folded Linear follows in jet_head_kernel)
@@ -828,7 +802,6 @@ __global__ void __launch_bounds__(kThreads, 1) absorb_head_tc_kernel(const HeadP
         }
         tc_fence_before();
         __syncthreads();  // X, the operand tiles and the tile's tables are rewritten by the next tile
-        STK_TRACE(17);
     }
     tc_fence_before();
     __syncthreads();
@@ -953,21 +926,6 @@ int launch_jet_head(const TfStack* st, const float* means, int B, float* out, cu
     return cuda_ok(cudaGetLastError(), "jet head launch");
 }
 
-// MMB_STACK_TRACE=1: per-phase clock64() stamps of the first jet of CTA 0 (tools/stack_trace.py reads them)
-static long long* g_stack_trace = nullptr;
-static long long* stack_trace_buffer() {
-    static const bool on = [] { const char* e = getenv("MMB_STACK_TRACE"); return e && e[0] == '1'; }();
-    if (!on) return nullptr;
-    if (!g_stack_trace && cudaMalloc(&g_stack_trace, 64 * sizeof(long long)) == cudaSuccess) cudaMemset(g_stack_trace, 0, 64 * sizeof(long long));
-    return g_stack_trace;
-}
-int stack_read_trace(long long* out, int n) {
-    if (!g_stack_trace) return 0;
-    cudaDeviceSynchronize();
-    cudaMemcpy(out, g_stack_trace, sizeof(long long) * (n < 64 ? n : 64), cudaMemcpyDeviceToHost);
-    return n < 64 ? n : 64;
-}
-
 int launch_tf_stack(const TfStack* st, int sm_count, const TfStackIO& io, int B, int N, cudaStream_t stream) {
     if (N < 1 || N > 128) return fail(MMB_EUNSUPPORTED, "transformer stack handles 1..128 particle slots per jet (got %d)", N);
     if (B == 0) return MMB_OK;
@@ -976,9 +934,7 @@ int launch_tf_stack(const TfStack* st, int sm_count, const TfStackIO& io, int B,
     p.mode = io.mode; p.S = io.S; p.hidden = io.hidden; p.mask = io.mask; p.onehot = io.onehot; p.x = io.x; p.nearest = io.nearest;
     p.tbias = io.tbias; p.tbias_stride = io.tbias_stride; p.B = B; p.N = N; p.logit_out = io.dot_out;
     p.n_jet = io.jet_out ? st->n_jet : 0; p.jet_out = io.jet_out;
-    p.trace = stack_trace_buffer();
-    static const bool no_pack = [] { const char* e = getenv("MMB_STACK_NO_PACK"); return e && e[0] == '1'; }();   // debug knob
-    if (io.pack_scratch && !no_pack) {   // bin the jets by the quarters of a tile they need (dead slots once, several jets per tile)
+    if (io.pack_scratch) {   // bin the jets by the quarters of a tile they need (dead slots once, several jets per tile)
         if (io.pack_scratch_ints < PackScratch::ints(B)) return fail(MMB_ENOMEM, "transformer stack: packing scratch too small");
         if (int rc = cuda_ok(cudaMemsetAsync(io.pack_scratch, 0, 8 * sizeof(int32_t), stream), "pack counters")) return rc;
         tf_pack_kernel<<<(B + 7) / 8, 256, 0, stream>>>(io.mask, io.hidden, io.H, io.onehot, io.S, io.mode, B, N, io.pack_scratch);
@@ -987,7 +943,7 @@ int launch_tf_stack(const TfStack* st, int sm_count, const TfStackIO& io, int B,
         p.pack = io.pack_scratch;
     }
     const size_t bytes = kOffTab + (size_t)(HeadTable::floats(st->n_blocks) + kMaxSeg * st->n_blocks * kC) * 4;
-    auto kern = p.trace ? absorb_head_tc_kernel<true> : absorb_head_tc_kernel<false>;
+    auto kern = absorb_head_tc_kernel;
     cudaFuncAttributes attr;
     if (int rc = cuda_ok(cudaFuncGetAttributes(&attr, kern), "head attributes")) return rc;
     if (bytes + attr.sharedSizeBytes > 232448)

@@ -448,16 +448,15 @@ static int host_chunks(int B, int n_chunks) {
     return n_chunks > B ? (B > 0 ? B : 1) : n_chunks;
 }
 
-// direct mode (n_chunks <= 0): flag | mask int64 | mask u8 | token int64 (range check only) | state between time slices | scratch
+// direct mode (n_chunks <= 0): flag | mask int64 | mask u8 | token int64 (range check only) | context | scratch
 struct HostDirectLayout {
-    size_t m64, m8, k64, ctx, xs, ks, scratch, total;
+    size_t m64, m8, k64, ctx, scratch, total;
     HostDirectLayout(const EpicModel* m, int B, int N, int n_steps) {
         const size_t P = (size_t)B * N;
         size_t at = 256;
         auto take = [&](size_t bytes) { const size_t o = at; at += (bytes + 255) & ~(size_t)255; return o; };
         m64 = take(P * 8); m8 = take(P); k64 = take(P * 8);
         ctx = take((size_t)B * m->dims.dim_context * sizeof(float));
-        xs = take(P * m->dims.dim_continuous * sizeof(float)); ks = take(P);
         scratch = take(mma_generate_scratch_floats(&m->dims, n_steps, B) * sizeof(float));
         total = at;
     }
@@ -545,7 +544,7 @@ int mmb_generate_host(const MmbEpicModel* handle, const float* x_in, const int64
                 rc = cuda_ok(cudaGetLastError(), "narrow launch");
             }
             const MmaHostIO io{static_cast<const float*>(dx_in), static_cast<const long long*>(dk_in), static_cast<float*>(dx_out),
-                               static_cast<long long*>(dk_out), d_bad, reinterpret_cast<float*>(ws + lay.xs), ws + lay.ks};
+                               static_cast<long long*>(dk_out), d_bad};
             float* dctx = X ? reinterpret_cast<float*>(ws + lay.ctx) : nullptr;
             if (!rc && X) rc = cuda_ok(cudaMemcpyAsync(dctx, context_in, (size_t)B * X * sizeof(float), cudaMemcpyHostToDevice, sa), "H2D context");
             if (!rc) rc = launch_generate_mma(m, nullptr, nullptr, dm8, dctx, table, reinterpret_cast<float*>(ws + lay.scratch), n, st->dt, nullptr, seed,
@@ -918,11 +917,5 @@ int mmb_kpd_mmd(const float* real, int64_t ldr, int n, const float* gen, int64_t
     return launch_kpd_mmd(real, ldr, gen, ldg, d, scale, idx_real, idx_gen, batches, B, degree, out, workspace,
                           static_cast<cudaStream_t>(stream));
 }
-
-// debug only (not part of include/mmbridge.h): phase timestamps of the tcgen05 generation kernel, see tools/tc_trace.py
-int mmb_debug_read_trace(long long* out, int n) { return tc_read_trace(out, n); }
-int mmb_debug_read_stack_trace(long long* out, int n) { return stack_read_trace(out, n); }
-int mmb_debug_read_wide_trace(long long* out, int n) { return wide_read_trace(out, n); }
-long long mmb_debug_read_mma_trace(unsigned long long* out, long long max_words) { return mma_read_trace(out, max_words); }
 
 }  // extern "C"

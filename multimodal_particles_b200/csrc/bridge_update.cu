@@ -4,15 +4,18 @@
 // token, all from registers.  Algorithmic traffic per particle-step (Dc=3, S=8): x r+w 24 B, v 12 B,
 // logits 32 B, one jump uniform 4 B, token r+w 2 B, mask r 1 B = 75 B (84 B with the absorbing
 // logit, its uniform and the mask write).  No data is reused, so there is nothing to stage in
-// shared memory: each thread owns FOUR consecutive particles, which makes every global access a
-// 16-byte vector (x/v: 3 x float4, logits: S x float4, u: float4) or a 4-byte word (tokens, masks),
-// fully coalesced, with all loads issued before the first use.
+// shared memory: each thread owns TWO consecutive particles, which makes every global access an
+// 8- or 16-byte vector (x/v: 3 x float2, logits: S/2 x float4, u: float2) or a 2-byte word (tokens,
+// masks), fully coalesced, with all loads issued before the first use.
 #include "mmb_device.cuh"
 #include "mmb_internal.h"
 
-#include <stdlib.h>
-
 namespace mmb {
+
+// particles per thread and CTAs per SM of the vector kernel: the variant with the highest bandwidth
+// at 32 768 jets and more in profiles/r01_update_variants.md
+constexpr int kPPT = 2;
+constexpr int kUpdateMinBlocks = 5;
 
 // NF consecutive floats -> registers with the widest aligned vector (16 B when NF % 4 == 0, else 8 B)
 template <int NF, bool STREAM>
@@ -91,12 +94,13 @@ __device__ __forceinline__ void draw_uniforms(const UpdateDraws& d, int stream_i
 }
 
 // Dc = 3.  Each thread owns PPT consecutive particles; group g covers particles [g*PPT, (g+1)*PPT).
-template <int S, int PPT, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+template <int S>
+__global__ void __launch_bounds__(256, kUpdateMinBlocks)
 bridge_update_vec_kernel(float* __restrict__ x, uint8_t* __restrict__ k, uint8_t* __restrict__ mask,
                          const float* __restrict__ v, const float* __restrict__ logits,
                          const float* __restrict__ absorb, const float* __restrict__ uj,
                          const float* __restrict__ ua, StepScalars sc, size_t groups, int flags, UpdateDraws draws) {
+    constexpr int PPT = kPPT;
     const size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= groups) return;
     const bool do_euler = !(flags & MMB_FLAG_NO_EULER), do_jump = !(flags & MMB_FLAG_NO_JUMP),
@@ -172,16 +176,6 @@ bridge_update_generic_kernel(float* __restrict__ x, uint8_t* __restrict__ k, uin
     }
 }
 
-// tuning knob MMB_UPDATE_VARIANT = 10*particles_per_thread + min CTAs/SM (profiles/r01_update_variants.md)
-static int update_variant() {
-    static int v = [] {
-        const char* e = getenv("MMB_UPDATE_VARIANT");
-        const int q = e ? atoi(e) : 25;
-        return (q == 42 || q == 24 || q == 26 || q == 18) ? q : 25;
-    }();
-    return v;
-}
-
 static bool aligned16(const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 int launch_bridge_update(float* x, uint8_t* k, uint8_t* mask, const float* v, const float* logits,
@@ -195,25 +189,13 @@ int launch_bridge_update(float* x, uint8_t* k, uint8_t* mask, const float* v, co
                         aligned16(logits) && aligned16(absorb) && aligned16(uj) && aligned16(ua) &&
                         (reinterpret_cast<uintptr_t>(k) & 3u) == 0 && (reinterpret_cast<uintptr_t>(mask) & 3u) == 0;
     if (vec_ok && P >= 4) {
-        const int var = update_variant();
-        const int ppt = var / 10;
-        const size_t groups = P / ppt;
+        const size_t groups = P / kPPT;
         const unsigned grid = (unsigned)((groups + 255) / 256);
-        const bool s4 = (S == 4 && !(flags & MMB_FLAG_NO_JUMP));
-#define MMB_LAUNCH(PP, MB)                                                                                              \
-    do {                                                                                                                \
-        if (s4) bridge_update_vec_kernel<4, PP, MB><<<grid, 256, 0, stream>>>(x, k, mask, v, logits, absorb, uj, ua, sc, groups, flags, draws); \
-        else bridge_update_vec_kernel<8, PP, MB><<<grid, 256, 0, stream>>>(x, k, mask, v, logits, absorb, uj, ua, sc, groups, flags, draws);   \
-    } while (0)
-        switch (var) {
-            case 42: MMB_LAUNCH(4, 2); break;
-            case 24: MMB_LAUNCH(2, 4); break;
-            case 26: MMB_LAUNCH(2, 6); break;
-            case 18: MMB_LAUNCH(1, 8); break;
-            default: MMB_LAUNCH(2, 5); break;
-        }
-#undef MMB_LAUNCH
-        done = groups * ppt;
+        if (S == 4 && !(flags & MMB_FLAG_NO_JUMP))
+            bridge_update_vec_kernel<4><<<grid, 256, 0, stream>>>(x, k, mask, v, logits, absorb, uj, ua, sc, groups, flags, draws);
+        else
+            bridge_update_vec_kernel<8><<<grid, 256, 0, stream>>>(x, k, mask, v, logits, absorb, uj, ua, sc, groups, flags, draws);
+        done = groups * kPPT;
     }
     if (done < P) {
         const size_t count = P - done;

@@ -31,8 +31,6 @@
 // mp/models/generative/multimodal_bridge_matching.py:90-113,199-216, bridges.py:38-45,106-132,179-201).
 #include <cuda_fp16.h>
 
-#include <stdlib.h>
-
 #include <type_traits>
 #include <vector>
 
@@ -42,25 +40,16 @@
 namespace mmb {
 namespace {
 
-#ifndef MMB_MMA_WARPS
-#define MMB_MMA_WARPS 8      // measured at C2 / dense: 8 warps x 2 CTAs per SM 4.07 / 1.98 M jets/s, 16 x 1: 3.93 / 1.73
-#endif
-#ifndef MMB_MMA_MINB
-#define MMB_MMA_MINB 2
-#endif
 constexpr int kH = 16;          // hidden width this engine is built for
-constexpr int kW = MMB_MMA_WARPS;   // warps per CTA; the grid is persistent: MMB_MMA_MINB CTAs per SM
+// warps per CTA; the grid is persistent: kMinBlocks CTAs per SM.  Measured at C2 / dense: 8 warps x 2 CTAs per SM 4.07 / 1.98 M
+// jets/s, 16 x 1: 3.93 / 1.73
+constexpr int kW = 8;
+constexpr int kMinBlocks = 2;
 constexpr int kRowsPerWarp = 64;
 constexpr int kMaxCls = 4;      // a jet spans at most this many warps (N <= 256)
 constexpr int kKeys = 4 * kMaxCls;   // work lists: key = 4 (cls - 1) + (m-tiles of the jet's last warp - 1)
 constexpr int kMaxL = 4;
-constexpr int kMaxSegs = 4;     // time slices of a single-warp jet (MMB_MMA_SEGS; see the scheduling loop)
-constexpr int kCounterInts = kKeys * (1 + kMaxSegs);   // counts [kKeys] | cursors [rounds][kKeys]
-constexpr unsigned long long kTraceRecords = 1ull << 18;
-// Measured cost of one jet of each key in ns of the whole chip (tools/mma_cost_by_size.py, default widths, 99 steps); only the
-// RATIOS matter: they decide how many SMs start on which key.  Keys of three- and four-warp jets (N > 128) are extrapolated.
-__constant__ float kKeyCost[kKeys] = {138.f, 150.f, 198.f, 228.f, 412.f, 428.f, 473.f, 518.f,
-                                      650.f, 665.f, 710.f, 755.f, 890.f, 905.f, 950.f, 995.f};
+constexpr int kCounterInts = 2 * kKeys;   // counts [kKeys] | cursors [kKeys]
 constexpr int kStageBytes = 3072;   // per warp: A tile [64 rows][48 B]  /  logits [64][8] f32 + velocity [64][4] f32
 constexpr int kSkipBytes = 4096;    // per warp: fp32 skip connection, [8][32 lanes] float4
 constexpr int kPoolFloats = 32;     // per warp: two (ping-pong) slots of 16 partial column sums
@@ -142,17 +131,9 @@ struct MmaParams {
     const float4* tvec;      // [n_steps][2 + 2L][8] bias quads of the per-step time vectors (prologue kernel)
     const float4* cvec;      // [B][1 + 2L][8] quads of the per-jet context terms of global_0 / fc_global1 / fc_local1, or null
     const int32_t* counts;   // [kKeys]: jets per key (empty jets are finished by the prologue and appear in no list)
-    int32_t* cursors;        // [rounds][kKeys]: next unclaimed jet of each key (teams of `cls` warps claim dynamically)
+    int32_t* cursors;        // [kKeys]: next unclaimed jet of each key (teams of `cls` warps claim dynamically)
     const int32_t* lists;    // [kKeys][B]: jets of each key
     const int32_t* jet_cnt;  // [B] live particles
-    // time slicing of single-warp jets (see the scheduling loop): state between two segments of a jet, and the number of
-    // segments of each jet that are complete.  Device mode: xs = x, ks = k (in place); HOSTIO: device scratch
-    float* xs;               // [B,N,Dc]
-    uint8_t* ks;             // [B,N]
-    int32_t* prog;           // [B], zeroed by the prologue
-    int home_keys;           // scheduling: every SM starts on its own key (1) / the whole chip walks the keys widest-first (0)
-    int max_segs;            // time slices per jet in small calls (1: none)
-    unsigned long long* trace;   // debug (MMB_MMA_TRACE=1, tools/mma_timeline.py): [0] = records written, then 4 words per job
 };
 
 // A column vector in the fragment layout (v[j][b] = element 8 j + 2 t + b, the same in every row group) as an A operand whose
@@ -166,7 +147,7 @@ __device__ __forceinline__ void vec_frag(uint32_t (&a)[4], float v00, float v01,
 }
 
 template <int DC, int S, int SH, int GT, bool HOSTIO, bool CTX>
-__global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kernel(const MmaParams p) {
+__global__ void __launch_bounds__(kW * 32, kMinBlocks) epic_mma_generate_kernel(const MmaParams p) {
     using LY = Lay<GT>;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x;
@@ -198,9 +179,7 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
 
     // One jet (or this warp's 64-row slice of it) through all solver steps.  `team` = index of the group of `cls` consecutive
     // warps that carries the jet: named barrier 1 + team, exchange buffers of the team's first warp onwards.
-    // Steps [step0, step1) of the jet; `first` / `last`: the segment starts from the caller's source state / ends with the result.
-    auto process = [&](const int jet, const int cls, const int slice, const int team, const int step0, const int step1, const bool first,
-                       const bool last) {
+    auto process = [&](const int jet, const int cls, const int slice, const int team) {
     // the two particles this lane OWNS (state, update): rows lane and lane + 32 of the warp's slice
     const int n0 = kRowsPerWarp * slice + lane, n1 = n0 + 32;
     const size_t jbase = (size_t)jet * N;
@@ -221,12 +200,11 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
         // harmless in HBM, a 3x cost over PCIe (direct mode).  With N % 4 == 0 the rows of a slice form whole 16-byte chunks:
         // the warp moves them as float4 through the staging tile.
         const bool vec_io = (N & 3) == 0;
-        // a later segment reads what another warp (any SM) stored: L2 loads (ld.global.cg), never the non-coherent path
-        const float* xin = first ? (HOSTIO ? p.x_in : p.x) : p.xs;
+        const float* xin = HOSTIO ? p.x_in : p.x;
         if (vec_io) {
             const int rows = min(16 * NMT, N - kRowsPerWarp * slice);
             const float4* src = reinterpret_cast<const float4*>(xin + (jbase + (size_t)kRowsPerWarp * slice) * DC);
-            for (int i = lane; i < rows * DC / 4; i += 32) reinterpret_cast<float4*>(stage)[i] = first ? __ldg(src + i) : __ldcg(src + i);
+            for (int i = lane; i < rows * DC / 4; i += 32) reinterpret_cast<float4*>(stage)[i] = __ldg(src + i);
             __syncwarp();
             const float* st = reinterpret_cast<const float*>(stage);
 #pragma unroll
@@ -238,14 +216,11 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
         } else {
 #pragma unroll
             for (int c = 0; c < DC; ++c) {
-                xs0[c] = live0 ? (first ? xin[(jbase + n0) * DC + c] : __ldcg(xin + (jbase + n0) * DC + c)) : 0.0f;
-                xs1[c] = (TWO && live1) ? (first ? xin[(jbase + n1) * DC + c] : __ldcg(xin + (jbase + n1) * DC + c)) : 0.0f;
+                xs0[c] = live0 ? xin[(jbase + n0) * DC + c] : 0.0f;
+                xs1[c] = (TWO && live1) ? xin[(jbase + n1) * DC + c] : 0.0f;
             }
         }
-        if (!first) {
-            if (live0) kk0 = __ldcg(p.ks + jbase + n0);
-            if (TWO && live1) kk1 = __ldcg(p.ks + jbase + n1);
-        } else if constexpr (HOSTIO) {
+        if constexpr (HOSTIO) {
             const long long q0 = live0 ? p.k_in[jbase + n0] : 0, q1 = (TWO && live1) ? p.k_in[jbase + n1] : 0;
             if (q0 < 0 || q0 >= S || q1 < 0 || q1 >= S) atomicOr(p.bad_tokens, 1);   // the reference asserts (bridges.py:111-115)
             kk0 = (int)q0 & (S - 1);
@@ -310,7 +285,7 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
             }
         };
 
-        for (int step = step0; step < step1; ++step) {
+        for (int step = 0; step < p.n_steps; ++step) {
             const float4* tvq = p.tvec + (size_t)step * (2 + 2 * L) * 8 + t;   // quad (v, j): tvq[8 v + 4 j]
             // time vector v (>= 1) plus the jet's context term of the same Linear (the reference's context = [t_emb | ctx])
             auto ctx_quad = [&](int v, int j) {
@@ -549,34 +524,6 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
             }
             __syncwarp();   // the staging tile becomes the A tile of the next step
         }
-        if (!last) {
-            // ---- hand-over to the jet's next segment: the rows this warp carries, then "segment done"
-            if (vec_io) {
-                float* st = reinterpret_cast<float*>(stage);
-#pragma unroll
-                for (int c = 0; c < DC; ++c) {
-                    st[lane * DC + c] = live0 ? xs0[c] : 0.0f;
-                    st[(lane + 32) * DC + c] = (TWO && live1) ? xs1[c] : 0.0f;
-                }
-                __syncwarp();
-                const int rows = min(16 * NMT, N - kRowsPerWarp * slice);
-                float4* dst = reinterpret_cast<float4*>(p.xs + (jbase + (size_t)kRowsPerWarp * slice) * DC);
-                for (int i = lane; i < rows * DC / 4; i += 32) dst[i] = reinterpret_cast<const float4*>(stage)[i];
-                __syncwarp();
-            } else {
-#pragma unroll
-                for (int c = 0; c < DC; ++c) {
-                    if (live0) p.xs[(jbase + n0) * DC + c] = xs0[c];
-                    if (TWO && live1) p.xs[(jbase + n1) * DC + c] = xs1[c];
-                }
-            }
-            if (live0) p.ks[jbase + n0] = (uint8_t)kk0;
-            if (TWO && live1) p.ks[jbase + n1] = (uint8_t)kk1;
-            __threadfence();
-            __syncwarp();
-            if (lane == 0) atomicAdd(p.prog + jet, 1);   // one per warp of the jet
-            return;
-        }
         // ---- final state: live particles as computed, dead ones 0 (x * mask, k * mask)
         if (vec_io) {
             float* st = reinterpret_cast<float*>(stage);
@@ -627,57 +574,20 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
     };
 
     // ---- persistent scheduling.  Jets wait in lists keyed by (warps they span, m-tiles of their last warp); a team of `cls`
-    // consecutive warps claims the next jet of a key with one atomic (single-warp jets, the bulk, warp by warp).  Default: the
-    // whole chip walks the keys widest-first, so that (a) the longest jobs start first (LPT) and (b) at any moment the warps of
-    // the chip work on neighbours in the list, i.e. run the same copy of the step loop.
-    // Two variations are built in and were measured with the kernel's own job records (tools/mma_timeline.py,
-    // profiles/r02_mma_timeline.md) — neither is on by default:
-    //  * MMB_MMA_HOME=1, home keys: every SM starts on its own key (the keys share the SMs in proportion to jets x measured cost,
-    //    kKeyCost) and walks the keys cyclically from there, so an SM stays inside ONE copy of the step loop.  Jobs are not
-    //    faster for it (the copies do not fight over the instruction cache as feared) and the static split ends less evenly.
-    //  * MMB_MMA_SEGS=3, time slicing: jets are claimed in rounds of a third of the steps each — the state between two steps is
-    //    just (x, k), handed over through L2 (p.xs / p.ks / p.prog) — to shorten the last jobs of a small call (4096 jets: the
-    //    chip is 91.5 % busy between the first and the last job, the tail is the rest).  A segment has to wait for the one
-    //    before it; warps that wait instead of taking other work cost more than the shorter tail gives (4096 jets: 1.35 ms
-    //    chip-wide order, 0.99 ms with home keys, against 0.94 ms unsliced).  Results are identical in every mode: the
-    //    arithmetic of a step knows nothing about keys or segments (segments start at multiples of four steps because a Philox
-    //    block serves four steps).
-    __shared__ int s_home;
-    if (tid == 0) {
-        unsigned smid, nsm;
-        asm("mov.u32 %0, %%smid;" : "=r"(smid));
-        asm("mov.u32 %0, %%nsmid;" : "=r"(nsm));
-        float total = 0.0f;
-        for (int i = 0; i < kKeys; ++i) total += kKeyCost[i] * (float)__ldg(p.counts + i);
-        const float target = total * ((float)(smid % nsm) + 0.5f) / (float)nsm;
-        int home = 0;
-        float acc = 0.0f;
-        for (int i = kKeys - 1; i >= 0; --i) {   // widest keys on the lowest SMs
-            acc += kKeyCost[i] * (float)__ldg(p.counts + i);
-            if (acc >= target) { home = i; break; }
-        }
-        s_home = p.home_keys ? home : kKeys - 1;
-    }
-    __syncthreads();
-    const int home = s_home;
-    // rounds: with time slicing, round r hands out segment r of every single-warp jet (multi-warp jets run whole, in round 0).
-    // A warp reaches round r + 1 only when no job of round r is left to claim, and jobs are claimed in the same order in every
-    // round, so the predecessor of a job was claimed a whole round earlier: the wait below practically never spins.
-    int n_single = 0;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) n_single += __ldg(p.counts + i);
-    const int n_rounds = (p.n_steps >= 8 * p.max_segs && n_single < 6 * (int)gridDim.x * kW) ? p.max_segs : 1;
-    for (int round = 0; round < n_rounds; ++round)
+    // consecutive warps claims the next jet of a key with one atomic (single-warp jets, the bulk, warp by warp).  The whole chip
+    // walks the keys widest-first, so that (a) the longest jobs start first (LPT) and (b) at any moment the warps of the chip
+    // work on neighbours in the list, i.e. run the same copy of the step loop.
+    // Two alternatives were measured with per-job records (profiles/r02_mma_timeline.md) and removed: every SM starting on its
+    // own key made no job faster and ended less evenly, and time slicing small calls cost more in warps waiting for the previous
+    // slice of a jet than the shorter tail gave back (4096 jets: 1.35 ms against 0.94 ms unsliced).
     for (int visit = 0; visit < kKeys; ++visit) {
-        const int key = (home - visit + kKeys) % kKeys;   // towards the narrower keys, then around
+        const int key = kKeys - 1 - visit;
         const int n_key = __ldg(p.counts + key);
         if (n_key == 0) continue;
         const int cls = key / 4 + 1;
-        const int n_seg = cls == 1 ? n_rounds : 1, seg = round;
-        if (seg >= n_seg) continue;
         const int team = warp / cls, slice = warp - team * cls;
         if ((team + 1) * cls > kW) continue;           // warps left over when cls does not divide kW sit this key out
-        int32_t* cursor = p.cursors + kKeys * round + key;
+        int32_t* cursor = p.cursors + key;
         for (;;) {
             int idx = 0;
             if (slice == 0) {
@@ -692,30 +602,7 @@ __global__ void __launch_bounds__(kW * 32, MMB_MMA_MINB) epic_mma_generate_kerne
             }
             if (idx >= n_key) break;
             const int jet = __ldg(p.lists + (size_t)key * p.B + idx);
-            const int step0 = seg == 0 ? 0 : (p.n_steps * seg / n_seg) & ~3;
-            const int step1 = seg == n_seg - 1 ? p.n_steps : (p.n_steps * (seg + 1) / n_seg) & ~3;
-            if (seg > 0) {   // every warp of the jet's previous segment has stored its rows
-                if (lane == 0)
-                    while (*reinterpret_cast<volatile int32_t*>(p.prog + jet) < seg * cls) __nanosleep(200);
-                __syncwarp();
-                __threadfence();
-            }
-            unsigned long long t0 = 0;
-            if (p.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-            process(jet, cls, slice, team, step0, step1, seg == 0, seg == n_seg - 1);
-            if (p.trace && lane == 0) {
-                unsigned long long t1;
-                unsigned smid;
-                asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-                asm("mov.u32 %0, %%smid;" : "=r"(smid));
-                const unsigned long long rec = atomicAdd(p.trace, 1ull);
-                if (rec < kTraceRecords) {
-                    unsigned long long* r = p.trace + 4 + 4 * rec;
-                    r[0] = t0; r[1] = t1;
-                    r[2] = ((unsigned long long)smid << 32) | ((unsigned long long)blockIdx.x << 8) | (unsigned)warp;
-                    r[3] = ((unsigned long long)jet << 16) | ((unsigned long long)key << 8) | (unsigned)seg;
-                }
-            }
+            process(jet, cls, slice, team);
         }
     }
 }
@@ -732,7 +619,7 @@ __global__ void __launch_bounds__(kPrologueThreads) mma_prologue_kernel(const fl
                                                                         const float* __restrict__ temb, int n_steps, float4* __restrict__ tvec,
                                                                         const float* __restrict__ context, float4* __restrict__ cvec, int ctx_blocks,
                                                                         const uint8_t* __restrict__ mask, int B, int N, int32_t* __restrict__ counts,
-                                                                        int32_t* __restrict__ lists, int32_t* __restrict__ jet_cnt, int32_t* __restrict__ prog,
+                                                                        int32_t* __restrict__ lists, int32_t* __restrict__ jet_cnt,
                                                                         float* __restrict__ x, uint8_t* __restrict__ k, long long* __restrict__ k64) {
     const int T = d.dim_time_emb, C = d.dim_cont_emb, D = d.dim_disc_emb, H = d.dim_hidden_local, G = d.dim_hidden_glob, L = d.num_blocks,
               X = d.dim_context, TX = T + X;
@@ -813,7 +700,6 @@ __global__ void __launch_bounds__(kPrologueThreads) mma_prologue_kernel(const fl
                 if (row[i]) { ++cnt; last = i + 1; }
         }
         jet_cnt[jet] = cnt;
-        prog[jet] = 0;
         cls = (last + kRowsPerWarp - 1) / kRowsPerWarp;
         if (cls > 0) {
             key = 4 * (cls - 1) + (last - kRowsPerWarp * (cls - 1) + 15) / 16 - 1;   // m-tiles of the jet's last warp
@@ -996,29 +882,7 @@ int mma_build_images(EpicModel* m, const float* packed_host) {
 static size_t tvec_floats(const MmbEpicDims* d, int n_steps) { return (size_t)n_steps * (2 + 2 * d->num_blocks) * 32; }
 static size_t cvec_floats(const MmbEpicDims* d, int B) { return d->dim_context > 0 ? (size_t)(B > 0 ? B : 0) * (1 + 2 * d->num_blocks) * 32 : 0; }
 size_t mma_generate_scratch_floats(const MmbEpicDims* d, int n_steps, int B) {
-    return tvec_floats(d, n_steps) + cvec_floats(d, B) + kCounterInts + (size_t)(B > 0 ? B : 0) * (2 + kKeys) + 16;
-}
-
-// MMB_MMA_TRACE=1: one record per (warp, job) — start / end (globaltimer ns), SM, CTA, warp, jet, key, segment — read through
-// mmb_debug_read_mma_trace (tools/mma_timeline.py)
-static unsigned long long* g_mma_trace = nullptr;
-static unsigned long long* mma_trace_buffer() {
-    static const bool on = [] { const char* e = getenv("MMB_MMA_TRACE"); return e && e[0] == '1'; }();
-    if (!on) return nullptr;
-    const size_t bytes = (4 + 4 * kTraceRecords) * sizeof(unsigned long long);
-    if (!g_mma_trace && cudaMalloc(&g_mma_trace, bytes) != cudaSuccess) { g_mma_trace = nullptr; return nullptr; }
-    cudaMemset(g_mma_trace, 0, 4 * sizeof(unsigned long long));
-    return g_mma_trace;
-}
-long long mma_read_trace(unsigned long long* out, long long max_words) {
-    if (!g_mma_trace) return 0;
-    cudaDeviceSynchronize();
-    unsigned long long n = 0;
-    cudaMemcpy(&n, g_mma_trace, sizeof(n), cudaMemcpyDeviceToHost);
-    if (n > kTraceRecords) n = kTraceRecords;
-    if ((long long)(4 * n) > max_words) n = (unsigned long long)(max_words / 4);
-    cudaMemcpy(out, g_mma_trace + 4, 4 * n * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-    return (long long)n;
+    return tvec_floats(d, n_steps) + cvec_floats(d, B) + kCounterInts + (size_t)(B > 0 ? B : 0) * (1 + kKeys) + 16;
 }
 
 int launch_generate_mma(const EpicModel* m, float* x, uint8_t* k, const uint8_t* mask, const float* context, const float* dev_table, float* scratch,
@@ -1044,27 +908,19 @@ int launch_generate_mma(const EpicModel* m, float* x, uint8_t* k, const uint8_t*
     int32_t* cursors = counts + kKeys;
     int32_t* jet_cnt = counts + kCounterInts;
     int32_t* lists = jet_cnt + B;
-    int32_t* prog = lists + (size_t)kKeys * B;
     if (int rc = cuda_ok(cudaMemsetAsync(counts, 0, kCounterInts * sizeof(int32_t), stream), "mma counters")) return rc;
     const int bin_blocks = (B + kPrologueThreads - 1) / kPrologueThreads;
     const int ctx_blocks = context ? (int)(((size_t)B * (1 + 2 * m->dims.num_blocks) * 8 + kPrologueThreads - 1) / kPrologueThreads) : 0;
     mma_prologue_kernel<<<n_steps + ctx_blocks + bin_blocks, kPrologueThreads, 0, stream>>>(m->w, m->layout, m->dims, dev_table + (size_t)n_steps * 4, n_steps,
                                                                                 reinterpret_cast<float4*>(scratch), context, cvec, ctx_blocks, mask, B, N, counts, lists,
-                                                                                jet_cnt, prog, p.x, k, host ? host->k_out : nullptr);
+                                                                                jet_cnt, p.x, k, host ? host->k_out : nullptr);
     if (int rc = cuda_ok(cudaGetLastError(), "mma prologue launch")) return rc;
     p.tvec = reinterpret_cast<const float4*>(scratch); p.cvec = cvec; p.counts = counts; p.cursors = cursors; p.lists = lists; p.jet_cnt = jet_cnt;
-    p.prog = prog;
-    static const int home_keys = [] { const char* e = getenv("MMB_MMA_HOME"); return e ? atoi(e) : 0; }();
-    static const int max_segs = [] { const char* e = getenv("MMB_MMA_SEGS"); const int v = e ? atoi(e) : 1; return v < 1 ? 1 : (v > kMaxSegs ? kMaxSegs : v); }();
-    p.home_keys = home_keys; p.max_segs = max_segs;
-    p.trace = mma_trace_buffer();
-    p.xs = host ? host->x_state : x;
-    p.ks = host ? host->k_state : k;
-    // Persistent grid: MMB_MMA_MINB CTAs per SM at most.  Any grid finishes any amount of work (warps claim jets until the
+    // Persistent grid: kMinBlocks CTAs per SM at most.  Any grid finishes any amount of work (warps claim jets until the
     // lists are empty), so the size only matters for speed: a small call takes about 1.25 warps per jet (the JetClass-like
     // mean is 1.14), which lets the kernels of neighbouring pipeline slices (mmb_generate_host) share the GPU side by side.
     const int want = (int)(((size_t)B * 5 + 4 * kW - 1) / (4 * kW));
-    const int grid = want < m->sm_count * MMB_MMA_MINB ? (want > 0 ? want : 1) : m->sm_count * MMB_MMA_MINB;
+    const int grid = want < m->sm_count * kMinBlocks ? (want > 0 ? want : 1) : m->sm_count * kMinBlocks;
     return dispatch(m->dims, p, grid, stream);
 }
 

@@ -37,8 +37,6 @@
 // mp/models/generative/multimodal_bridge_matching.py:90-113,199-216, bridges.py:38-45,106-132,179-201).
 #include <cuda_bf16.h>
 
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include <vector>
@@ -283,11 +281,10 @@ struct TcParams {
     uint64_t seed, jet_offset;
     int B, N;
     float *v_out, *logits_out, *hidden_out;  // forward outputs
-    // generate, optional: jets binned by tc_bin kernels — big_list [counts[0]] jets with a live particle at index >= 64 (one per
-    // tile), small_list [counts[1]] the others (two per tile, 64 rows each); null = jet s on tile s
+    // generate: jets binned by tc_bin kernels — big_list [counts[0]] jets with a live particle at index >= 64 (one per tile),
+    // small_list [counts[1]] the others (two per tile, 64 rows each); forward: null, jet s on tile s
     const int32_t *big_list, *small_list, *counts;
     const float* tvec;     // generate: [n_steps][2+2L][16] per-step time vectors from tc_time_vectors_kernel; forward: null
-    long long* trace;      // debug: clock64() stamps of jet 0, step 3 (tools/tc_trace.py); null in production
 };
 
 // per-group shared memory: A tile (4 KB), mask tile (4 KB), dynamic bias operand of local_0 (512 B)
@@ -301,7 +298,7 @@ struct JetVec {
     uint32_t live16[4];   // per row quarter: bit 0 / 1 = rows 0-15 / 16-31 of the quarter hold a live particle
 };
 
-template <int DC, int S, int SH, bool GENERATE, bool TRACE = false>
+template <int DC, int S, int SH, bool GENERATE>
 __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const TcLayout& lay = p.lay;
@@ -319,12 +316,10 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
     int n_big = 0, n_small = 0;
     long n_slots = p.B;
     if constexpr (GENERATE) {
-        if (p.counts) {
-            n_big = __ldg(p.counts);
-            n_small = __ldg(p.counts + 1);
-            n_slots = (long)n_big + (n_small + 1) / 2;
-            if ((long)blockIdx.x * kJPC >= n_slots) return;
-        }
+        n_big = __ldg(p.counts);
+        n_small = __ldg(p.counts + 1);
+        n_slots = (long)n_big + (n_small + 1) / 2;
+        if ((long)blockIdx.x * kJPC >= n_slots) return;
     }
 
     // ---- one-time: weights -> smem, ones, barriers, TMEM
@@ -356,7 +351,7 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
     bool paired = false;
     int jet = (int)slot;    // the jet of THIS thread's rows (-1: none); 32-bit on purpose: it stays live through the whole loop
     if constexpr (GENERATE) {
-        if (p.counts && have) {
+        if (have) {
             const long n_pairs = (n_small + 1) / 2;   // paired tiles take longer per step: they go first, the single-jet tiles fill the tail
             if (slot >= n_pairs) {
                 jet = __ldg(p.big_list + (slot - n_pairs));
@@ -472,7 +467,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
         const int o16 = lane & 15, hf = lane >> 4;
 
         const int n_steps = GENERATE ? p.n_steps : 1;
-#define MMB_TRACE(id) do { if constexpr (TRACE) { if (p.trace && jet == 0 && step == 3 && n == 0) p.trace[id] = clock64(); } } while (0)
         // The step loop exists twice: once for row warps (and special warps that also carry live particles), once for a special
         // warp without live particles (SOLO) — there no per-particle state is alive, so the whole register budget is free to
         // pipeline the shared-memory loads of the per-jet global MLP, the longest serial stretch of a step.  All mutable
@@ -489,24 +483,17 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
         for (int c = 0; c < DC; ++c) xs[c] = xs_in[c];
         int kk = kk_in;
         uint32_t phase = 0;
-        int trace_step = 0;
         // MMA completion: every warp that is going to read the accumulator polls the mbarrier itself (try_wait suspends in
         // hardware, and 60 % of the issue slots are idle anyway); warps without row work, the special warp included, do not
         // wait at all — the barrier after the epilogue is what orders the next MMA behind this one's readers.
-        auto wait_mma = [&](int trace_id = -1) {
-            if constexpr (ROWS) {
-                mbar_wait(mbar, phase);
-                if constexpr (TRACE) { if (trace_id >= 0 && p.trace && jet == 0 && trace_step == 3 && lane == 0) p.trace[trace_id] = clock64(); }
-            }
+        auto wait_mma = [&]() {
+            if constexpr (ROWS) mbar_wait(mbar, phase);
             phase ^= 1;
         };
-#define MMB_TRACE_X(id) do { if constexpr (TRACE) { if (p.trace && jet == 0 && step == 3 && special_here && lane == 0) p.trace[id] = clock64(); } } while (0)
         uint32_t uq0 = 0, uq1 = 0, uq2 = 0, uq3 = 0;   // this particle's jump uniforms of the current group of four steps
         for (int step = 0; step < n_steps; ++step) {
-            trace_step = step;
-            MMB_TRACE(0);
             // ---- (a) time vectors (warp 0) and the first A row [x_hi, x_lo, onehot(k)] * m
-            if (GENERATE && p.tvec) {
+            if constexpr (GENERATE) {
                 // the time is shared by all jets at generation: the vectors were computed once per step by the prologue kernel
                 if (special_here) {
                     const float* tv = p.tvec + (size_t)step * (2 + 2 * L) * 16;
@@ -523,7 +510,7 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                     }
                 }
             } else if (special_here) {
-                const float* te = GENERATE ? p.temb + (size_t)step * T : p.temb + (size_t)jet * p.temb_stride;
+                const float* te = p.temb + (size_t)jet * p.temb_stride;
                 const int t0 = hf * (T / 2), t1 = t0 + T / 2;
                 float a0 = hf ? 0.0f : s_wf[lay.c0 + o16], a1 = hf ? 0.0f : s_wf[lay.g0b + o16];
                 for (int t = t0; t < t1; ++t) {
@@ -567,19 +554,15 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
             }
             fence_proxy_async();
             group_bar(1 + grp);
-            MMB_TRACE(1);
             // ---- (b) local_0
-            MMB_TRACE_X(20);
             if (issuer_here && elect_one()) {
                 tc_fence_after();
                 gemm(lay.bop_local0());
                 umma(d_main, amask_desc, bb0_desc, idesc_k, 1);  // + bias on live rows; dead rows stay exactly 0
                 umma_commit(mbar);
             }
-            MMB_TRACE_X(21);
-            wait_mma(22);
+            wait_mma();
             tc_fence_after();
-            MMB_TRACE(2);
             float acc[16], xl[16];
             if constexpr (ROWS) {
                 tmem_ld16(t_main, acc);
@@ -590,7 +573,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
             tc_fence_before();
             fence_proxy_async();
             group_bar(1 + grp);
-            MMB_TRACE(3);
 
             for (int l = 0; l < L; ++l) {
                 const float* Wl = s_wf + lay.layer0 + l * lay.layer_stride;
@@ -650,7 +632,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                     tc_fence_before();
                 }
                 group_bar(1 + grp);
-                MMB_TRACE(4 + 4 * l);
                 // ---- (f) fc_local1 epilogue -> A operand of fc_local2
                 tc_fence_after();
                 if constexpr (ROWS) {
@@ -663,18 +644,14 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                 tc_fence_before();
                 fence_proxy_async();
                 group_bar(1 + grp);
-                MMB_TRACE(5 + 4 * l);
                 // ---- (g) fc_local2
-                if (l == 0) MMB_TRACE_X(23);
                 if (issuer_here && elect_one()) {
                     tc_fence_after();
                     gemm(lay.bop_l2(l));
                     umma(d_main, amask_desc, bop_desc(lay.bop_bias_l2(l)), idesc_k, 1);
                     umma_commit(mbar);
                 }
-                if (l == 0) MMB_TRACE_X(24);
-                wait_mma(l == 0 ? 25 : -1);
-                MMB_TRACE(6 + 4 * l);
+                wait_mma();
                 tc_fence_after();
                 if constexpr (ROWS) {
                     tmem_ld16(t_main, acc);
@@ -689,7 +666,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                 tc_fence_before();
                 fence_proxy_async();
                 group_bar(1 + grp);
-                MMB_TRACE(7 + 4 * l);
             }
             // ---- (i) output layer (epic.py:158-162)
             if (issuer_here && elect_one()) {
@@ -703,7 +679,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
             }
             wait_mma();
             tc_fence_after();
-            MMB_TRACE(12);
             float h[16];
             if constexpr (ROWS) tmem_ld16(t_main, h);   // h[0..DC) = velocity (0 on dead rows); h[DC..) = head pre-activation or raw logits
             float lg[S];
@@ -725,7 +700,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                 }
                 wait_mma();
                 tc_fence_after();
-                MMB_TRACE(14);
                 if constexpr (!ROWS) {
                 } else if constexpr (S <= 8) {
                     float l8[8];
@@ -742,7 +716,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                 for (int s = 0; s < S; ++s) lg[s] = h[DC + s];
             }
             tc_fence_before();  // orders this step's last tcgen05.ld before the next step's first MMA (via the group barrier)
-            MMB_TRACE(15);
 
             if constexpr (GENERATE && ROWS) {
                 // ---- (k) hybrid update in registers (bridges.py:38-45,179-201)
@@ -774,7 +747,6 @@ __global__ void __launch_bounds__(kJPC * 128, 2) epic_tc_kernel(const TcParams p
                                              : u01(ph == 0 ? uq0 : ph == 1 ? uq1 : ph == 2 ? uq2 : uq3);
                     kk = telegraph_jump_fast<S>(lg, kk, u, sc) * m;
                 }
-                MMB_TRACE(16);
             }
             if constexpr (!GENERATE) {
                 if (valid) {
@@ -823,10 +795,10 @@ size_t tc_smem_bytes(const TcLayout& lay) {
     return (size_t)lay.n_bops * 512 + 4096 + 8192 + (size_t)lay.n_floats * 4 + kJPC * grp + 1024;
 }
 
-template <int DC, int S, int SH, bool GEN, bool TRACE = false>
+template <int DC, int S, int SH, bool GEN>
 int launch(const TcParams& p, cudaStream_t stream) {
     const size_t bytes = tc_smem_bytes(p.lay);
-    auto kern = epic_tc_kernel<DC, S, SH, GEN, TRACE>;
+    auto kern = epic_tc_kernel<DC, S, SH, GEN>;
     if (int rc = cuda_ok(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes), "tc smem attribute")) return rc;
     const int grid = (p.B + kJPC - 1) / kJPC;
     kern<<<grid, kJPC * 128, bytes, stream>>>(p);
@@ -836,9 +808,6 @@ int launch(const TcParams& p, cudaStream_t stream) {
 template <bool GEN>
 int dispatch(const MmbEpicDims& d, const TcParams& p, cudaStream_t stream) {
     const int sh = d.disc_head_hidden;
-    if constexpr (GEN) {   // the phase trace (tools/tc_trace.py) is a separate instantiation: production kernels carry none of it
-        if (p.trace && d.dim_continuous == 3 && d.vocab_size == 8 && sh == 8) return launch<3, 8, 8, true, true>(p, stream);
-    }
     if (d.dim_continuous == 3 && d.vocab_size == 8 && sh == 8) return launch<3, 8, 8, GEN>(p, stream);
     if (d.dim_continuous == 3 && d.vocab_size == 8 && sh == 0) return launch<3, 8, 0, GEN>(p, stream);
     if (d.dim_continuous == 3 && d.vocab_size == 4 && sh == 4) return launch<3, 4, 4, GEN>(p, stream);
@@ -952,7 +921,8 @@ __global__ void tc_time_vectors_kernel(const uint8_t* __restrict__ image, TcLayo
 // ---- binning of the jets of a generation call: "small" = no live particle at index >= 64 (two of them share a tile) ---------
 // Order-preserving (deterministic) compaction in three small kernels: per-block counts, a one-warp scan, the fill.
 constexpr int kBinThreads = 256;
-__global__ void __launch_bounds__(kBinThreads) tc_bin_count_kernel(const uint8_t* __restrict__ mask, int B, int N, int vec_ok, int first_dead, uint8_t* __restrict__ flag,
+constexpr int kPairRows = kRows / 2;   // rows of a small jet in a paired tile
+__global__ void __launch_bounds__(kBinThreads) tc_bin_count_kernel(const uint8_t* __restrict__ mask, int B, int N, int vec_ok, uint8_t* __restrict__ flag,
                                                                    int32_t* __restrict__ block_small) {
     const int jet = blockIdx.x * kBinThreads + threadIdx.x;
     int small = 0;
@@ -960,12 +930,12 @@ __global__ void __launch_bounds__(kBinThreads) tc_bin_count_kernel(const uint8_t
         small = 1;
         const uint8_t* row = mask + (size_t)jet * N;
         if (vec_ok) {
-            for (int n = first_dead; n < N; n += 16) {
+            for (int n = kPairRows; n < N; n += 16) {
                 const uint4 q = __ldg(reinterpret_cast<const uint4*>(row + n));
                 if (q.x | q.y | q.z | q.w) small = 0;
             }
         } else {
-            for (int n = first_dead; n < N; ++n) if (row[n]) small = 0;
+            for (int n = kPairRows; n < N; ++n) if (row[n]) small = 0;
         }
         flag[jet] = (uint8_t)small;
     }
@@ -1019,26 +989,9 @@ struct BinLayout {   // in 4-byte units after the time vectors
         total = at;
     }
 };
-constexpr int kBinMinJets = 1;   // every call is binned: where a jet runs (paired tile or not, which rotation) depends on the jet alone,
-                                 // so its result does not depend on the size or composition of the call
 
 size_t tc_generate_scratch_floats(const MmbEpicDims* d, int n_steps, int B) {
     return (((size_t)n_steps * (2 + 2 * d->num_blocks) * 16 + 3) & ~(size_t)3) + BinLayout(B > 0 ? B : 0).total;
-}
-
-// MMB_TC_TRACE=1: per-phase clock64() stamps of jet 0 (tools/tc_trace.py reads them through mmb_debug_read_trace)
-static long long* g_trace_dev = nullptr;
-static long long* tc_trace_buffer() {
-    static const bool on = [] { const char* e = getenv("MMB_TC_TRACE"); return e && e[0] == '1'; }();
-    if (!on) return nullptr;
-    if (!g_trace_dev && cudaMalloc(&g_trace_dev, 64 * sizeof(long long)) == cudaSuccess) cudaMemset(g_trace_dev, 0, 64 * sizeof(long long));
-    return g_trace_dev;
-}
-int tc_read_trace(long long* out, int n) {
-    if (!g_trace_dev) return 0;
-    cudaDeviceSynchronize();
-    cudaMemcpy(out, g_trace_dev, sizeof(long long) * (n < 64 ? n : 64), cudaMemcpyDeviceToHost);
-    return n < 64 ? n : 64;
 }
 
 bool tc_supported(const MmbEpicDims* d, int N) {
@@ -1187,26 +1140,22 @@ int launch_generate_tc(const EpicModel* m, float* x, uint8_t* k, const uint8_t* 
     p.step_tab = dev_table; p.temb = dev_table + (size_t)n_steps * 4; p.temb_stride = 0;
     p.n_steps = n_steps; p.dt = dt; p.u_jump = u_jump; p.seed = seed; p.jet_offset = jet_offset;
     p.B = B; p.N = N;
-    p.trace = tc_trace_buffer();
-    if (scratch) {
-        tc_time_vectors_kernel<<<n_steps, 16 * (2 + 2 * kMaxL), 0, stream>>>(p.image, p.lay, p.temb, scratch);
-        if (int rc = cuda_ok(cudaGetLastError(), "tc_time_vectors launch")) return rc;
-        p.tvec = scratch;
-        static const int pair_max = [] { const char* e = getenv("MMB_PAIR_MAX"); return e ? atoi(e) : 64; }();
-        if (B >= kBinMinJets && pair_max > 0) {   // bin the jets: big ones get a tile each, small ones share tiles in pairs
-            const BinLayout bl(B);
-            int32_t* base = reinterpret_cast<int32_t*>(scratch + (((size_t)n_steps * (2 + 2 * m->dims.num_blocks) * 16 + 3) & ~(size_t)3));
-            uint8_t* flag = reinterpret_cast<uint8_t*>(base + bl.flag);
-            tc_bin_count_kernel<<<bl.nblocks, kBinThreads, 0, stream>>>(mask, B, N, ((N & 15) == 0 && (reinterpret_cast<uintptr_t>(mask) & 15) == 0) ? 1 : 0, pair_max,
-                                                                        flag, base + bl.block_small);
-            tc_bin_scan_kernel<<<1, 32, 0, stream>>>(base + bl.block_small, bl.nblocks, B, base + bl.block_off, base + bl.counts);
-            tc_bin_fill_kernel<<<bl.nblocks, kBinThreads, 0, stream>>>(flag, base + bl.block_off, B, base + bl.small_list, base + bl.big_list);
-            if (int rc = cuda_ok(cudaGetLastError(), "tc_bin launch")) return rc;
-            p.counts = base + bl.counts;
-            p.small_list = base + bl.small_list;
-            p.big_list = base + bl.big_list;
-        }
-    }
+    tc_time_vectors_kernel<<<n_steps, 16 * (2 + 2 * kMaxL), 0, stream>>>(p.image, p.lay, p.temb, scratch);
+    if (int rc = cuda_ok(cudaGetLastError(), "tc_time_vectors launch")) return rc;
+    p.tvec = scratch;
+    // bin the jets, every call: big ones get a tile each, small ones share tiles in pairs.  Where a jet runs (paired tile or
+    // not, which rotation) depends on the jet alone, so its result does not depend on the size or composition of the call
+    const BinLayout bl(B);
+    int32_t* base = reinterpret_cast<int32_t*>(scratch + (((size_t)n_steps * (2 + 2 * m->dims.num_blocks) * 16 + 3) & ~(size_t)3));
+    uint8_t* flag = reinterpret_cast<uint8_t*>(base + bl.flag);
+    tc_bin_count_kernel<<<bl.nblocks, kBinThreads, 0, stream>>>(mask, B, N, ((N & 15) == 0 && (reinterpret_cast<uintptr_t>(mask) & 15) == 0) ? 1 : 0,
+                                                                flag, base + bl.block_small);
+    tc_bin_scan_kernel<<<1, 32, 0, stream>>>(base + bl.block_small, bl.nblocks, B, base + bl.block_off, base + bl.counts);
+    tc_bin_fill_kernel<<<bl.nblocks, kBinThreads, 0, stream>>>(flag, base + bl.block_off, B, base + bl.small_list, base + bl.big_list);
+    if (int rc = cuda_ok(cudaGetLastError(), "tc_bin launch")) return rc;
+    p.counts = base + bl.counts;
+    p.small_list = base + bl.small_list;
+    p.big_list = base + bl.big_list;
     return dispatch<true>(m->dims, p, stream);
 }
 

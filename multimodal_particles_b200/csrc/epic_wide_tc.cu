@@ -30,8 +30,6 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
-#include <stdlib.h>
-
 #include <vector>
 
 #include "mmb_device.cuh"
@@ -213,7 +211,6 @@ struct WideParams {
     float* v_out;                    // [B,N,3]
     float* logits_out;               // [B,N,S]
     float* hidden_out;               // [B,N,128] or null
-    long long* trace;                // debug: clock64() stamps of the first pair of CTA 0 (tools/wide_trace.py); null in production
 };
 
 // dynamic shared memory
@@ -413,10 +410,8 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
         sw[lo_off + g * stride + word] = lo;
     };
 
-#define WIDE_TRACE(id) do { if (p.trace && blockIdx.x == 0 && pi == 0 && tid == 0) p.trace[id] = clock64(); } while (0)
     for (int pi = 0; pi < my_pairs; ++pi) {
         const int pair = (int)blockIdx.x + pi * (int)gridDim.x;
-        WIDE_TRACE(0);
         // ---- the pair's tiles: records, row map (row i of a segment = its i-th live particle), context vectors ---------------
         if (tid < 2 * kRec) {
             const int t = tid / kRec, i = tid % kRec, tile = 2 * pair + t;
@@ -488,7 +483,6 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
             *reinterpret_cast<uint4*>(q + 128) = make_uint4(w[4], w[5], w[6], w[7]);
         }
         publish();
-        WIDE_TRACE(1);
         // ---- local_0 (one K-step) for both tiles; meanwhile the per-jet time vector of its bias -> bl1 buffer
         gemm(0, wseq, dX[0], 1, idesc128, false, false);
         if (has_b) gemm(1, wseq, dX[1], 1, idesc128, false, false);
@@ -561,14 +555,11 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
                 sv[Vec::part + t * 16 * 32 + warp * 32 + lane] = 0.0f;
             }
         };
-        WIDE_TRACE(2);
         epilogue(0, 0, false);
-        WIDE_TRACE(3);
         publish();
         gemm(0, wseq + 1, dACC[0], 8, idesc128, false, false);                       // fc_local1 of layer 0, tile A
         if (has_b) epilogue(1, 0, false);
         publish();
-        WIDE_TRACE(4);
         matrix_done();                                                               // local_0 served both tiles
         if (has_b) gemm(1, wseq, dACC[1], 8, idesc128, false, false);
         // ---- EPiC_Projection globals (epic.py:187-190): g0 = lrelu(G0 [mean, sum, ctx]), g1 = lrelu(G1 g0), xg = lrelu(G2 g1)
@@ -601,12 +592,10 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
             }
             compute_sync();
         }
-        WIDE_TRACE(5);
         // ---- EPiC layers (epic.py:217-241, 152-155)
         for (int l = 0; l < L; ++l) {
             const float* tl = p.tab + ly.layer0 + (size_t)l * ly.layer_stride;
             const uint2* fl = p.frag + ly.f_layer0 + (size_t)l * ly.f_layer_stride;
-            if (l == 1) WIDE_TRACE(6);
             {   // per-jet path: fc_global1 -> fc_global2 (+ residual) -> the per-jet part of fc_local1
                 FragRegs<kMaxKS> f;
                 FragRegs<8> f2;
@@ -620,17 +609,13 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
                 const float2 bias1 = __ldg(reinterpret_cast<const float2*>(tl + ly.o_blg1 + ob));
                 const float2 bias2 = warp < Gq / 8 ? __ldg(reinterpret_cast<const float2*>(tl + ly.o_blg2 + ob)) : make_float2(0.f, 0.f);
                 const float2 bias3 = __ldg(reinterpret_cast<const float2*>(tl + ly.o_bl1 + ob));
-                if (l == 1) WIDE_TRACE(16);
                 if (l > 0) {
                     pool_to_input();
                     compute_sync();
                 }
-                if (l == 1) WIDE_TRACE(17);
                 stage(f, ly.KS_1(), 16, sw + Vec::in1_hi, sw + Vec::in1_lo, kIn1Stride, c, 16);
-                if (l == 1) WIDE_TRACE(18);
                 if (g < kMaxJ) put_pair(Vec::gva_hi, Vec::gva_lo, kGvStride, 4 * warp + t4, lrelu(c[0] + bias1.x), lrelu(c[1] + bias1.y));
                 compute_sync();
-                if (l == 1) WIDE_TRACE(19);
                 stage(f2, 8, Gq / 8, sw + Vec::gva_hi, sw + Vec::gva_lo, kGvStride, c);
                 if (g < kMaxJ && warp < Gq / 8) {
                     const int o = 8 * warp + 2 * t4;
@@ -642,9 +627,7 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
                     put_pair(Vec::in1_hi, Vec::in1_lo, kIn1Stride, 128 + TXq / 2 + 4 * warp + t4, xg[0], xg[1]);
                 }
                 compute_sync();
-                if (l == 1) WIDE_TRACE(20);
                 stage(f3, ly.KS_2(), 16, sw + Vec::cx_hi, sw + Vec::cx_lo, kCxStride, c);
-                if (l == 1) WIDE_TRACE(21);
                 if (g < kMaxJ) {
                     const int o = 8 * warp + 2 * t4;
                     sv[Vec::bl1 + g * 128 + o] = c[0] + bias3.x;
@@ -653,29 +636,21 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
                 compute_sync();
             }
             const bool last = l == L - 1;
-            if (l == 1) WIDE_TRACE(7);
             epilogue(0, 1, false);
-            if (l == 1) WIDE_TRACE(8);
             publish();
             gemm(0, wseq + 1, dX[0], 8, idesc128, true, true);                      // fc_local2 accumulates onto X
-            if (l == 1) WIDE_TRACE(9);
             if (has_b) epilogue(1, 1, false);
-            if (l == 1) WIDE_TRACE(10);
             publish();
             matrix_done();                                                           // fc_local1 served both tiles
             if (has_b) gemm(1, wseq, dX[1], 8, idesc128, true, true);
-            if (l == 1) WIDE_TRACE(11);
             epilogue(0, 2, last);
-            if (l == 1) WIDE_TRACE(12);
             publish();
             gemm(0, wseq + 1, dACC[0], 8, last ? idesc16 : idesc128, false, last);  // next fc_local1, or the output layer
             if (has_b) epilogue(1, 2, last);
             publish();
             matrix_done();                                                           // fc_local2 served both tiles
             if (has_b) gemm(1, wseq, dACC[1], 8, last ? idesc16 : idesc128, false, last);
-            if (l == 1) WIDE_TRACE(13);
         }
-        WIDE_TRACE(14);
         // ---- output layer + discrete head (epic.py:158-162, mbm.py:105-113) for the live particles: the rows of tile A are served by
         // the threads of column slice 0, those of tile B by slice 1, side by side
         wait_tile(0);
@@ -714,15 +689,12 @@ __global__ void __launch_bounds__(kThreads, 1) epic_wide_kernel(const WideParams
         }
         tc_fence_before();
         compute_sync();
-        WIDE_TRACE(15);
         matrix_done();   // output layer served both tiles
     }
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem, 512);
 }
-
-__device__ long long g_wide_trace[32];
 
 inline uint32_t host_pack_bf16(float lo, float hi) {
     const __nv_bfloat16 a = __float2bfloat16(lo), b = __float2bfloat16(hi);
@@ -868,12 +840,6 @@ int wide_build_image(EpicModel* m, const float* W) {
     return rc;
 }
 
-int wide_read_trace(long long* out, int n) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_wide_trace, sizeof(long long) * (n < 32 ? n : 32));
-    return n < 32 ? n : 32;
-}
-
 int launch_epic_forward_wide(const EpicModel* m, const float* x, const uint8_t* k, const uint8_t* mask, const float* temb, int temb_stride,
                              int B, int N, float* v_out, float* logits_out, float* hidden_out, cudaStream_t stream) {
     const WideImage* w = static_cast<const WideImage*>(m->wide);
@@ -889,8 +855,6 @@ int launch_epic_forward_wide(const EpicModel* m, const float* x, const uint8_t* 
     p.image = static_cast<const uint8_t*>(w->image); p.tab = w->tab; p.frag = w->frag; p.lay = w->lay; p.pack = pack;
     p.x = x; p.k = k; p.mask = mask; p.temb = temb; p.temb_stride = temb_stride; p.B = B; p.N = N;
     p.v_out = v_out; p.logits_out = logits_out; p.hidden_out = hidden_out;
-    static const bool trace_on = [] { const char* e = getenv("MMB_WIDE_TRACE"); return e && e[0] == '1'; }();   // debug knob
-    if (trace_on) cudaGetSymbolAddress(reinterpret_cast<void**>(&p.trace), g_wide_trace);
     int rc = cuda_ok(cudaMemsetAsync(pack, 0, 8 * sizeof(int32_t), stream), "wide pre-pass counters");
     if (!rc) {
         wide_pack_kernel<<<(B + 7) / 8, 256, 0, stream>>>(mask, B, N, w->lay.S, w->tab + w->lay.dead_logits, v_out, logits_out, hidden_out, pack);

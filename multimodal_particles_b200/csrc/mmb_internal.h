@@ -85,7 +85,6 @@ int tf_stack_build(TfStack* st, const float* proj_in, int Cin, const float* bloc
                    const float* jet_w, const float* jet_b, int n_jet);
 void tf_stack_free(TfStack* st);
 int launch_tf_stack(const TfStack* st, int sm_count, const TfStackIO& io, int B, int N, cudaStream_t stream);
-int stack_read_trace(long long* out, int n);
 // out [B][n_jet] = folded per-jet Linear of the stack applied to the slot means written by launch_tf_stack
 int launch_jet_head(const TfStack* st, const float* means, int B, float* out, cudaStream_t stream);
 
@@ -162,7 +161,6 @@ int launch_epic_loss_grad(const MmbEpicDims& d, const float* W, const float* x, 
 
 // epic_tc.cu — tcgen05 path
 bool tc_supported(const MmbEpicDims* d, int N);
-int tc_read_trace(long long* out, int n);
 int tc_build_image(EpicModel* m, const float* packed_host);
 int launch_epic_forward_tc(const EpicModel* m, const float* x, const uint8_t* k, const uint8_t* mask,
                            const float* temb, int temb_stride, int B, int N,
@@ -176,13 +174,11 @@ int launch_generate_tc(const EpicModel* m, float* x, uint8_t* k, const uint8_t* 
 bool wide_supported(const MmbEpicDims* d, int N);
 int wide_build_image(EpicModel* m, const float* packed_host);
 void wide_free_image(EpicModel* m);
-int wide_read_trace(long long* out, int n);
 int launch_epic_forward_wide(const EpicModel* m, const float* x, const uint8_t* k, const uint8_t* mask, const float* temb, int temb_stride,
                              int B, int N, float* v_out, float* logits_out, float* hidden_out, cudaStream_t stream);
 
 // epic_mma.cu — warp-level MMA engine (register-resident chains), generation only
 bool mma_supported(const MmbEpicDims* d, int N);
-long long mma_read_trace(unsigned long long* out, long long max_words);
 int mma_build_images(EpicModel* m, const float* packed_host);
 size_t mma_generate_scratch_floats(const MmbEpicDims* d, int n_steps, int B);
 struct MmaHostIO {          // direct mode of mmb_generate_host: device-visible addresses of the caller's page-locked host buffers
@@ -191,8 +187,6 @@ struct MmaHostIO {          // direct mode of mmb_generate_host: device-visible 
     float* x_out;           // [B,N,Dc]
     long long* k_out;       // [B,N] int64
     int* bad_tokens;        // DEVICE flag
-    float* x_state;         // DEVICE scratch [B,N,Dc] / [B,N]: state of a jet between two of its time slices (epic_mma.cu)
-    uint8_t* k_state;
 };
 int launch_generate_mma(const EpicModel* m, float* x, uint8_t* k, const uint8_t* mask, const float* context, const float* dev_table, float* scratch,
                         int n_steps, float dt, const float* u_jump, uint64_t seed, uint64_t jet_offset,
