@@ -129,18 +129,9 @@ __global__ void __launch_bounds__(kLossThreads) bridge_losses_partial_kernel(con
     float mse = 0.0f, ce = 0.0f, cnt = 0.0f;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < P; i += (size_t)gridDim.x * blockDim.x) {
         if (!mask[i]) continue;
-        float e = 0.0f;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            const float d = __ldg(v + i * 3 + c) - (__ldg(x1 + i * 3 + c) - __ldg(x0 + i * 3 + c));
-            e = fmaf(d, d, e);
-        }
-        float mx = -INFINITY;
-        for (int s = 0; s < S; ++s) mx = fmaxf(mx, __ldg(logits + i * S + s));
-        float se = 0.0f;
-        for (int s = 0; s < S; ++s) se += expf(__ldg(logits + i * S + s) - mx);
-        mse += e;
-        ce += (mx + logf(se)) - __ldg(logits + i * S + k1[i]);
+        const float2 t = bridge_loss_terms(v + i * 3, x0 + i * 3, x1 + i * 3, 3, logits + i * S, S, k1[i]);
+        mse += t.x;
+        ce += t.y;
         cnt += 1.0f;
     }
 #pragma unroll

@@ -73,12 +73,6 @@ __device__ __forceinline__ void fmul2(float& d0, float& d1, float a0, float a1, 
         : "=f"(d0), "=f"(d1) : "f"(a0), "f"(a1), "f"(b0), "f"(b1));
 }
 
-// acc + sum_i w[i]*in[i], ascending i, one fmaf per term (the fp32 forward's dot product; epic_fp32.cu, epic_grad.cu)
-__device__ __forceinline__ float dot_from(float acc, const float* __restrict__ w, const float* in, int n) {
-    for (int i = 0; i < n; ++i) acc = __fmaf_rn(__ldg(w + i), in[i], acc);
-    return acc;
-}
-
 __device__ __forceinline__ float lrelu(float a) { return a > 0.0f ? a : __fmul_rn(a, 0.01f); }
 // the tensor-core engines' branch-free form
 __device__ __forceinline__ float lrelu_fast(float a) { return fmaxf(a, 0.01f * a); }
@@ -270,6 +264,23 @@ __device__ __forceinline__ int absorbing_birth(int m, float a, float u, const St
 
 __device__ __forceinline__ float euler(float x, float v, float dt, float mf) {
     return __fmul_rn(__fadd_rn(x, __fmul_rn(dt, v)), mf);
+}
+
+// The loss terms of one live particle (mbm.py:167-197): the squared error of its drift v against x1 - x0 over Dc components,
+// and its cross entropy max + log sum exp - logits[k1].  Shared by the bridge losses and the loss-gradient kernel.
+// Plain loads, not __ldg: the loss-gradient kernel passes rows it wrote earlier in the same launch.
+__device__ __forceinline__ float2 bridge_loss_terms(const float* v, const float* x0, const float* x1, int Dc, const float* logits,
+                                                    int S, int k1) {
+    float e = 0.0f;
+    for (int c = 0; c < Dc; ++c) {
+        const float d = v[c] - (x1[c] - x0[c]);
+        e = fmaf(d, d, e);
+    }
+    float mx = -INFINITY;
+    for (int s = 0; s < S; ++s) mx = fmaxf(mx, logits[s]);
+    float se = 0.0f;
+    for (int s = 0; s < S; ++s) se += expf(logits[s] - mx);
+    return make_float2(e, (mx + logf(se)) - logits[k1]);
 }
 
 }  // namespace mmb
